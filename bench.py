@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- RJMCMC iterations/s (all chains) at 1M lineages, and the K1 HBM roofline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W]            # the CUDA arm (one JSON line on rank 0)
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--dump-outputs DIR]    # the CUDA arm (one JSON line on rank 0)
     python bench.py --impl reference [--steps K] [--warmup W]      # the CPU arm (oracle port, all host cores)
 
 Workload (BASELINE.json configs[2]): synthetic 1M lineages x 200 one-year bins, 256 chains on one B200,
@@ -57,7 +57,12 @@ def _args():
     p.add_argument("--no-e2e", action="store_true")
     p.add_argument("--no-real-roofline", action="store_true", help="skip K1 on the real-valued tables (roofline_real, roofline_real_sorted)")
     p.add_argument("--no-multi", action="store_true", help="N > 1: skip BASELINE configs[3]/[4] (multi_gpu)")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed (rank 0's sample records and per-bin "
+                                                           "statistics) as DIR/<name>.npy in float64, to compare two builds output for output")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    return a
 
 
 def _workload(a, n_gpus):
@@ -121,6 +126,25 @@ def _peaks():
             return float(json.load(fh)["hbm_gbs"]), "MEASURED_PEAKS.json hbm_gbs (copy kernel, read+write)"
     except Exception:
         return 6650.0, "fallback 6.65 TB/s of B200_PROFILING.md (MEASURED_PEAKS.json absent)"
+
+
+DUMP_BYTES = 60 << 20    # array data of --dump-outputs; the index files and .npy headers stay within the remaining 4 MB of 64 MB
+
+
+def _dump_outputs(out_dir, arrays):
+    """Saves every (name, array, axis) as out_dir/<name>.npy in float64.  Past DUMP_BYTES in all, every array keeps the same
+    fraction of its slices along `axis`, picked with a fixed seed (so two runs keep the same ones); <name>_index.npy lists them."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    total = 8 * sum(x.size for _, x, _ in arrays)
+    for name, x, axis in arrays:
+        x = np.asarray(x, dtype=np.float64)
+        if total > DUMP_BYTES:
+            n = x.shape[axis]
+            keep = np.sort(np.random.default_rng(0).choice(n, max(1, n * DUMP_BYTES // total), replace=False))
+            x = np.take(x, keep, axis=axis)
+            np.save(os.path.join(out_dir, name + "_index.npy"), keep.astype(np.float64))
+        np.save(os.path.join(out_dir, name + ".npy"), x)
 
 
 def _sha16(path):
@@ -316,6 +340,7 @@ def run_cuda(a):
     cfg = E.default_config(0)
     k1_ms, k3_ms = [], []
     k1_build = ["k1_bin_kernel"]
+    last_stats = [None]                                    # (sp, ex, br) of the latest step, for --dump-outputs
 
     def step(k, timed):
         """One pass of the hot path with device-resident lineages."""
@@ -328,6 +353,7 @@ def run_cuda(a):
         e1.record()
         k1_build[0] = dev.bin_last_build()
         sp, ex, br = dev.bin_finalize_device(acc, nb, fe_ref=fe_ref, stream=stream.cuda_stream)
+        last_stats[0] = (sp, ex, br)
         ds = E.Dataset.from_device(dev, sp, ex, br, 0, float(FIRST_BIN), end_time, stream=stream.cuda_stream)
         ch = E.Chains(ds, chains, seed=2026 + k, cfg=cfg, chain_id0=rank * chains, rep_of_chain=rep_of_chain)
         e2.record()
@@ -402,7 +428,7 @@ def run_cuda(a):
                 e2e_push(k)
             pipe.flush(out=hrec)
             barrier()
-            n_e2e = max(2, a.steps)                  # as many steps as the device-timed value; the last step's chains cannot overlap a copy
+            n_e2e = a.steps                          # as many steps as the device-timed value; the last step's chains cannot overlap a copy
             t0 = time.perf_counter()
             for k in range(n_e2e):
                 tp = time.perf_counter()
@@ -573,6 +599,9 @@ def run_cuda(a):
                           % (cores, bins, nb, n, iters),
                 "loop_it_per_s_1core": r["it_per_s_loop_1core"], "binning_s_per_bin_1core": r["s_per_bin_1core"],
                 "whole_workload_s": r["whole_workload_s"]}
+        if a.dump_outputs:
+            sp, ex, br = (x.cpu().numpy() for x in last_stats[0])
+            _dump_outputs(a.dump_outputs, [("records", rec, 1), ("sp_events_bin", sp, 0), ("ex_events_bin", ex, 0), ("br_length_bin", br, 0)])
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.barrier()
