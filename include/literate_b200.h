@@ -74,9 +74,12 @@ int lr_sync(lr_handle_t h);
  *   sp, ex     int64 [n_rep][n_bins]  births  ts in [t0,t1), deaths te in (t0,t1]   (:120-121)
  *   br         fp64  [n_rep][n_bins]  sum_i max(0, min(te_i,t1) - max(ts_i,t0))      (:111-116)
  *
- * Counts are exact.  br is the correctly rounded exact sum (fractions are accumulated in 2^-52
- * fixed point), hence bit-identical to the reference for dyadic data and run-to-run
- * deterministic for any data.
+ * Counts are exact (from the raw doubles).  br is the correctly rounded exact sum of the clipped lifetimes, with every
+ * endpoint on the 2^-52 grid: fractions are accumulated in 2^-52 fixed point, a birth as
+ * floor(ts) + rint((ts - floor(ts)) * 2^52) / 2^52 and a death as c + rint((te - c) * 2^52) / 2^52, c = ceil(te) - 1, both
+ * differences taken in fp64 (ties to even).  For |t| >= 1 that is the time itself (the difference is exact and on the grid),
+ * so br is the exact sum there; times in (-1, 1) are first rounded to the grid.  Hence bit-identical to the reference for
+ * dyadic data and run-to-run deterministic for any data (oracle/k1_exact.py restates this definition).
  */
 #define LR_ACC_ROWS 8
 /* row stride (in int64) of the raw accumulator block of one replicate */
@@ -115,10 +118,13 @@ int lr_bin_stats_host(lr_handle_t h, const double* h_ts, const double* h_te, int
                       int64_t* h_sp, int64_t* h_ex, double* h_br);
 
 /* The same pass for tables of INTEGER YEARS held as int32 (8 bytes per lineage instead of 16 -- every table the
- * reference ships is of this kind once parsed, LiteRateForward.py:440-451): ts = year, te = year + death_jitter with
- * 0 <= death_jitter <= 1 (:471), i.e. what the fp64 entry points see after `te = te + death_jitter`.  Same accumulators,
- * bit for bit; finalize them with fe_ref = lr_fe_ref_of_jitter(death_jitter).  Pad ragged replicates with INT32_MIN in
- * both columns (a lineage that ends before the window: no contribution). */
+ * reference ships is of this kind once parsed, LiteRateForward.py:440-451): ts = year, te = year + death_jitter (:471),
+ * i.e. what the fp64 entry points see after `te = te + death_jitter`.  Every regular death is counted with the fraction
+ * death_jitter itself, which is what fl(year + death_jitter) leaves for every |year| < 2^31 only when death_jitter is a
+ * multiple of 2^-22 in [0, 1] (0, 0.25, 0.5, 1; not 0.1 or 1e-14): other jitters are refused (LR_ERR_INVALID) -- bin
+ * those tables through the fp64 entry points.  Same accumulators, bit for bit; finalize them with
+ * fe_ref = lr_fe_ref_of_jitter(death_jitter).  Pad ragged replicates with INT32_MIN in both columns (a lineage that ends
+ * before the window: no contribution). */
 int lr_bin_accumulate_i32(lr_handle_t h, const int32_t* d_ts, const int32_t* d_te, int64_t n, int64_t ld,
                           int32_t n_rep, int64_t first_bin, int32_t n_bins, double death_jitter,
                           int32_t dead_only, double end_time, int64_t* d_acc, void* stream);

@@ -780,7 +780,11 @@ extern "C" int lr_bin_accumulate_i32(lr_handle_t h, const int32_t* d_ts, const i
     LR_REQUIRE(h != nullptr, "lr_bin_accumulate_i32: null handle");
     LR_REQUIRE(n >= 0 && n_rep >= 1 && ld >= n, "lr_bin_accumulate_i32: need n >= 0, n_rep >= 1, ld >= n");
     LR_REQUIRE(n_bins >= 1, "lr_bin_accumulate_i32: n_bins must be >= 1");
-    LR_REQUIRE(death_jitter >= 0.0 && death_jitter <= 1.0, "lr_bin_accumulate_i32: death_jitter must lie in [0, 1] (te = year + jitter)");
+    // every regular death is counted with the fraction death_jitter: the fp64 table's fl(year + jitter) has it for every
+    // |year| < 2^31 iff the jitter is a multiple of 2^-22
+    LR_REQUIRE(death_jitter >= 0.0 && death_jitter <= 1.0 && ldexp(death_jitter, 22) == floor(ldexp(death_jitter, 22)),
+               "lr_bin_accumulate_i32: death_jitter must be a multiple of 2^-22 in [0, 1] (year + jitter exact for every int32 year); "
+               "bin other jitters as fp64 tables");
     LR_REQUIRE(d_acc != nullptr && (n == 0 || (d_ts != nullptr && d_te != nullptr)), "lr_bin_accumulate_i32: null pointer");
     const size_t smem = 2 * (size_t)n_bins * sizeof(unsigned);
     if (first_bin <= -(1ll << 30) || first_bin >= (1ll << 30) || smem + 1024 > (size_t)h->max_smem_optin) {

@@ -56,6 +56,16 @@ class BinStats:
 YEAR_PAD = np.iinfo(np.int32).min      # padding of ragged int32 year tables (both columns): contributes nothing
 
 
+def year_jitter_ok(death_jitter) -> bool:
+    """Whether an int32 year table with this death jitter gives the fp64 table's statistics exactly.
+
+    The int32 pass counts every regular death's fraction as exactly `death_jitter`; the fp64 pass sees fl(year + jitter).  The
+    two agree for every |year| < 2^31 iff year + jitter is exact there, i.e. 0 <= jitter <= 1 and jitter * 2^22 is an integer
+    (0, 0.25, 0.5, 1 are; 0.1 and 1e-14 are not).  The same check guards lr_bin_accumulate_i32."""
+    j = float(death_jitter)
+    return 0.0 <= j <= 1.0 and math.ldexp(j, 22).is_integer()
+
+
 def window(ts, te):
     """(first_bin, n_bins) = range(int(min ts), int(max te)) of :519 for host arrays."""
     first = int(np.min(ts))
@@ -105,15 +115,18 @@ class Device:
 
         ``ts``/``te`` are float64 arrays of shape [n] or [n_rep, n] (te already jittered, as after
         LiteRateForward.py:471) -- or int32 arrays of YEARS (te before the jitter, which ``death_jitter``
-        then supplies): half the bytes over PCIe, the same statistics bit for bit.  With ``only_dead`` the
-        extinct-only statistics of :529-549 are added, for lineages with te < end_time.
+        then supplies): half the bytes over PCIe, the same statistics bit for bit as the float64 table
+        (ts, te + death_jitter).  That holds only for jitters that are multiples of 2^-22 in [0, 1]
+        (year_jitter_ok); any other jitter raises ValueError for int32 tables -- pass the float64 table.
+        With ``only_dead`` the extinct-only statistics of :529-549 are added, for lineages with te < end_time.
         """
         years = np.asarray(ts).dtype == np.int32 and np.asarray(te).dtype == np.int32
         if years:
             # compact tables: integer YEARS as int32 (8 bytes per lineage over PCIe instead of 16); te is the year BEFORE the
             # jitter of :471, which the kernel adds (lr_bin_stats_host_i32).  Pad ragged replicates with YEAR_PAD.
-            if not 0.0 <= death_jitter <= 1.0:
-                raise ValueError("int32 year tables need 0 <= death_jitter <= 1")
+            if not year_jitter_ok(death_jitter):
+                raise ValueError("int32 year tables need a death_jitter in [0, 1] that is a multiple of 2^-22 (year + jitter "
+                                 "exact); bin the float64 table instead")
             ts = np.ascontiguousarray(ts); te = np.ascontiguousarray(te)
         else:
             ts = np.ascontiguousarray(ts, dtype=np.float64)
@@ -198,6 +211,8 @@ class Device:
         if ts.dtype == torch.int32:
             # int32 YEARS: `death_jitter` takes the place of fe_ref (te = year + jitter); finalize with fe_ref_for_jitter(death_jitter)
             jit = fe_ref if death_jitter is None else death_jitter
+            if not year_jitter_ok(jit):
+                raise ValueError("int32 year tables need a death_jitter in [0, 1] that is a multiple of 2^-22 (year + jitter exact)")
             N.check(self.lib.lr_bin_accumulate_i32(self.h, C.c_void_p(ts.data_ptr()), C.c_void_p(te.data_ptr()), n, ld, n_rep,
                                                    int(first_bin), int(n_bins), float(jit), 1 if dead_only else 0, float(end_time),
                                                    C.c_void_p(acc.data_ptr()), st), "lr_bin_accumulate_i32")

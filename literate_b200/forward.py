@@ -117,9 +117,11 @@ def parse_lineages(path, TBP=False, rev_se=0, first_year=-1, last_year=-1, death
 
 def as_year_table(ts, te, death_jitter):
     """(ts, te) as parse_lineages returns them -> int32 YEARS (ts, te - jitter) if the table is one of integer years (every table
-    the reference ships), else None.  The int32 entry point of K1 takes half the bytes and adds the jitter itself; the
-    statistics are the same bit for bit."""
-    if not 0.0 <= death_jitter <= 1.0:
+    the reference ships) and the jitter is one the int32 entry point reproduces exactly (E.year_jitter_ok: a multiple of
+    2^-22 in [0, 1], such as the default .5), else None.  The int32 entry point of K1 takes half the bytes and adds the jitter
+    itself; the statistics are the same bit for bit.  Other jitters (-death_jitter 0.1, say) give fl(year + jitter) a
+    fraction that differs from year to year, so such tables stay float64."""
+    if not E.year_jitter_ok(death_jitter):
         return None
     ok = ~np.isnan(ts)
     ey = te - death_jitter

@@ -1,14 +1,14 @@
 """GPU: K1 (lineages -> per-bin statistics) through the C ABI against the oracle.
 
-Bar: counts bit-exact always; br bit-exact for dyadic data (all shipped data: integer years + .5),
-<= 1e-12 relative for arbitrary real-valued times (the reference's own NumPy pairwise sum carries that
-much rounding; the kernel returns the correctly rounded exact sum).
+Bar: counts bit-exact always; br bit-exact against the exact reference (oracle/k1_exact.py: the correctly rounded exact
+sum the kernel promises) for any data -- equal to the oracle's own NumPy sums for dyadic data (all shipped data: integer
+years + .5), within their rounding for real-valued times.  tests/test_gpu_binstats_exact.py runs every entry point and build.
 """
 import numpy as np
 import pytest
 
 from conftest import golden_input
-from oracle import literate_oracle as O
+from oracle import k1_exact as K, literate_oracle as O
 from literate_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -24,19 +24,21 @@ def k1_build(request, monkeypatch):
     return request.param
 
 
-def _check(dev, ts, te, jitter, exact=True, only_dead=True):
+def _exact(ts, te, first_bin, n_bins, only_dead=False):
+    return K.exact_bin_stats(ts, te, first_bin, n_bins, only_dead=only_dead, end_time=np.max(te))
+
+
+def _check(dev, ts, te, jitter, only_dead=True):
     got = dev.bin_stats(ts, te, death_jitter=jitter, only_dead=only_dead)
     want = O.bin_stats(ts, te, only_dead=only_dead)
     assert got.first_bin == want.first_bin and got.n_bins == want.n_bins
     assert (got.sp[0] == want.sp).all() and (got.ex[0] == want.ex).all()
     if only_dead:
         assert (got.ex_dead[0] == want.ex_dead).all()
-    pairs = [(got.br[0], want.br)] + ([(got.br_dead[0], want.br_dead)] if only_dead else [])
+    exact = _exact(ts, te, want.first_bin, want.n_bins, only_dead)
+    pairs = [(got.br[0], exact[2])] + ([(got.br_dead[0], exact[4])] if only_dead else [])
     for g, w in pairs:
-        if exact:
-            assert (g == w).all()
-        else:
-            np.testing.assert_allclose(g, w, rtol=1e-12, atol=1e-12)
+        assert (g == w).all()
 
 
 def test_example_tad_and_tbp(device):
@@ -60,7 +62,7 @@ def test_random_integer_and_real(device, k1_build):
         ts, te = synth.syn_int(n, replicate=n)
         _check(device, ts, te, 0.5)
         ts, te = synth.syn_real(n, replicate=n)
-        _check(device, ts, te, 0.0, exact=False)
+        _check(device, ts, te, 0.0)
         # a wrong fe_ref hint must not change the result
         a = device.bin_stats(ts, te, fe_ref=0.5)
         b = device.bin_stats(ts, te, fe_ref=1.0)
@@ -83,7 +85,7 @@ def test_sorted_real_valued_tables_take_the_warp_merge(device, k1_build):
     ref = device.bin_stats(ts, te, death_jitter=0.0)
     want = O.bin_stats_fast(ts, te)
     assert (ref.sp[0] == want.sp).all() and (ref.ex[0] == want.ex).all()
-    np.testing.assert_allclose(ref.br[0], want.br, rtol=1e-12)
+    assert (ref.br[0] == _exact(ts, te, want.first_bin, want.n_bins)[2]).all()
     orders = {"by birth": np.argsort(ts), "by death": np.argsort(te), "first half by birth": np.r_[np.argsort(ts[:n // 2]), n // 2 + rng.permutation(n - n // 2)],
               "runs of 40": np.argsort(np.floor(ts) * 1e6 + np.arange(n) // 40 % 7)}
     for name, o in orders.items():
@@ -110,7 +112,7 @@ def test_degenerate_inputs(device, k1_build):
     # unsorted real values with many lineages born and dying in the same bin
     rng = np.random.default_rng(3)
     ts = 50 + rng.uniform(0, 20, 3000); te = ts + rng.uniform(0, 0.7, 3000); te[0] = 71.25
-    _check(device, ts, te, 0.0, exact=False)
+    _check(device, ts, te, 0.0)
 
 
 def test_explicit_window_with_lineages_outside(device, k1_build):
@@ -188,7 +190,7 @@ def test_full_size_one_million(device, k1_build):
     got = device.bin_stats(tr, er, death_jitter=0.0)
     want = O.bin_stats_fast(tr, er)
     assert (got.sp[0] == want.sp).all() and (got.ex[0] == want.ex).all()
-    np.testing.assert_allclose(got.br[0], want.br, rtol=1e-11)
+    assert (got.br[0] == _exact(tr, er, 1800, 200)[2]).all()
     again = device.bin_stats(tr, er, death_jitter=0.0)
     assert (again.br == got.br).all()          # run-to-run deterministic (integer accumulation)
 
@@ -234,7 +236,8 @@ def test_full_size_hundred_million_lineages(device):
 def test_int32_year_tables_give_the_same_statistics(device, metal_path):
     """lr_bin_stats_host_i32 / lr_bin_accumulate_i32: integer years as int32 (8 bytes per lineage), the death jitter of
     LiteRateForward.py:471 added by the kernel.  Same statistics as the fp64 entry points on the jittered table, bit for
-    bit: shipped tables, every jitter in [0, 1], extinct-only statistics, lineages outside / before the window, te < ts,
+    bit: shipped tables, jitters that are multiples of 2^-22 in [0, 1] (0, 0.25, 0.5, 1: the int32 entry points refuse any other),
+    extinct-only statistics, lineages outside / before the window, te < ts,
     ragged replicates padded with YEAR_PAD, row pitches that are not multiples of four, one lineage."""
     import torch
     from literate_b200 import engine as E
@@ -323,11 +326,11 @@ def test_lane_private_build_is_bit_identical_and_carries_into_the_third_word(dev
         got = res["1", False]
         if name.startswith("one bin"):
             assert got.sp[0, 0] == n and got.ex[0, 0] == n
-            np.testing.assert_allclose(got.br[0, 0], np.sum(te - ts), rtol=1e-12)
+            assert got.br[0, 0] == _exact(ts, te, 10, 1)[2][0]
             continue
         want = O.bin_stats_fast(ts, te)
         assert (got.sp[0] == want.sp).all() and (got.ex[0] == want.ex).all(), name
-        np.testing.assert_allclose(got.br[0], want.br, rtol=1e-12, atol=1e-9)
+        assert (got.br[0] == _exact(ts, te, want.first_bin, want.n_bins)[2]).all(), name
     # replicates with a ragged pitch, device entry point, raw accumulators
     tdev = torch.device("cuda:0")
     n_rep, n, ld, nb = 5, 70_001, 70_004, 37
@@ -369,8 +372,11 @@ def test_lane_private_build_is_bit_identical_and_carries_into_the_third_word(dev
     _same_accumulators(accs[0], accs[1])
     assert accs[0][0, 0, 1] == n and accs[0][0, 1, 1] == n
     sp, ex, br = device.bin_finalize_device(torch.from_numpy(accs[1]).to(tdev), 3, fe_ref=1.0)
-    want = float((e - t).sum())
-    assert abs(float(br[0, 1]) - want) <= 1e-9 * want and float(br[0, 0]) == 0.0 and float(br[0, 2]) == 0.0
+    # every lineage lies in [10, 11]: the exact time at risk is sum((te - 10) * 2^52 - (ts - 10) * 2^52), integers below 2^52
+    from fractions import Fraction
+    d = ((e - 10.0) * 2.0 ** 52).to(torch.int64) - ((t - 10.0) * 2.0 ** 52).to(torch.int64)
+    want = float(Fraction(int((d & ((1 << 26) - 1)).sum()) + (int((d >> 26).sum()) << 26), 1 << 52))
+    assert float(br[0, 1]) == want and float(br[0, 0]) == 0.0 and float(br[0, 2]) == 0.0
 
 
 def test_choice_of_build(device, monkeypatch):
