@@ -1406,13 +1406,6 @@ extern "C" int lr_proposal_eval_host(lr_dataset_t ds, int32_t n, const int32_t* 
     return LR_OK;
 }
 
-static inline int chain_grid(int n_chains, int& threads) {
-    // few chains: one warp per CTA so that they spread over all SMs; many chains: 4 warps per CTA
-    const int wpb = n_chains <= 1024 ? 1 : 4;
-    threads = wpb * 32;
-    return (n_chains + wpb - 1) / wpb;
-}
-
 extern "C" int lr_chains_create(lr_handle_t h, lr_dataset_t ds, int32_t n_chains, const lr_chain_config* cfg,
                                 uint64_t seed, int64_t chain_id0, const int32_t* h_rep_of_chain, lr_chains_t* out) {
     LR_REQUIRE(h && ds && cfg && out, "lr_chains_create: null pointer");
@@ -1442,7 +1435,7 @@ extern "C" int lr_chains_create(lr_handle_t h, lr_dataset_t ds, int32_t n_chains
         LR_CUDA(cudaMemcpyAsync(d_rep, h_rep_of_chain, (size_t)n_chains * 4, cudaMemcpyHostToDevice, h->stream));
     }
     int threads;
-    const int blocks = chain_grid(n_chains, threads);
+    const int blocks = lr_chain_grid(n_chains, threads);
     k3_init_kernel<<<blocks, threads, 0, h->stream>>>(c->st, n_chains, d_rep, chain_id0, (uint32_t)seed, (uint32_t)(seed >> 32),
                                                       ds->start_time, cfg->poisson_prior, c->cfg.beta);
     LR_CUDA(cudaGetLastError());
@@ -1464,15 +1457,9 @@ extern "C" int lr_chains_destroy(lr_chains_t c) {
 extern "C" int64_t lr_chains_records_per_run(lr_chains_t c, int64_t n_iter, int64_t sample_every) {
     if (!c || n_iter <= 0 || sample_every <= 0) return 0;
     long long it0 = c->it_host;
-    if (it0 < 0) {          // chains were given different iteration counters through set_state: chain 0's counts, as before
-        cudaSetDevice(c->h->device);
-        lr_order(c->h, &c->last, c->h->stream);
-        cudaStreamSynchronize(c->h->stream);
-        if (cudaMemcpy(&it0, &c->st[0].it, sizeof(long long), cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
-    }
-    const long long first = (it0 + sample_every - 1) / sample_every * sample_every;
-    const long long it1 = it0 + n_iter;
-    return first < it1 ? (it1 - 1 - first) / sample_every + 1 : 0;
+    // chains were given different iteration counters through set_state: chain 0's counts, as before
+    if (it0 < 0 && !lr_read_counter(c->h, &c->last, &c->st[0].it, &it0)) return -1;
+    return lr_records_per_run(it0, n_iter, sample_every);
 }
 
 extern "C" int lr_chains_run(lr_chains_t c, int64_t n_iter, int64_t sample_every, double* d_records, void* stream) {
@@ -1494,7 +1481,7 @@ extern "C" int lr_chains_run(lr_chains_t c, int64_t n_iter, int64_t sample_every
     P.records = sample_every > 0 ? d_records : nullptr;
     P.with_adequacy = 1;
     int threads;
-    const int blocks = chain_grid(c->n_chains, threads);
+    const int blocks = lr_chain_grid(c->n_chains, threads);
     // loop_variant: 0 = choose by population size (measured cross-over on B200), 1 = warp-specialised build
     // (one CTA of 4 warps per chain), 2 = compact build (one warp per chain)
     // loop_variant 0 picks by population size (measured on B200, 148 SMs; M it/s for one-chain CTAs / four-chain CTAs / compact):
@@ -1580,21 +1567,9 @@ extern "C" int lr_chains_run(lr_chains_t c, int64_t n_iter, int64_t sample_every
 
 extern "C" int lr_chains_run_host(lr_chains_t c, int64_t n_iter, int64_t sample_every, double* h_records) {
     LR_REQUIRE(c != nullptr, "lr_chains_run_host: null chains");
-    lr_handle_t h = c->h;
     const int64_t nrec = (h_records && sample_every > 0) ? lr_chains_records_per_run(c, n_iter, sample_every) : 0;
-    LR_REQUIRE(nrec >= 0, "lr_chains_run_host: could not read the iteration counter");
-    const size_t bytes = (size_t)nrec * c->n_chains * LR_REC_DOUBLES * sizeof(double);
-    double* d_rec = nullptr;
-    if (bytes) {
-        int rc = lr_ws_acquire(h, bytes, h->stream);
-        if (rc != LR_OK) return rc;
-        d_rec = (double*)h->ws;
-    }
-    int rc = lr_chains_run(c, n_iter, bytes ? sample_every : 0, d_rec, h->stream);
-    if (rc != LR_OK) return rc;
-    if (bytes) LR_CUDA(cudaMemcpyAsync(h_records, d_rec, bytes, cudaMemcpyDeviceToHost, h->stream));
-    LR_CUDA(cudaStreamSynchronize(h->stream));
-    return LR_OK;
+    return lr_run_into_host(c->h, "lr_chains_run_host", nrec, (size_t)c->n_chains * LR_REC_DOUBLES * sizeof(double), h_records,
+                            [&](double* d_rec) { return lr_chains_run(c, n_iter, d_rec ? sample_every : 0, d_rec, c->h->stream); });
 }
 
 extern "C" int lr_chains_counters_host(lr_chains_t c, int64_t* h_counters) {
@@ -1625,7 +1600,7 @@ extern "C" int lr_chains_get_state_host(lr_chains_t c, double* h_records) {
     int rc = lr_ws_acquire(h, bytes, h->stream);
     if (rc != LR_OK) return rc;
     int threads;
-    const int blocks = chain_grid(c->n_chains, threads);
+    const int blocks = lr_chain_grid(c->n_chains, threads);
     k3_get_state_kernel<<<blocks, threads, 0, h->stream>>>(c->st, c->n_chains, (double*)h->ws, c->ds->tab, c->ds->cst, c->ds->n_bins,
                                                            c->ds->s0f, c->ds->start_time, c->ds->end_time);
     LR_CUDA(cudaGetLastError());
@@ -1652,7 +1627,7 @@ extern "C" int lr_chains_set_state_host(lr_chains_t c, const double* h_records) 
     if (rc != LR_OK) return rc;
     LR_CUDA(cudaMemcpyAsync(h->ws, h_records, bytes, cudaMemcpyHostToDevice, h->stream));
     int threads;
-    const int blocks = chain_grid(c->n_chains, threads);
+    const int blocks = lr_chain_grid(c->n_chains, threads);
     k3_set_state_kernel<<<blocks, threads, 0, h->stream>>>(c->st, c->n_chains, (const double*)h->ws, c->ds->tab, c->ds->cst,
                                                            c->ds->n_bins, c->ds->s0f, c->ds->start_time, c->ds->end_time);
     LR_CUDA(cudaGetLastError());
@@ -1683,7 +1658,7 @@ extern "C" int lr_chains_swap_info(lr_chains_t c, double* d_info, void* stream) 
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     { int rc0 = lr_order(h, &c->last, st); if (rc0 == LR_OK) rc0 = lr_order(h, &c->ds->last, st); if (rc0 != LR_OK) return rc0; }
     int threads;
-    const int blocks = chain_grid(c->n_chains, threads);
+    const int blocks = lr_chain_grid(c->n_chains, threads);
     k3_swap_info_kernel<<<blocks, threads, 0, st>>>(c->st, c->n_chains, d_info, c->ds->tab, c->ds->cst, c->ds->n_bins, c->ds->s0f,
                                                     c->ds->start_time, c->ds->end_time);
     LR_CUDA(cudaGetLastError());
@@ -1702,7 +1677,7 @@ static int swap_apply(lr_chains_t c, const double* d_info_all, int64_t table_fir
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     { int rc0 = lr_order(h, &c->last, st); if (rc0 != LR_OK) return rc0; }
     int threads;
-    const int blocks = chain_grid(c->n_chains, threads);
+    const int blocks = lr_chain_grid(c->n_chains, threads);
     k3_swap_apply_kernel<<<blocks, threads, 0, st>>>(c->st, c->n_chains, d_info_all, table_first, n_all, first, ladder, round,
                                                      (uint32_t)c->seed, (uint32_t)(c->seed >> 32));
     LR_CUDA(cudaGetLastError());

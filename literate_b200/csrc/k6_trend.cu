@@ -13,7 +13,6 @@
 // two side sums come out of one butterfly.  A side none of whose parameters was touched keeps its stored likelihood (the
 // reference recomputes the identical number).  Nothing but the read-only per-bin table (L1-resident) is read inside the
 // loop; the only global writes are the sample records.
-#include <stdlib.h>
 #include "lr_common.cuh"
 
 #define TR_NPAR 6
@@ -57,12 +56,10 @@ struct TrendView {
     int nb, nbp, const_b, const_d;
     double Sx, Sxx;
     // the bins of the likelihood sums this warp owns: first + lane (statistics in registers), then every `stride`-th after it.
-    // One warp per chain: first = 0, stride = 32.  W warps per chain (wide build): first = 32 w, stride = 32 W.
+    // One warp per chain: first = 0, stride = 32.  W warps per chain: first = 32 w, stride = 32 W.
     int first, stride;
     double sp0, ex0, br0, lnT0;
 };
-// warps per chain of the wide build, by the number of bins
-__host__ __device__ inline int trend_groups(int nb) { return nb > 128 ? 4 : (nb > 64 ? 2 : 1); }
 
 __device__ __forceinline__ TrendView trend_view(const double* tab_all, const double* cst_all, int rep, int nb, int nbp,
                                                 int const_b, int const_d, int lane, int first = 0, int stride = 32) {
@@ -90,12 +87,8 @@ __device__ __forceinline__ double trend_rate(double a, double b, double c, doubl
 // T**delta and T**gamma of the first 32 bins (one per lane): they change only when delta / gamma are proposed
 struct PowCache { double b, d; };
 
-// both side likelihoods (uniform over the warp); a side with do_* == false keeps the value passed in.  newPowB/newPowD: the
-// exponent of that side differs from the one `pc` was computed for (pc is updated in place)
-// `extra`: a per-lane term (Hastings share + prior difference of the lane's parameter) that rides the same butterfly; its
-// warp total comes back in place.
 // partial sums over the bins this warp owns (per lane, not yet reduced)
-// termB / termD (wide build): if not null, every bin's term is also stored at its bin index
+// termB / termD (W > 1): if not null, every bin's term is also stored at its bin index
 __device__ __forceinline__ void trend_lik_partial(const TrendView& v, const double* p, int lane, bool doB, bool doD, bool newPowB, bool newPowD,
                                                   PowCache& pc, double& sB, double& sD, double* termB = nullptr, double* termD = nullptr) {
     sB = 0.0; sD = 0.0;
@@ -135,10 +128,26 @@ __device__ __forceinline__ void trend_lik_partial(const TrendView& v, const doub
     }
 }
 
+// both side likelihoods (uniform over the warp); a side with do_* == false keeps the value passed in.  newPowB/newPowD: the
+// exponent of that side differs from the one `pc` was computed for (pc is updated in place)
+// `extra`: a per-lane term (Hastings share + prior difference of the lane's parameter) that rides the same butterfly; its
+// warp total comes back in place.
+// W warps per chain (W > 1): termB / termD are this iteration's [nbp] buffers of shared memory.  Every warp stores the terms
+// of its bins there and then adds up all bins exactly as one warp per chain does -- lane l its bins l, l + 32, ... in
+// ascending order (0.0 for a side that was not evaluated), then one butterfly -- so the chain does not depend on W.
+template <int W = 1>
 __device__ __forceinline__ void trend_lik(const TrendView& v, const double* p, int lane, bool doB, bool doD, bool newPowB, bool newPowD,
-                                          PowCache& pc, double& likB, double& likD, double& extra) {
+                                          PowCache& pc, double& likB, double& likD, double& extra, double* termB = nullptr,
+                                          double* termD = nullptr) {
     double sB, sD;
-    trend_lik_partial(v, p, lane, doB, doD, newPowB, newPowD, pc, sB, sD);
+    if constexpr (W == 1) {
+        trend_lik_partial(v, p, lane, doB, doD, newPowB, newPowD, pc, sB, sD);
+    } else {
+        trend_lik_partial(v, p, lane, doB, doD, newPowB, newPowD, pc, sB, sD, termB, termD);
+        __syncthreads();
+        sB = 0.0; sD = 0.0;
+        for (int j = lane; j < v.nb; j += 32) { sB += termB[j]; sD += termD[j]; }
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         sB += __shfl_xor_sync(0xffffffffu, sB, o);
@@ -245,12 +254,21 @@ struct TrendRun {
     double fd_mult[TR_NPAR], fd_norm[TR_NPAR];  // Bernoulli probability of every parameter under the two proposal kinds
 };
 
-__global__ void __launch_bounds__(128, 4) k6_trend_kernel(const TrendRun P) {
-    const int lane = threadIdx.x & 31;
-    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+// W == 1: one warp per chain, four chains per CTA.  W = 2 or 4 (the wide build): one CTA of W warps per chain.  With a few
+// hundred chains and hundreds of bins one warp per chain leaves the GPU idle (ncu, round 1: sm__throughput 10 %, 7 bins per
+// lane in series, each an exp -> log chain).  There warp w evaluates bins 32 w + lane (+ 32 W k) -- at 200 bins and W = 4 two
+// per lane instead of seven.  Every warp draws the same random numbers, builds the same proposal and takes the same accept
+// decision; the warps exchange their per-bin terms through shared memory (double-buffered by iteration parity: one
+// __syncthreads per iteration) and add them up in the one-warp order (trend_lik), so the chain is the one-warp chain, bit for
+// bit (tests/test_gpu_trend.py), and does not depend on scheduling.
+template <int W>
+__global__ void __launch_bounds__(W == 1 ? 128 : 32 * W, W == 1 ? 4 : 2) k6_trend_kernel(const TrendRun P) {
+    extern __shared__ double terms[];                  // W > 1: [2 parities][2 sides][nbp]
+    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
+    const int c = W == 1 ? blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5) : blockIdx.x;
     if (c >= P.n_chains) return;
     TrendChain* S = P.st + c;
-    const TrendView v = trend_view(P.tab, P.cst, S->rep, P.nb, P.nbp, P.const_b, P.const_d, lane);
+    const TrendView v = trend_view(P.tab, P.cst, S->rep, P.nb, P.nbp, P.const_b, P.const_d, lane, W == 1 ? 0 : 32 * w, 32 * W);
     const unsigned chain = S->chain;
     double mine = lane < TR_NPAR ? S->p[lane] : 0.0;       // this lane's parameter; p[] = the broadcast copies
     double p[TR_NPAR];
@@ -265,6 +283,7 @@ __global__ void __launch_bounds__(128, 4) k6_trend_kernel(const TrendRun P) {
     const double fm = lane < TR_NPAR ? P.fd_mult[lane] : 0.0, fn = lane < TR_NPAR ? P.fd_norm[lane] : 0.0;
     long long next_sample = (it + P.sample_every - 1) / P.sample_every * P.sample_every;
     long long rec_idx = 0;
+    if constexpr (W > 1) __syncthreads();              // every warp has read the chain's state before warp 0 may rewrite it
 
     for (; it < it_end; ++it) {
         const Philox4 r = philox4x32_10((uint32_t)it, (uint32_t)((unsigned long long)it >> 32), (uint32_t)lane | (0x60u << 8), chain, P.k0, P.k1);
@@ -287,89 +306,9 @@ __global__ void __launch_bounds__(128, 4) k6_trend_kernel(const TrendRun P) {
         double hp = h + trend_prior_delta(lane, mine, prop, h);
         double nB = likB, nD = likD;
         PowCache npc = pc;
-        trend_lik(v, q, lane, (touched & 0x15u) != 0, (touched & 0x2au) != 0, (touched & 0x10u) != 0, (touched & 0x20u) != 0, npc, nB, nD, hp);
-        const double x = ((nB + nD) - (likB + likD)) + hp;
-        if (it == 0 || mh_accept_gt(x, u_acc)) {                            // trend_rate.py:176
-#pragma unroll
-            for (int k = 0; k < TR_NPAR; ++k) p[k] = q[k];
-            mine = prop;
-            likB = nB; likD = nD; pc = npc;
-            ++accepted;
-        }
-        if (it == next_sample) {                                             // trend_rate.py:184
-            if (P.records) trend_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v, p, mine, likB, likD, it, accepted, lane);
-            ++rec_idx;
-            next_sample += P.sample_every;
-        }
-    }
-    const double prior = warp_sum(trend_prior_term(lane, mine));
-    if (lane < TR_NPAR) S->p[lane] = mine;
-    if (lane == 0) { S->likB = likB; S->likD = likD; S->prior = prior; S->it = it; S->accepted = accepted; }
-}
-
-// WIDE build: W warps (one CTA) per chain.  With a few hundred chains and hundreds of bins one warp per chain leaves the GPU
-// idle (ncu, round 1: sm__throughput 10 %, 7 bins per lane in series, each an exp -> log chain).  Here warp w evaluates bins
-// 32 w + lane (+ 32 W k) -- at 200 bins and W = 4 two per lane instead of seven.  Every warp draws the same random numbers, builds
-// the same proposal and takes the same accept decision; the warps exchange their PER-BIN terms through shared memory
-// (double-buffered by iteration parity: one __syncthreads per iteration) and every warp then adds them up exactly as the
-// one-warp kernel does -- lane l its bins l, l + 32, l + 64, ... in ascending order, then one butterfly -- so the chain is
-// the one-warp kernel's chain, bit for bit (tests/test_gpu_trend.py), and does not depend on scheduling.
-template <int W>
-__global__ void __launch_bounds__(W * 32, 2) k6_trend_wide_kernel(const TrendRun P) {
-    extern __shared__ double terms[];                  // [2 parities][2 sides][nbp]
-    const int lane = threadIdx.x & 31, w = threadIdx.x >> 5;
-    const int c = blockIdx.x;
-    if (c >= P.n_chains) return;
-    TrendChain* S = P.st + c;
-    const TrendView v = trend_view(P.tab, P.cst, S->rep, P.nb, P.nbp, P.const_b, P.const_d, lane, 32 * w, 32 * W);
-    const unsigned chain = S->chain;
-    double mine = lane < TR_NPAR ? S->p[lane] : 0.0;
-    double p[TR_NPAR];
-    bcast6(mine, p);
-    double likB = S->likB, likD = S->likD;
-    PowCache pc;
-    pc.b = v.const_b ? 1.0 : exp(p[4] * v.lnT0);
-    pc.d = v.const_d ? 1.0 : exp(p[5] * v.lnT0);
-    long long it = S->it, accepted = S->accepted;
-    const long long it_end = it + P.n_iter;
-    const double fm = lane < TR_NPAR ? P.fd_mult[lane] : 0.0, fn = lane < TR_NPAR ? P.fd_norm[lane] : 0.0;
-    long long next_sample = (it + P.sample_every - 1) / P.sample_every * P.sample_every;
-    long long rec_idx = 0;
-    __syncthreads();                                   // every warp has read the chain's state before warp 0 may rewrite it
-
-    for (; it < it_end; ++it) {
-        const Philox4 r = philox4x32_10((uint32_t)it, (uint32_t)((unsigned long long)it >> 32), (uint32_t)lane | (0x60u << 8), chain, P.k0, P.k1);
-        const double ua = u01(r.x, r.y), ub = u01(r.z, r.w);
-        const double rr = __shfl_sync(0xffffffffu, ua, 6);
-        const double u_acc = __shfl_sync(0xffffffffu, ub, 6);
-        const int kind_normal = rr < 0.33;                                  // trend_rate.py:167
-        const double um = ((double)r.x + 0.5) * 2.3283064365386963e-10;
-        const bool on = um < (kind_normal ? fn : fm);
-        double draw = u01(r.y, r.z);
-        if (kind_normal) draw = normal_f32(draw, r.w);
-        double h;
-        const double prop = trend_propose(kind_normal, mine, on, draw, h);
-        const unsigned touched = __ballot_sync(0xffffffffu, on);
-        double q[TR_NPAR];
-        bcast6(prop, q);
-        double hp = h + trend_prior_delta(lane, mine, prop, h);
-        const bool doB = (touched & 0x15u) != 0, doD = (touched & 0x2au) != 0;
-        PowCache npc = pc;
         double* tB = terms + (size_t)(it & 1) * 2 * P.nbp;
         double* tD = tB + P.nbp;
-        double sB, sD;
-        trend_lik_partial(v, q, lane, doB, doD, (touched & 0x10u) != 0, (touched & 0x20u) != 0, npc, sB, sD, tB, tD);
-        __syncthreads();
-        // the one-warp kernel's order: lane l adds its bins l, l + 32, ... ascending (0.0 for a side that was not evaluated)
-        sB = 0.0; sD = 0.0;
-        for (int j = lane; j < P.nb; j += 32) { sB += tB[j]; sD += tD[j]; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            sB += __shfl_xor_sync(0xffffffffu, sB, o);
-            sD += __shfl_xor_sync(0xffffffffu, sD, o);
-            hp += __shfl_xor_sync(0xffffffffu, hp, o);
-        }
-        const double nB = doB ? sB : likB, nD = doD ? sD : likD;
+        trend_lik<W>(v, q, lane, (touched & 0x15u) != 0, (touched & 0x2au) != 0, (touched & 0x10u) != 0, (touched & 0x20u) != 0, npc, nB, nD, hp, tB, tD);
         const double x = ((nB + nD) - (likB + likD)) + hp;
         if (it == 0 || mh_accept_gt(x, u_acc)) {                            // trend_rate.py:176
 #pragma unroll
@@ -379,15 +318,16 @@ __global__ void __launch_bounds__(W * 32, 2) k6_trend_wide_kernel(const TrendRun
             ++accepted;
         }
         if (it == next_sample) {                                             // trend_rate.py:184
-            if (P.records && w == 0) {
-                const TrendView v0 = trend_view(P.tab, P.cst, S->rep, P.nb, P.nbp, P.const_b, P.const_d, lane);
+            if (P.records && (W == 1 || w == 0)) {
+                // W > 1: re-reading the view here keeps its constants out of registers across the loop (142, not 146)
+                const TrendView v0 = W == 1 ? v : trend_view(P.tab, P.cst, S->rep, P.nb, P.nbp, P.const_b, P.const_d, lane);
                 trend_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v0, p, mine, likB, likD, it, accepted, lane);
             }
             ++rec_idx;
             next_sample += P.sample_every;
         }
     }
-    if (w == 0) {
+    if (W == 1 || w == 0) {
         const double prior = warp_sum(trend_prior_term(lane, mine));
         if (lane < TR_NPAR) S->p[lane] = mine;
         if (lane == 0) { S->likB = likB; S->likD = likD; S->prior = prior; S->it = it; S->accepted = accepted; }
@@ -478,12 +418,6 @@ __global__ void k6_eval_kernel(const double* tab, const double* cst, int nb, int
         }
 }
 
-inline int trend_grid(int n, int& threads) {
-    const int wpb = n <= 1024 ? 1 : 4;      // few chains: one warp per CTA so that they spread over all SMs
-    threads = wpb * 32;
-    return (n + wpb - 1) / wpb;
-}
-
 // per-parameter Bernoulli probabilities of the two proposal kinds (trend_rate.py:122-134)
 void move_weights(int const_b, int const_d, double* f_mult, double* f_norm) {
     double m[TR_NPAR] = {1, 1, 0, 0, 1, 1}, nn[TR_NPAR] = {0, 0, 1, 1, 0, 0};
@@ -541,7 +475,7 @@ extern "C" int lr_trend_create(lr_handle_t h, int32_t n_rep, int32_t n_bins, con
     k6_build_tables<<<n_rep, 128, 0, st>>>((const long long*)d_sp, (const long long*)d_ex, d_br, d_trend, n_bins, t->nbp, t->tab, t->cst);
     LR_CUDA_CLEAN(cudaGetLastError(), undo());
     int threads;
-    const int blocks = trend_grid(n_chains, threads);
+    const int blocks = lr_chain_grid(n_chains, threads);
     k6_init_kernel<<<blocks, threads, 0, st>>>(t->st, n_chains, d_rep, chain_id0, t->tab, t->cst, n_bins, t->nbp, t->const_b, t->const_d);
     LR_CUDA_CLEAN(cudaGetLastError(), undo());
     h->launches += 2;
@@ -558,16 +492,10 @@ extern "C" int lr_trend_create_host(lr_handle_t h, int32_t n_rep, int32_t n_bins
                                     lr_trend_t* out) {
     LR_REQUIRE(h && h_sp && h_ex && h_br, "lr_trend_create_host: null pointer");
     LR_REQUIRE(n_rep >= 1 && n_bins >= 1, "lr_trend_create_host: bad sizes");
-    LR_CUDA(cudaSetDevice(h->device));
-    const size_t cnt = (size_t)n_rep * n_bins;
-    int rc = lr_ws_acquire(h, cnt * 24, h->stream);
+    int64_t *d_sp, *d_ex;
+    double* d_br;
+    int rc = lr_upload_bin_stats(h, (size_t)n_rep * n_bins, h_sp, h_ex, h_br, &d_sp, &d_ex, &d_br);
     if (rc != LR_OK) return rc;
-    int64_t* d_sp = (int64_t*)h->ws;
-    int64_t* d_ex = d_sp + cnt;
-    double* d_br = (double*)(d_ex + cnt);
-    LR_CUDA(cudaMemcpyAsync(d_sp, h_sp, cnt * 8, cudaMemcpyHostToDevice, h->stream));
-    LR_CUDA(cudaMemcpyAsync(d_ex, h_ex, cnt * 8, cudaMemcpyHostToDevice, h->stream));
-    LR_CUDA(cudaMemcpyAsync(d_br, h_br, cnt * 8, cudaMemcpyHostToDevice, h->stream));
     return lr_trend_create(h, n_rep, n_bins, d_sp, d_ex, d_br, h_trend, const_birth, const_death, n_chains, seed, chain_id0,
                            h_rep_of_chain, h->stream, out);
 }
@@ -586,13 +514,8 @@ extern "C" int lr_trend_destroy(lr_trend_t t) {
 extern "C" int64_t lr_trend_records_per_run(lr_trend_t t, int64_t n_iter, int64_t sample_every) {
     if (!t || n_iter <= 0 || sample_every <= 0) return 0;
     long long it0 = 0;
-    cudaSetDevice(t->h->device);
-    lr_order(t->h, &t->last, t->h->stream);
-    cudaStreamSynchronize(t->h->stream);
-    if (cudaMemcpy(&it0, &t->st[0].it, sizeof(long long), cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
-    const long long first = (it0 + sample_every - 1) / sample_every * sample_every;
-    const long long it1 = it0 + n_iter;
-    return first < it1 ? (it1 - 1 - first) / sample_every + 1 : 0;
+    if (!lr_read_counter(t->h, &t->last, &t->st[0].it, &it0)) return -1;
+    return lr_records_per_run(it0, n_iter, sample_every);
 }
 
 extern "C" int lr_trend_run(lr_trend_t t, int64_t n_iter, int64_t sample_every, double* d_records, void* stream) {
@@ -611,17 +534,15 @@ extern "C" int lr_trend_run(lr_trend_t t, int64_t n_iter, int64_t sample_every, 
     P.rec_doubles = (int)lr_trend_record_doubles(t->n_bins);
     for (int k = 0; k < TR_NPAR; ++k) { P.fd_mult[k] = t->f_mult[k]; P.fd_norm[k] = t->f_norm[k]; }
     int threads;
-    const int blocks = trend_grid(t->n_chains, threads);
+    const int blocks = lr_chain_grid(t->n_chains, threads);
     // wide build (one warp per canonical group of bins) when one warp per chain would leave most of the GPU idle: measured on
     // B200 at 200 bins, M it/s one-warp / wide: 256 chains 82 / 141, 2048 chains 454 / 213.  Same chains either way.
-    int W = trend_groups(t->n_bins);
-    if ((long long)t->n_chains * W > (long long)h->sm_count * 8) W = 1;
-    { const char* e = getenv("LR_TREND_WIDE"); if (e) W = atoi(e) ? trend_groups(t->n_bins) : 1; }         // development override
+    int W = lr_chain_width(t->n_bins, t->n_chains, h->sm_count, "LR_TREND_WIDE");
     const size_t smem = (size_t)4 * t->nbp * sizeof(double);
     if (W > 1 && smem > 40 * 1024) W = 1;
-    if (W == 4) k6_trend_wide_kernel<4><<<t->n_chains, 128, smem, st>>>(P);
-    else if (W == 2) k6_trend_wide_kernel<2><<<t->n_chains, 64, smem, st>>>(P);
-    else k6_trend_kernel<<<blocks, threads, 0, st>>>(P);
+    if (W == 4) k6_trend_kernel<4><<<t->n_chains, 128, smem, st>>>(P);
+    else if (W == 2) k6_trend_kernel<2><<<t->n_chains, 64, smem, st>>>(P);
+    else k6_trend_kernel<1><<<blocks, threads, 0, st>>>(P);
     LR_CUDA(cudaGetLastError());
     h->launches += 1;
     return LR_OK;
@@ -629,21 +550,9 @@ extern "C" int lr_trend_run(lr_trend_t t, int64_t n_iter, int64_t sample_every, 
 
 extern "C" int lr_trend_run_host(lr_trend_t t, int64_t n_iter, int64_t sample_every, double* h_records) {
     LR_REQUIRE(t != nullptr, "lr_trend_run_host: null chains");
-    lr_handle_t h = t->h;
     const int64_t nrec = (h_records && sample_every > 0) ? lr_trend_records_per_run(t, n_iter, sample_every) : 0;
-    LR_REQUIRE(nrec >= 0, "lr_trend_run_host: could not read the iteration counter");
-    const size_t bytes = (size_t)nrec * t->n_chains * lr_trend_record_doubles(t->n_bins) * sizeof(double);
-    double* d_rec = nullptr;
-    if (bytes) {
-        int rc = lr_ws_acquire(h, bytes, h->stream);
-        if (rc != LR_OK) return rc;
-        d_rec = (double*)h->ws;
-    }
-    int rc = lr_trend_run(t, n_iter, bytes ? sample_every : 0, d_rec, h->stream);
-    if (rc != LR_OK) return rc;
-    if (bytes) LR_CUDA(cudaMemcpyAsync(h_records, d_rec, bytes, cudaMemcpyDeviceToHost, h->stream));
-    LR_CUDA(cudaStreamSynchronize(h->stream));
-    return LR_OK;
+    return lr_run_into_host(t->h, "lr_trend_run_host", nrec, (size_t)t->n_chains * lr_trend_record_doubles(t->n_bins) * sizeof(double),
+                            h_records, [&](double* d_rec) { return lr_trend_run(t, n_iter, d_rec ? sample_every : 0, d_rec, t->h->stream); });
 }
 
 extern "C" int lr_trend_eval_host(lr_trend_t t, int32_t n, const int32_t* rep, const double* params, const int32_t* kind,

@@ -14,7 +14,6 @@
 // parameters was touched keeps its stored value, and so do the logarithms of the niche of the first 32 bins.  The genre term of
 // -m_birth 3 needs births and time at risk of the genre table inside [origin, origin + x0) and [origin + x0, present):
 // one strided pass over the (small, L1-resident) genre table whenever x0 is proposed, cached otherwise.
-#include <stdlib.h>
 #include "lr_common.cuh"
 
 #define DD_NPAR LR_DD_NPAR
@@ -143,11 +142,8 @@ __device__ __forceinline__ DDBin0 dd_bin0(const DDView& v, int lane, int first =
     return b;
 }
 
-// newL / newC: a parameter of the logistic / constant carrying capacity differs from the one `c` was computed for
-// `extra`: a per-lane term (Hastings share + prior difference of the lane's parameter) that rides the same butterfly; its warp
-// total comes back in place.
 // Per-lane partial sums over the bins first + lane, first + lane + stride, ... (one warp per chain: first 0, stride 32; warp w of
-// the wide build: first 32 w, stride 32 W).  termB / termD (wide build): every bin's term is also stored at its bin index.
+// W per chain: first 32 w, stride 32 W).  termB / termD (W > 1): every bin's term is also stored at its bin index.
 __device__ __forceinline__ void dd_lik_partial(const DDView& v, const DDBin0& b0, int first, int stride, const double* p, int lane, bool doB,
                                                bool doD, bool newL, bool newC, DDCache& c, double& sB, double& sD,
                                                double* termB = nullptr, double* termD = nullptr) {
@@ -212,10 +208,22 @@ __device__ __forceinline__ void dd_lik_partial(const DDView& v, const DDBin0& b0
 // newL / newC: a parameter of the logistic / constant carrying capacity differs from the one `c` was computed for
 // `extra`: a per-lane term (Hastings share + prior difference of the lane's parameter) that rides the same butterfly; its warp
 // total comes back in place.
+// W warps per chain (W > 1): this warp's bins start at `first`; termB / termD are this iteration's [nbp] buffers of shared
+// memory.  Every warp stores the terms of its bins there and then adds up all bins in the one-warp order (lane l its bins l,
+// l + 32, ... ascending, then one butterfly), so the chain does not depend on W.
+template <int W = 1>
 __device__ __forceinline__ void dd_lik(const DDView& v, const DDBin0& b0, const double* p, int lane, bool doB, bool doD, bool newL,
-                                       bool newC, DDCache& c, double& likB, double& likD, double& extra) {
+                                       bool newC, DDCache& c, double& likB, double& likD, double& extra, int first = 0,
+                                       double* termB = nullptr, double* termD = nullptr) {
     double sB, sD;
-    dd_lik_partial(v, b0, 0, 32, p, lane, doB, doD, newL, newC, c, sB, sD);
+    if constexpr (W == 1) {
+        dd_lik_partial(v, b0, 0, 32, p, lane, doB, doD, newL, newC, c, sB, sD);
+    } else {
+        dd_lik_partial(v, b0, first, 32 * W, p, lane, doB, doD, newL, newC, c, sB, sD, termB, termD);
+        __syncthreads();
+        sB = 0.0; sD = 0.0;
+        for (int j = lane; j < v.nb; j += 32) { sB += termB[j]; sD += termD[j]; }
+    }
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) {
         sB += __shfl_xor_sync(0xffffffffu, sB, o);
@@ -376,97 +384,15 @@ struct DDRun {
     int tail_n;            // entries per buffer of the shared-memory log-niche cache of the bins beyond the first 32 (0: none)
 };
 
-__global__ void __launch_bounds__(128, 3) k7_dd_kernel(const DDRun P) {
-    const int lane = threadIdx.x & 31;
-    const int c = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    if (c >= P.n_chains) return;
-    DDChain* S = P.st + c;
-    const DDView v = dd_select(P.v, S->rep);
-    const unsigned chain = S->chain;
-    double mine = lane < DD_NPAR ? S->p[lane] : 0.0;
-    double p[DD_NPAR];
-    dd_bcast(mine, p);
-    double likB = S->likB, likD = S->likD, likG = S->likG;
-    double g[4] = {S->g[0], S->g[1], S->g[2], S->g[3]};
-    const DDBin0 b0 = dd_bin0(v, lane);
-    const DDPriorLane pl = dd_prior_lane(v, lane);
-    const unsigned maskL = (1u << P_K) | (1u << P_X0) | (1u << P_DIV0) | (1u << P_L), maskC = (1u << P_DIV0) | (1u << P_L);
-    extern __shared__ double tail_s[];
-    DDCache cache;
-    cache.nt = P.tail_n; cache.sel = 0;
-    cache.tail = P.tail_n > 0 ? tail_s + (size_t)(threadIdx.x >> 5) * 2 * P.tail_n : nullptr;
-    if (cache.tail != nullptr)
-        for (int j = lane + 32; j < v.nb; j += 32) cache.tail[j - 32] = log(dd_niche_logistic(p, j));
-    cache.lnL0 = log(dd_niche_logistic(p, lane));
-    cache.lnC = log(p[P_L] + p[P_DIV0]);
-    cache.lg1 = log(p[P_G1]); cache.lg2 = log(p[P_G2]);
-    long long it = S->it, accepted = S->accepted;
-    const long long it_end = it + P.n_iter;
-    double fmine = 0.0;
-#pragma unroll
-    for (int k = 0; k < DD_NPAR; ++k)
-        if (lane == k) fmine = P.f[k];
-    const bool can_slide = v.mb >= 1 || v.md >= 1;
-    long long next_sample = (it + P.sample_every - 1) / P.sample_every * P.sample_every;
-    long long rec_idx = 0;
-
-    for (; it < it_end; ++it) {
-        const Philox4 r = philox4x32_10((uint32_t)it, (uint32_t)((unsigned long long)it >> 32), (uint32_t)lane | (0x70u << 8), chain, P.k0, P.k1);
-        const double ua = u01(r.x, r.y), ub = u01(r.z, r.w);
-        const double rr1 = __shfl_sync(0xffffffffu, ua, 11), rr2 = __shfl_sync(0xffffffffu, ub, 11);
-        const double us = __shfl_sync(0xffffffffu, ua, 12);
-        const double u_acc = __shfl_sync(0xffffffffu, ub, 12);
-        const int kind = (rr1 < 0.1 && can_slide) ? (rr2 < 0.5 ? 1 : 2) : 0;                  // :248-258
-        const bool on = kind == 0 && (((double)r.x + 0.5) * 2.3283064365386963e-10) < fmine;
-        double h;
-        const double prop = dd_propose(v, lane, kind, mine, on, kind == 0 ? u01(r.y, r.z) : us, h);
-        unsigned touched = __ballot_sync(0xffffffffu, on);
-        if (kind == 1) touched = 1u << P_X0;
-        if (kind == 2) touched = 1u << P_MMUL;
-        double q[DD_NPAR];
-        dd_bcast(prop, q);
-        double hp = h + dd_prior_delta(v, pl, mine, prop, h);       // summed in the butterfly of the likelihood
-        double nB = likB, nD = likD, nG = likG;
-        double ng[4] = {g[0], g[1], g[2], g[3]};
-        DDCache nc = cache;
-        dd_lik(v, b0, q, lane, (touched & P.depB) != 0, (touched & P.depD) != 0, (touched & maskL) != 0, (touched & maskC) != 0, nc, nB, nD, hp);
-        if (v.mb == 3) {
-            if (touched & (1u << P_X0)) dd_genre_stats(v, q[P_X0], lane, ng);
-            if (touched & ((1u << P_X0) | (1u << P_G1) | (1u << P_G2)))
-                nG = dd_genre_lik(q, ng, (touched & (1u << P_G1)) != 0, (touched & (1u << P_G2)) != 0, nc);
-        }
-        const double x = ((nB + nD + nG) - (likB + likD + likG)) + hp;
-        if (it == 0 || mh_accept_gt(x, u_acc)) {                                                 // :263
-#pragma unroll
-            for (int k = 0; k < DD_NPAR; ++k) p[k] = q[k];
-            mine = prop;
-            likB = nB; likD = nD; likG = nG; cache = nc;
-            g[0] = ng[0]; g[1] = ng[1]; g[2] = ng[2]; g[3] = ng[3];
-            ++accepted;
-        }
-        if (it == next_sample) {                                                                 // :274
-            if (P.records) dd_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v, p, mine, likB, likD, likG, it, accepted, lane);
-            ++rec_idx;
-            next_sample += P.sample_every;
-        }
-    }
-    const double prior = warp_sum(dd_prior_term(v, lane, mine));
-    if (lane < DD_NPAR) S->p[lane] = mine;
-    if (lane == 0) {
-        S->likB = likB; S->likD = likD; S->likG = likG; S->prior = prior; S->it = it; S->accepted = accepted;
-        S->g[0] = g[0]; S->g[1] = g[1]; S->g[2] = g[2]; S->g[3] = g[3];
-    }
-}
-
-// WIDE build: W warps (one CTA) per chain, as k6_trend_wide_kernel: warp w evaluates bins 32 w + lane (+ 32 W k), every warp draws
-// the same random numbers and takes the same decision, the per-bin terms are exchanged through shared memory (double-buffered by
-// iteration parity, one __syncthreads per iteration) and added in the one-warp kernel's order -- the same chain, bit for bit.
-// The log-niche cache of the bins beyond each warp's register bin is one CTA-wide array indexed by bin.
+// W == 1: one warp per chain, four chains per CTA.  W = 2 or 4 (the wide build, as k6_trend_kernel<W>): one CTA of W warps per
+// chain; warp w evaluates bins 32 w + lane (+ 32 W k), every warp draws the same random numbers and takes the same decision, the
+// per-bin terms are exchanged through shared memory (double-buffered by iteration parity, one __syncthreads per iteration) and
+// added in the one-warp order (dd_lik) -- the same chain, bit for bit.
 template <int W>
-__global__ void __launch_bounds__(W * 32, 2) k7_dd_wide_kernel(const DDRun P) {
+__global__ void __launch_bounds__(W == 1 ? 128 : 32 * W, W == 1 ? 3 : 2) k7_dd_kernel(const DDRun P) {
     const int lane = threadIdx.x & 31, wq = threadIdx.x >> 5;
-    const int first = 32 * wq, stride = 32 * W;
-    const int c = blockIdx.x;
+    const int first = W == 1 ? 0 : 32 * wq, stride = 32 * W;
+    const int c = W == 1 ? blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5) : blockIdx.x;
     if (c >= P.n_chains) return;
     DDChain* S = P.st + c;
     const DDView v = dd_select(P.v, S->rep);
@@ -479,11 +405,13 @@ __global__ void __launch_bounds__(W * 32, 2) k7_dd_wide_kernel(const DDRun P) {
     const DDBin0 b0 = dd_bin0(v, lane, first);
     const DDPriorLane pl = dd_prior_lane(v, lane);
     const unsigned maskL = (1u << P_K) | (1u << P_X0) | (1u << P_DIV0) | (1u << P_L), maskC = (1u << P_DIV0) | (1u << P_L);
-    extern __shared__ double tail_s[];                 // [2][tail_n] log-niche cache, then [2 parities][2 sides][nbp] per-bin terms
+    // the log-niche cache of the bins beyond each warp's register bin: W == 1 [warp][2][tail_n], W > 1 one CTA-wide [2][tail_n]
+    // indexed by bin, followed by the per-bin terms [2 parities][2 sides][nbp]
+    extern __shared__ double tail_s[];
     double* terms = tail_s + 2 * (size_t)P.tail_n;
     DDCache cache;
     cache.nt = P.tail_n; cache.sel = 0;
-    cache.tail = P.tail_n > 0 ? tail_s : nullptr;
+    cache.tail = P.tail_n > 0 ? (W == 1 ? tail_s + (size_t)(threadIdx.x >> 5) * 2 * P.tail_n : tail_s) : nullptr;
     if (cache.tail != nullptr)
         for (int j = first + lane + stride; j < v.nb; j += stride) cache.tail[j - 32] = log(dd_niche_logistic(p, j));
     cache.lnL0 = log(dd_niche_logistic(p, first + lane));
@@ -498,7 +426,7 @@ __global__ void __launch_bounds__(W * 32, 2) k7_dd_wide_kernel(const DDRun P) {
     const bool can_slide = v.mb >= 1 || v.md >= 1;
     long long next_sample = (it + P.sample_every - 1) / P.sample_every * P.sample_every;
     long long rec_idx = 0;
-    __syncthreads();                                   // every warp has read the chain's state before warp 0 may rewrite it
+    if constexpr (W > 1) __syncthreads();              // every warp has read the chain's state before warp 0 may rewrite it
 
     for (; it < it_end; ++it) {
         const Philox4 r = philox4x32_10((uint32_t)it, (uint32_t)((unsigned long long)it >> 32), (uint32_t)lane | (0x70u << 8), chain, P.k0, P.k1);
@@ -522,19 +450,7 @@ __global__ void __launch_bounds__(W * 32, 2) k7_dd_wide_kernel(const DDRun P) {
         const bool doB = (touched & P.depB) != 0, doD = (touched & P.depD) != 0;
         double* tB = terms + (size_t)(it & 1) * 2 * v.nbp;
         double* tD = tB + v.nbp;
-        double sB, sD;
-        dd_lik_partial(v, b0, first, stride, q, lane, doB, doD, (touched & maskL) != 0, (touched & maskC) != 0, nc, sB, sD, tB, tD);
-        __syncthreads();
-        sB = 0.0; sD = 0.0;                             // the one-warp kernel's order: lane l adds its bins l, l + 32, ... ascending
-        for (int j = lane; j < v.nb; j += 32) { sB += tB[j]; sD += tD[j]; }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) {
-            sB += __shfl_xor_sync(0xffffffffu, sB, o);
-            sD += __shfl_xor_sync(0xffffffffu, sD, o);
-            hp += __shfl_xor_sync(0xffffffffu, hp, o);
-        }
-        if (doB) nB = sB;
-        if (doD) nD = v.md >= 1 ? sD : v.likD_const;
+        dd_lik<W>(v, b0, q, lane, doB, doD, (touched & maskL) != 0, (touched & maskC) != 0, nc, nB, nD, hp, first, tB, tD);
         if (v.mb == 3) {
             if (touched & (1u << P_X0)) dd_genre_stats(v, q[P_X0], lane, ng);
             if (touched & ((1u << P_X0) | (1u << P_G1) | (1u << P_G2)))
@@ -550,12 +466,13 @@ __global__ void __launch_bounds__(W * 32, 2) k7_dd_wide_kernel(const DDRun P) {
             ++accepted;
         }
         if (it == next_sample) {                                                                 // :274
-            if (P.records && wq == 0) dd_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v, p, mine, likB, likD, likG, it, accepted, lane);
+            if (P.records && (W == 1 || wq == 0))
+                dd_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v, p, mine, likB, likD, likG, it, accepted, lane);
             ++rec_idx;
             next_sample += P.sample_every;
         }
     }
-    if (wq != 0) return;
+    if (W > 1 && wq != 0) return;
     const double prior = warp_sum(dd_prior_term(v, lane, mine));
     if (lane < DD_NPAR) S->p[lane] = mine;
     if (lane == 0) {
@@ -659,12 +576,6 @@ __global__ void k7_eval_kernel(const DDView v_all, int n, const int* rep, const 
     if (series) dd_series(series + (size_t)s * 4 * v.nb, v, p, lane);
 }
 
-inline int dd_grid(int n, int& threads) {
-    const int wpb = n <= 1024 ? 1 : 4;
-    threads = wpb * 32;
-    return (n + wpb - 1) / wpb;
-}
-
 // update_multiplier (:208-225) and the parameters every term depends on
 void dd_model_tables(int mb, int md, double* f, unsigned& depB, unsigned& depD) {
     double w[DD_NPAR];
@@ -746,7 +657,7 @@ extern "C" int lr_dd_create(lr_handle_t h, int32_t n_rep, int32_t n_bins, const 
     if (ce != cudaSuccess) { lr_set_error("lr_dd_create: %s", cudaGetErrorString(ce)); undo(); return LR_ERR_CUDA; }
     if (bad >= 0) { lr_set_error("lr_dd_create: replicate %d has no time at risk in any bin", bad); undo(); return LR_ERR_INVALID; }
     int threads;
-    const int blocks = dd_grid(n_chains, threads);
+    const int blocks = lr_chain_grid(n_chains, threads);
     k7_init_kernel<<<blocks, threads, 0, st>>>(t->st, n_chains, d_rep, chain_id0, dd_view(t));
     LR_CUDA_CLEAN(cudaGetLastError(), undo());
     h->launches += 2;
@@ -762,16 +673,10 @@ extern "C" int lr_dd_create_host(lr_handle_t h, int32_t n_rep, int32_t n_bins, c
                                  int32_t n_chains, uint64_t seed, int64_t chain_id0, const int32_t* h_rep_of_chain, lr_dd_t* out) {
     LR_REQUIRE(h && h_sp && h_ex && h_br, "lr_dd_create_host: null pointer");
     LR_REQUIRE(n_rep >= 1 && n_bins >= 1, "lr_dd_create_host: bad sizes");
-    LR_CUDA(cudaSetDevice(h->device));
-    const size_t cnt = (size_t)n_rep * n_bins;
-    int rc = lr_ws_acquire(h, cnt * 24, h->stream);
+    int64_t *d_sp, *d_ex;
+    double* d_br;
+    int rc = lr_upload_bin_stats(h, (size_t)n_rep * n_bins, h_sp, h_ex, h_br, &d_sp, &d_ex, &d_br);
     if (rc != LR_OK) return rc;
-    int64_t* d_sp = (int64_t*)h->ws;
-    int64_t* d_ex = d_sp + cnt;
-    double* d_br = (double*)(d_ex + cnt);
-    LR_CUDA(cudaMemcpyAsync(d_sp, h_sp, cnt * 8, cudaMemcpyHostToDevice, h->stream));
-    LR_CUDA(cudaMemcpyAsync(d_ex, h_ex, cnt * 8, cudaMemcpyHostToDevice, h->stream));
-    LR_CUDA(cudaMemcpyAsync(d_br, h_br, cnt * 8, cudaMemcpyHostToDevice, h->stream));
     return lr_dd_create(h, n_rep, n_bins, d_sp, d_ex, d_br, origin, present, m_birth, m_death, h_gts, h_gte, n_genre, n_chains, seed,
                         chain_id0, h_rep_of_chain, h->stream, out);
 }
@@ -791,13 +696,8 @@ extern "C" int lr_dd_destroy(lr_dd_t t) {
 extern "C" int64_t lr_dd_records_per_run(lr_dd_t t, int64_t n_iter, int64_t sample_every) {
     if (!t || n_iter <= 0 || sample_every <= 0) return 0;
     long long it0 = 0;
-    cudaSetDevice(t->h->device);
-    lr_order(t->h, &t->last, t->h->stream);
-    cudaStreamSynchronize(t->h->stream);
-    if (cudaMemcpy(&it0, &t->st[0].it, sizeof(long long), cudaMemcpyDeviceToHost) != cudaSuccess) return -1;
-    const long long first = (it0 + sample_every - 1) / sample_every * sample_every;
-    const long long it1 = it0 + n_iter;
-    return first < it1 ? (it1 - 1 - first) / sample_every + 1 : 0;
+    if (!lr_read_counter(t->h, &t->last, &t->st[0].it, &it0)) return -1;
+    return lr_records_per_run(it0, n_iter, sample_every);
 }
 
 extern "C" int lr_dd_run(lr_dd_t t, int64_t n_iter, int64_t sample_every, double* d_records, void* stream) {
@@ -817,27 +717,21 @@ extern "C" int lr_dd_run(lr_dd_t t, int64_t n_iter, int64_t sample_every, double
     for (int k = 0; k < DD_NPAR; ++k) P.f[k] = t->f[k];
     P.depB = t->depB; P.depD = t->depD;
     int threads;
-    const int blocks = dd_grid(t->n_chains, threads);
-    // log-niche cache of the bins beyond the first 32: [warp][2 buffers][tail_n] doubles of shared memory, if it fits 48 KB
+    const int blocks = lr_chain_grid(t->n_chains, threads);
+    // Shared memory, up to 48 KB: the log-niche cache of the bins beyond the first 32 (W == 1: [warp][2 buffers][tail_n]
+    // doubles, left out if it does not fit), and for W > 1 one [2][tail_n] cache plus the per-bin terms [2][2][nbp] (one warp
+    // per chain if they do not fit)
+    int W = lr_chain_width(t->n_bins, t->n_chains, h->sm_count, "LR_DD_WIDE");
     P.tail_n = t->n_bins > 32 ? t->nbp - 32 : 0;
-    size_t smem = (size_t)(threads / 32) * 2 * P.tail_n * sizeof(double);
-    if (smem > 48 * 1024) { P.tail_n = 0; smem = 0; }
-    // wide build (W warps per chain) when one warp per chain would leave most of the GPU idle and there are bins to share
-    int W = t->n_bins > 128 ? 4 : (t->n_bins > 64 ? 2 : 1);
-    if ((long long)t->n_chains * W > (long long)h->sm_count * 8) W = 1;
-    { const char* e = getenv("LR_DD_WIDE"); if (e) W = atoi(e) ? (t->n_bins > 128 ? 4 : (t->n_bins > 64 ? 2 : 1)) : 1; }      // development override
-    if (W > 1) {
-        P.tail_n = t->nbp - 32;
-        const size_t wsmem = ((size_t)2 * P.tail_n + (size_t)4 * t->nbp) * sizeof(double);
-        if (wsmem > 48 * 1024) W = 1;
-        else if (W == 4) k7_dd_wide_kernel<4><<<t->n_chains, 128, wsmem, st>>>(P);
-        else k7_dd_wide_kernel<2><<<t->n_chains, 64, wsmem, st>>>(P);
-    }
+    size_t smem = ((size_t)2 * P.tail_n + (size_t)4 * t->nbp) * sizeof(double);
+    if (W > 1 && smem > 48 * 1024) W = 1;
     if (W == 1) {
-        P.tail_n = t->n_bins > 32 ? t->nbp - 32 : 0;
-        if ((size_t)(threads / 32) * 2 * P.tail_n * sizeof(double) > 48 * 1024) P.tail_n = 0;
-        k7_dd_kernel<<<blocks, threads, smem, st>>>(P);
+        smem = (size_t)(threads / 32) * 2 * P.tail_n * sizeof(double);
+        if (smem > 48 * 1024) { P.tail_n = 0; smem = 0; }
     }
+    if (W == 4) k7_dd_kernel<4><<<t->n_chains, 128, smem, st>>>(P);
+    else if (W == 2) k7_dd_kernel<2><<<t->n_chains, 64, smem, st>>>(P);
+    else k7_dd_kernel<1><<<blocks, threads, smem, st>>>(P);
     LR_CUDA(cudaGetLastError());
     h->launches += 1;
     return LR_OK;
@@ -845,21 +739,9 @@ extern "C" int lr_dd_run(lr_dd_t t, int64_t n_iter, int64_t sample_every, double
 
 extern "C" int lr_dd_run_host(lr_dd_t t, int64_t n_iter, int64_t sample_every, double* h_records) {
     LR_REQUIRE(t != nullptr, "lr_dd_run_host: null chains");
-    lr_handle_t h = t->h;
     const int64_t nrec = (h_records && sample_every > 0) ? lr_dd_records_per_run(t, n_iter, sample_every) : 0;
-    LR_REQUIRE(nrec >= 0, "lr_dd_run_host: could not read the iteration counter");
-    const size_t bytes = (size_t)nrec * t->n_chains * lr_dd_record_doubles(t->n_bins) * sizeof(double);
-    double* d_rec = nullptr;
-    if (bytes) {
-        int rc = lr_ws_acquire(h, bytes, h->stream);
-        if (rc != LR_OK) return rc;
-        d_rec = (double*)h->ws;
-    }
-    int rc = lr_dd_run(t, n_iter, bytes ? sample_every : 0, d_rec, h->stream);
-    if (rc != LR_OK) return rc;
-    if (bytes) LR_CUDA(cudaMemcpyAsync(h_records, d_rec, bytes, cudaMemcpyDeviceToHost, h->stream));
-    LR_CUDA(cudaStreamSynchronize(h->stream));
-    return LR_OK;
+    return lr_run_into_host(t->h, "lr_dd_run_host", nrec, (size_t)t->n_chains * lr_dd_record_doubles(t->n_bins) * sizeof(double),
+                            h_records, [&](double* d_rec) { return lr_dd_run(t, n_iter, d_rec ? sample_every : 0, d_rec, t->h->stream); });
 }
 
 extern "C" int lr_dd_eval_host(lr_dd_t t, int32_t n, const int32_t* rep, const double* params, const int32_t* kind, const int32_t* on,

@@ -3,6 +3,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <stdlib.h>
 #include <string.h>
 #include "../../include/literate_b200.h"
 
@@ -83,6 +84,73 @@ struct lr_last_stream { cudaStream_t s; int valid; };
 int lr_order(lr_handle_t h, lr_last_stream* last, cudaStream_t now);
 // the workspace, at least `bytes` large, for work submitted to `stream` (ordered after its previous user)
 int lr_ws_acquire(lr_handle_t h, size_t bytes, cudaStream_t stream);
+
+// ---- host plumbing of the chain objects (K3 lr_chains_t, K6 lr_trend_t, K7 lr_dd_t) -------------------------------------------
+// launch grid of the one-warp-per-chain kernels: few chains get one warp per CTA so that they spread over all SMs, many chains 4
+inline int lr_chain_grid(int n, int& threads) {
+    const int wpb = n <= 1024 ? 1 : 4;
+    threads = wpb * 32;
+    return (n + wpb - 1) / wpb;
+}
+
+// Warps per chain of the K6 / K7 chain loop.  W warps (one CTA) share a chain's bins when one warp per chain would leave most
+// of the GPU idle and there are bins to share.  The environment variable `env` overrides the population rule (development):
+// 0 one warp per chain, anything else the width by the bins.
+inline int lr_chain_width(int n_bins, int n_chains, int sm_count, const char* env) {
+    const int W = n_bins > 128 ? 4 : (n_bins > 64 ? 2 : 1);
+    if (const char* e = getenv(env)) return atoi(e) ? W : 1;
+    return (long long)n_chains * W > (long long)sm_count * 8 ? 1 : W;
+}
+
+// records a run of n_iter iterations from iteration it0 writes: one per multiple of sample_every in [it0, it0 + n_iter)
+inline long long lr_records_per_run(long long it0, long long n_iter, long long sample_every) {
+    const long long first = (it0 + sample_every - 1) / sample_every * sample_every;
+    const long long it1 = it0 + n_iter;
+    return first < it1 ? (it1 - 1 - first) / sample_every + 1 : 0;
+}
+
+// iteration counter of a chain, read from the device after everything submitted to the object so far; false on failure
+inline bool lr_read_counter(lr_handle_t h, lr_last_stream* last, const long long* d_it, long long* it) {
+    cudaSetDevice(h->device);
+    lr_order(h, last, h->stream);
+    cudaStreamSynchronize(h->stream);
+    return cudaMemcpy(it, d_it, sizeof(long long), cudaMemcpyDeviceToHost) == cudaSuccess;
+}
+
+// The *_run_host entry points: `nrec` samples of `sample_bytes` each (nrec < 0: the iteration counter could not be read) are
+// recorded into the workspace by run(d_records) -- d_records null: no records -- and copied to h_records; returns when done.
+template <class Run>
+int lr_run_into_host(lr_handle_t h, const char* fn, int64_t nrec, size_t sample_bytes, double* h_records, Run run) {
+    LR_REQUIRE(nrec >= 0, "%s: could not read the iteration counter", fn);
+    const size_t bytes = (size_t)nrec * sample_bytes;
+    double* d_rec = nullptr;
+    if (bytes) {
+        int rc = lr_ws_acquire(h, bytes, h->stream);
+        if (rc != LR_OK) return rc;
+        d_rec = (double*)h->ws;
+    }
+    int rc = run(d_rec);
+    if (rc != LR_OK) return rc;
+    if (bytes) LR_CUDA(cudaMemcpyAsync(h_records, d_rec, bytes, cudaMemcpyDeviceToHost, h->stream));
+    LR_CUDA(cudaStreamSynchronize(h->stream));
+    return LR_OK;
+}
+
+// The *_create_host entry points of K6 / K7: the per-bin statistics sp, ex, br [cnt] from the host into the workspace, on the
+// handle's stream
+inline int lr_upload_bin_stats(lr_handle_t h, size_t cnt, const int64_t* h_sp, const int64_t* h_ex, const double* h_br, int64_t** d_sp,
+                               int64_t** d_ex, double** d_br) {
+    LR_CUDA(cudaSetDevice(h->device));
+    int rc = lr_ws_acquire(h, cnt * 24, h->stream);
+    if (rc != LR_OK) return rc;
+    *d_sp = (int64_t*)h->ws;
+    *d_ex = *d_sp + cnt;
+    *d_br = (double*)(*d_ex + cnt);
+    LR_CUDA(cudaMemcpyAsync(*d_sp, h_sp, cnt * 8, cudaMemcpyHostToDevice, h->stream));
+    LR_CUDA(cudaMemcpyAsync(*d_ex, h_ex, cnt * 8, cudaMemcpyHostToDevice, h->stream));
+    LR_CUDA(cudaMemcpyAsync(*d_br, h_br, cnt * 8, cudaMemcpyHostToDevice, h->stream));
+    return LR_OK;
+}
 
 // ---- small device helpers --------------------------------------------------------------------
 __device__ __forceinline__ double2 ld_stream_f64x2(const double2* p) {

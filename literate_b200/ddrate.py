@@ -12,10 +12,8 @@ New flags: -chains (chain k is named like a reference run with seed + k), -devic
 """
 from __future__ import annotations
 
-import argparse
 import csv
 import ctypes as C
-import glob
 import os
 import time
 
@@ -23,8 +21,9 @@ import numpy as np
 
 from . import _native as N
 from . import engine as E
+from . import library as L
 from . import parallel as P
-from .trend import bin_window, parse_ts_te
+from .library import bin_window, parse_ts_te
 
 BANNER = "\n\n             DDRate  (literate_b200: B200-native path)\n"
 PARAMS = ["l_f", "l_mul", "k", "x0", "div_0", "L", "m_mul", "nuB", "nuD", "g_lambda1", "g_lambda2"]
@@ -32,48 +31,26 @@ REC_HEAD, NPAR = N.LR_DD_REC_HEAD, N.LR_DD_NPAR
 
 
 def build_parser():
-    p = argparse.ArgumentParser(prog="DDRatev3.py")
-    p.add_argument('-v', action='version', version='%(prog)s')
-    p.add_argument('-d', type=str, help='data file', default="", metavar="")
-    p.add_argument('-n', type=int, help='n. MCMC iterations', default=10000000, metavar=10000000)
-    p.add_argument('-p', type=int, help='print frequency', default=1000, metavar=1000)
-    p.add_argument('-s', type=int, help='sampling frequency', default=1000, metavar=1000)
-    p.add_argument('-seed', type=int, help='seed (set to -1 to make it random)', default=-1, metavar=-1)
-    p.add_argument('-TBP', help='Default is AD. Include for TBP.', default=False, action='store_true')
-    p.add_argument('-first_year', type=int, help='different start of the dataset', default=-1, metavar=-1)
-    p.add_argument('-last_year', type=int, help='different end of the dataset', default=-1, metavar=-1)
-    p.add_argument('-death_jitter', type=float, help='amount to jitter death times', default=.5, metavar=.5)
-    p.add_argument('-rm_first_bin', type=float, help='if set to 1 it removes the first time bin', default=0, metavar=0)
-    p.add_argument('-print_emp', help='Prints empirical rates', default=False, action='store_true')
-    p.add_argument('-m_birth', type=int, help='0) use const b rates 1) DD birth 2) niche dep DD b', default=2, metavar=2)
-    p.add_argument('-m_death', type=int, help='-1) fixed d rate 0) use const d rates 1) DD death 2) niche dep DD d', default=2, metavar=2)
-    p.add_argument('-fix_birth', type=float, help='Fix birth rate (with -m_birth -1)', default=0.1, metavar=0.1)
-    p.add_argument('-fix_death', type=float, help='Fix death rate (with -m_death -1)', default=0.1, metavar=0.1)
-    p.add_argument('--genre_times', '-g', type=str, help='Genre Data File', default='', metavar='')
-    # ---- not in the reference
-    p.add_argument('-chains', type=int, help='number of independent chains run concurrently on the GPU', default=1, metavar=1)
-    p.add_argument('-device', type=int, help='CUDA device index', default=0, metavar=0)
-    p.add_argument('-quiet', type=int, help='1: no per-sample progress on stdout', default=0, metavar=0)
-    return p
+    def own(p):                                                       # DDRatev3.py:25-29
+        p.add_argument('-m_birth', type=int, help='0) use const b rates 1) DD birth 2) niche dep DD b', default=2, metavar=2)
+        p.add_argument('-m_death', type=int, help='-1) fixed d rate 0) use const d rates 1) DD death 2) niche dep DD d', default=2, metavar=2)
+        p.add_argument('-fix_birth', type=float, help='Fix birth rate (with -m_birth -1)', default=0.1, metavar=0.1)
+        p.add_argument('-fix_death', type=float, help='Fix death rate (with -m_death -1)', default=0.1, metavar=0.1)
+        p.add_argument('--genre_times', '-g', type=str, help='Genre Data File', default='', metavar='')
+    return L.build_parser("DDRatev3.py", own)
 
 
-class DDChains:
+class DDChains(L.ChainObject):
     """lr_dd_t: the per-bin table, the genre table and a population of independent DDRate chains on one device."""
+    PREFIX, STATE_DOUBLES = "dd", N.LR_DD_STATE_DOUBLES
 
     def __init__(self, dev: E.Device, sp, ex, br, origin, present, m_birth=2, m_death=2, gts=None, gte=None, n_chains=1, seed=1,
                  chain_id0=0, rep_of_chain=None):
-        sp = np.ascontiguousarray(np.atleast_2d(sp), dtype=np.int64)
-        ex = np.ascontiguousarray(np.atleast_2d(ex), dtype=np.int64)
-        br = np.ascontiguousarray(np.atleast_2d(br), dtype=np.float64)
+        sp, ex, br, rep = self._inputs(sp, ex, br, rep_of_chain, n_chains)
         if not (sp.shape == ex.shape == br.shape):
             raise ValueError("sp, ex, br must be [n_bins] or [n_rep, n_bins]")
         self.dev, self.n_chains, self.n_rep, self.n_bins = dev, int(n_chains), sp.shape[0], sp.shape[1]
         self.m_birth, self.m_death, self.origin = int(m_birth), int(m_death), float(origin)
-        rep = None
-        if rep_of_chain is not None:
-            rep = np.ascontiguousarray(rep_of_chain, dtype=np.int32)
-            if rep.shape != (self.n_chains,):
-                raise ValueError("rep_of_chain must have one entry per chain")
         ng = 0
         if gts is not None:
             gts = np.ascontiguousarray(gts, dtype=np.float64)
@@ -83,41 +60,7 @@ class DDChains:
         N.check(dev.lib.lr_dd_create_host(dev.h, self.n_rep, self.n_bins, N.np_ptr(sp), N.np_ptr(ex), N.np_ptr(br), float(origin),
                                           float(present), self.m_birth, self.m_death, N.np_ptr(gts), N.np_ptr(gte), ng, self.n_chains,
                                           C.c_uint64(int(seed) & (2**64 - 1)), int(chain_id0), N.np_ptr(rep), C.byref(t)), "lr_dd_create_host")
-        self.t = t
-        self.rec_doubles = int(dev.lib.lr_dd_record_doubles(self.n_bins))
-
-    def close(self):
-        if getattr(self, "t", None):
-            self.dev.lib.lr_dd_destroy(self.t)
-            self.t = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def records_per_run(self, n_iter, sample_every):
-        return int(self.dev.lib.lr_dd_records_per_run(self.t, int(n_iter), int(sample_every)))
-
-    def run(self, n_iter, sample_every=0):
-        """n_iter iterations of every chain; returns records [n_samples, n_chains, 24 + 4 n_bins] (host) or None."""
-        if sample_every and sample_every > 0:
-            out = np.empty((self.records_per_run(n_iter, sample_every), self.n_chains, self.rec_doubles), dtype=np.float64)
-            N.check(self.dev.lib.lr_dd_run_host(self.t, int(n_iter), int(sample_every), N.np_ptr(out)), "lr_dd_run_host")
-            return out
-        N.check(self.dev.lib.lr_dd_run_host(self.t, int(n_iter), 0, None), "lr_dd_run_host")
-        return None
-
-    def run_device(self, n_iter, sample_every, records, stream=None):
-        st = C.c_void_p(None) if isinstance(stream, str) and stream == "handle" else E._stream_ptr(stream)
-        ptr = C.c_void_p(records.data_ptr()) if records is not None else None
-        N.check(self.dev.lib.lr_dd_run(self.t, int(n_iter), int(sample_every) if records is not None else 0, ptr, st), "lr_dd_run")
-
-    def state(self):
-        out = np.empty((self.n_chains, N.LR_DD_STATE_DOUBLES), dtype=np.float64)
-        N.check(self.dev.lib.lr_dd_state_host(self.t, N.np_ptr(out)), "lr_dd_state_host")
-        return out
+        self._created(t)
 
     def evaluate(self, params, kind=None, on=None, draw=None, rep=None):
         """Parity entry point: the three likelihood terms, prior, per-bin series, adequacy and genre statistics of explicit
@@ -195,34 +138,10 @@ def run(args, device=None):
                          "DDRatev3.py:192-195)")
     if args.m_birth == 3 and not args.genre_times:
         raise SystemExit("-m_birth 3 needs the genre table: -g <file> (DDRatev3.py:36-38)")
-    if args.seed == -1:
-        if world > 1:
-            raise SystemExit("give -seed explicitly when running on several GPUs (every rank must use the same one)")
-        seed = int(np.random.randint(0, 9999))
-    else:
-        seed = args.seed
-    if args.chains < max(1, world):
-        raise SystemExit("-chains must be >= 1 and at least the number of GPUs")
-    # -d may name a DIRECTORY of tables (stochastic imputations of one data set): one replicate each, common window
-    if os.path.isdir(args.d):
-        tables = sorted(f for f in glob.glob(os.path.join(args.d, "*")) if os.path.isfile(f) and f.lower().endswith((".tsv", ".txt"))
-                        and os.path.abspath(f) != os.path.abspath(args.genre_times or "-"))
-        if not tables:
-            raise SystemExit("no .tsv/.txt table in " + args.d)
-    else:
-        tables = [args.d]
-    parsed = [parse_ts_te(f, args.TBP, args.first_year, args.last_year, args.death_jitter) for f in tables]
-    n_tab = len(parsed)
-    if args.chains == 1 and n_tab > 1:
-        args.chains = n_tab
-    if args.chains % n_tab:
-        raise SystemExit("-chains must be a multiple of the number of tables (%d)" % n_tab)
-    present, origin = max(p[2] for p in parsed), min(p[3] for p in parsed)
+    seed = L.seed_and_chains(args, world)
+    tables, ts, te, present, origin = L.read_tables(args, exclude=args.genre_times or "-")
+    n_tab = len(tables)
     first_bin, n_bins = bin_window(origin, present, args.rm_first_bin)
-    n_max = max(len(p[0]) for p in parsed)
-    ts = np.full((n_tab, n_max), np.nan); te = np.full((n_tab, n_max), np.nan)      # NaN rows carry no event and no time at risk
-    for i, p in enumerate(parsed):
-        ts[i, :len(p[0])], te[i, :len(p[1])] = p[0], p[1]
     dev = device if device is not None else E.Device(local_rank if world > 1 else args.device)
     t0 = time.time()
     stats = dev.bin_stats(ts, te, first_bin=first_bin, n_bins=n_bins, death_jitter=args.death_jitter)
@@ -258,25 +177,8 @@ def run(args, device=None):
         else:
             write_div_log(stem + ".div.log", sp[r], ex[r], br[r], gstats.sp[0], gstats.ex[0], gstats.br[0])
 
-    s_freq = max(1, args.s)
-    max_rec = max(1, (256 << 20) // (n_local * chains.rec_doubles * 8))
-    per_launch = max(s_freq, min(max_rec * s_freq, 4_000_000) // s_freq * s_freq)
-    done = 0
-    t_run = time.time()
-    while done < args.n:
-        n_it = min(per_launch, args.n - done)
-        recs = chains.run(n_it, s_freq)
-        done += n_it
-        for r in range(recs.shape[0]):
-            for k in range(n_local):
-                writers[k].writerow(record_row(recs[r, k], n_bins, args.m_birth, origin))
-            if not args.quiet:
-                print(int(recs[r, 0, 0]), recs[r, 0, 1], recs[r, 0, 5:5 + NPAR])       # :280
-        for fh in files:
-            fh.flush()
-    t_run = time.time() - t_run
-    for fh in files:
-        fh.close()
+    t_run = L.sample_and_write(chains, args.n, args.s, files, writers, lambda rec: record_row(rec, n_bins, args.m_birth, origin),
+                               lambda rec: print(int(rec[0]), rec[1], rec[5:5 + NPAR]), args.quiet)       # :280
     if not args.quiet:
         acc = chains.state()[:, 16].sum() / max(1, n_local * args.n)
         print("literate_b200: %d DDRate chains x %d iterations in %.3f s (%.3g it/s, acceptance %.3f); binning %.4f s"

@@ -15,19 +15,18 @@ stream whatever the number of GPUs.
 """
 from __future__ import annotations
 
-import argparse
 import csv
 import ctypes as C
-import glob
 import os
 import time
-from warnings import warn
 
 import numpy as np
 
 from . import _native as N
 from . import engine as E
+from . import library as L
 from . import parallel as P
+from .library import bin_window, parse_ts_te  # noqa: F401  (parse_ts_te: callers of this module keep importing it from here)
 
 BANNER = "\n\n             TrendRate - 20190205  (literate_b200: B200-native path)\n"
 SMALL_NUMBER = 0.000000000000001                         # trend_rate.py:55
@@ -41,80 +40,14 @@ def _flag(v):
 
 
 def build_parser():
-    p = argparse.ArgumentParser(prog="trend_rate.py")
-    p.add_argument('-v', action='version', version='%(prog)s')
-    p.add_argument('-d', type=str, help='data file', default="", metavar="")
-    p.add_argument('-n', type=int, help='n. MCMC iterations', default=10000000, metavar=10000000)
-    p.add_argument('-p', type=int, help='print frequency', default=1000, metavar=1000)
-    p.add_argument('-s', type=int, help='sampling frequency', default=1000, metavar=1000)
-    p.add_argument('-seed', type=int, help='seed (set to -1 to make it random)', default=-1, metavar=-1)
-    p.add_argument('-TBP', help='Default is AD. Include for TBP.', default=False, action='store_true')
-    p.add_argument('-first_year', type=int, help='different start of the dataset', default=-1, metavar=-1)
-    p.add_argument('-last_year', type=int, help='different end of the dataset', default=-1, metavar=-1)
-    p.add_argument('-death_jitter', type=float, help='amount to jitter death times', default=.5, metavar=.5)
-    p.add_argument('-rm_first_bin', type=float, help='if set to 1 it removes the first time bin', default=0, metavar=0)
-    p.add_argument('-print_emp', help='Prints empirical rates', default=False, action='store_true')
-    p.add_argument('-trend_data', metavar='<path to trend file>', type=str, default="",
-                   help='Input trend file should be columns tab-separated with headers. No missing values.')
-    p.add_argument('-trend_index', type=int, help='Column of trend in trend file.', default=0, metavar=0)
-    p.add_argument('-const_B', type=_flag, help='F) Vary rates with trend T) Constant rates', default=False, metavar=False)
-    p.add_argument('-const_D', type=_flag, help='F) Vary rates with trend T) Constant rates', default=False, metavar=False)
-    p.add_argument('-no_death', type=_flag, help='F) Calculate death rate T) Likelihood based on births only', default=False, metavar=False)
-    # ---- not in the reference
-    p.add_argument('-chains', type=int, help='number of independent chains run concurrently on the GPU', default=1, metavar=1)
-    p.add_argument('-device', type=int, help='CUDA device index', default=0, metavar=0)
-    p.add_argument('-quiet', type=int, help='1: no per-sample progress on stdout', default=0, metavar=0)
-    return p
-
-
-def parse_ts_te(path, TBP=False, first_year=-1, last_year=-1, death_jitter=0.5):
-    """literate_library.parse_ts_te (:196-229) -> (ts, te, present, origin); the same pandas parser as the reference."""
-    import pandas as pd
-    t = pd.read_csv(path, delimiter="\t").to_numpy()
-    if t.shape[1] == 4:
-        warn('Four column (with clade) LiteRate input is deprecated. Use three columns.', FutureWarning)
-        ts_y, te_y = t[:, 2], t[:, 3]
-    else:
-        ts_y, te_y = t[:, 1], t[:, 2]
-    ts_y = np.asarray(ts_y, dtype=np.float64)
-    te_y = np.asarray(te_y, dtype=np.float64).copy()
-    if TBP:
-        if first_year != -1:
-            keep = ts_y <= first_year
-            ts_y, te_y = ts_y[keep], te_y[keep]
-        if last_year != -1:                      # (the reference masks te with the already filtered ts, :210-211)
-            keep = ts_y >= last_year
-            ts_y, te_y = ts_y[keep], te_y[keep]
-            te_y[te_y < last_year] = last_year
-        root = np.max(ts_y)
-        ts, te = root - ts_y, root - te_y
-    else:
-        if first_year != -1:
-            keep = ts_y >= first_year
-            ts_y, te_y = ts_y[keep], te_y[keep]
-        if last_year != -1:
-            keep = ts_y <= last_year
-            ts_y, te_y = ts_y[keep], te_y[keep]
-            te_y[te_y > last_year] = last_year
-        ts, te = ts_y, te_y
-    te = te + death_jitter
-    return ts, te, float(np.max(te)), float(np.min(ts))
-
-
-def bin_window(origin, present, rm_first_bin=0):
-    """(first_bin, n_bins) of literate_library.create_bins (:231-257): unit bins over np.arange(origin, present + 1), the
-    last one always dropped, the first one too with -rm_first_bin."""
-    if origin != np.floor(origin):
-        raise SystemExit("the first birth time (%r) is not an integer: the unit bins of create_bins would not be aligned with "
-                         "the integer bin edges K1 works on" % origin)
-    n_edges = len(np.arange(origin, present + 1))
-    n_bins = n_edges - 2
-    first = int(origin)
-    if rm_first_bin:
-        first, n_bins = first + 1, n_bins - 1
-    if n_bins < 1:
-        raise SystemExit("the time window holds no bin after dropping the last one")
-    return first, n_bins
+    def own(p):                                                       # trend_rate.py:34-38
+        p.add_argument('-trend_data', metavar='<path to trend file>', type=str, default="",
+                       help='Input trend file should be columns tab-separated with headers. No missing values.')
+        p.add_argument('-trend_index', type=int, help='Column of trend in trend file.', default=0, metavar=0)
+        p.add_argument('-const_B', type=_flag, help='F) Vary rates with trend T) Constant rates', default=False, metavar=False)
+        p.add_argument('-const_D', type=_flag, help='F) Vary rates with trend T) Constant rates', default=False, metavar=False)
+        p.add_argument('-no_death', type=_flag, help='F) Calculate death rate T) Likelihood based on births only', default=False, metavar=False)
+    return L.build_parser("trend_rate.py", own)
 
 
 def parse_trend_data(path, index, rm_first_bin=0):
@@ -130,64 +63,23 @@ def parse_trend_data(path, index, rm_first_bin=0):
     return trend
 
 
-class TrendChains:
+class TrendChains(L.ChainObject):
     """lr_trend_t: the per-bin table and a population of independent TrendRate chains on one device."""
+    PREFIX, STATE_DOUBLES = "trend", N.LR_TREND_STATE_DOUBLES
 
     def __init__(self, dev: E.Device, sp, ex, br, trend, n_chains, seed, const_birth=False, const_death=False, chain_id0=0,
                  rep_of_chain=None):
-        sp = np.ascontiguousarray(np.atleast_2d(sp), dtype=np.int64)
-        ex = np.ascontiguousarray(np.atleast_2d(ex), dtype=np.int64)
-        br = np.ascontiguousarray(np.atleast_2d(br), dtype=np.float64)
+        sp, ex, br, rep = self._inputs(sp, ex, br, rep_of_chain, n_chains)
         trend = np.ascontiguousarray(trend, dtype=np.float64)
         if not (sp.shape == ex.shape == br.shape) or trend.shape != (sp.shape[1],):
             raise ValueError("sp, ex, br must be [n_rep, n_bins] and trend [n_bins] (the reference fails to broadcast, trend_rate.py:82)")
         self.dev, self.n_chains, self.n_rep, self.n_bins = dev, int(n_chains), sp.shape[0], sp.shape[1]
-        rep = None
-        if rep_of_chain is not None:
-            rep = np.ascontiguousarray(rep_of_chain, dtype=np.int32)
-            if rep.shape != (self.n_chains,):
-                raise ValueError("rep_of_chain must have one entry per chain")
         t = C.c_void_p()
         N.check(dev.lib.lr_trend_create_host(dev.h, self.n_rep, self.n_bins, N.np_ptr(sp), N.np_ptr(ex), N.np_ptr(br), N.np_ptr(trend),
                                              int(bool(const_birth)), int(bool(const_death)), self.n_chains,
                                              C.c_uint64(int(seed) & (2**64 - 1)), int(chain_id0), N.np_ptr(rep), C.byref(t)),
                 "lr_trend_create_host")
-        self.t = t
-        self.rec_doubles = int(dev.lib.lr_trend_record_doubles(self.n_bins))
-
-    def close(self):
-        if getattr(self, "t", None):
-            self.dev.lib.lr_trend_destroy(self.t)
-            self.t = None
-
-    def __del__(self):
-        try:
-            self.close()
-        except Exception:
-            pass
-
-    def records_per_run(self, n_iter, sample_every):
-        return int(self.dev.lib.lr_trend_records_per_run(self.t, int(n_iter), int(sample_every)))
-
-    def run(self, n_iter, sample_every=0):
-        """n_iter iterations of every chain; returns records [n_samples, n_chains, 16 + 2 n_bins] (host) or None."""
-        if sample_every and sample_every > 0:
-            out = np.empty((self.records_per_run(n_iter, sample_every), self.n_chains, self.rec_doubles), dtype=np.float64)
-            N.check(self.dev.lib.lr_trend_run_host(self.t, int(n_iter), int(sample_every), N.np_ptr(out)), "lr_trend_run_host")
-            return out
-        N.check(self.dev.lib.lr_trend_run_host(self.t, int(n_iter), 0, None), "lr_trend_run_host")
-        return None
-
-    def run_device(self, n_iter, sample_every, records, stream=None):
-        """Asynchronous: `records` is a float64 CUDA tensor [n_samples, n_chains, rec_doubles] or None."""
-        st = C.c_void_p(None) if isinstance(stream, str) and stream == "handle" else E._stream_ptr(stream)
-        ptr = C.c_void_p(records.data_ptr()) if records is not None else None
-        N.check(self.dev.lib.lr_trend_run(self.t, int(n_iter), int(sample_every) if records is not None else 0, ptr, st), "lr_trend_run")
-
-    def state(self):
-        out = np.empty((self.n_chains, N.LR_TREND_STATE_DOUBLES), dtype=np.float64)
-        N.check(self.dev.lib.lr_trend_state_host(self.t, N.np_ptr(out)), "lr_trend_state_host")
-        return out
+        self._created(t)
 
     def evaluate(self, params, rep=None, kind=None, on=None, draw=None):
         """Parity entry point: likelihood, prior, rates and adequacy of explicit parameter vectors [n, 6], optionally after one
@@ -245,41 +137,17 @@ def run(args, device=None):
     no_death = bool(args.no_death)
     const_birth = bool(args.const_B)
     const_death = True if no_death else bool(args.const_D)            # :42-45
-    if args.seed == -1:                                               # set_seed, literate_library.py:282-288
-        if world > 1:
-            raise SystemExit("give -seed explicitly when running on several GPUs (every rank must use the same one)")
-        seed = int(np.random.randint(0, 9999))
-    else:
-        seed = args.seed
-    if args.chains < max(1, world):
-        raise SystemExit("-chains must be >= 1 and at least the number of GPUs")
+    seed = L.seed_and_chains(args, world)
     if const_birth and const_death:
         raise SystemExit("-const_B with -const_D / -no_death leaves the additive move without a parameter: the reference stops "
                          "with ValueError in np.random.binomial (trend_rate.py:129-134, :168)")
-    # -d may name a DIRECTORY of tables (stochastic imputations of one data set): one replicate each, common window
-    if os.path.isdir(args.d):
-        tables = sorted(f for f in glob.glob(os.path.join(args.d, "*")) if os.path.isfile(f) and f.lower().endswith((".tsv", ".txt"))
-                        and os.path.abspath(f) != os.path.abspath(args.trend_data))
-        if not tables:
-            raise SystemExit("no .tsv/.txt table in " + args.d)
-    else:
-        tables = [args.d]
-    parsed = [parse_ts_te(f, args.TBP, args.first_year, args.last_year, args.death_jitter) for f in tables]
-    n_tab = len(parsed)
-    if args.chains == 1 and n_tab > 1:
-        args.chains = n_tab
-    if args.chains % n_tab:
-        raise SystemExit("-chains must be a multiple of the number of tables (%d)" % n_tab)
-    present, origin = max(p[2] for p in parsed), min(p[3] for p in parsed)
+    tables, ts, te, present, origin = L.read_tables(args, exclude=args.trend_data)
+    n_tab = len(tables)
     first_bin, n_bins = bin_window(origin, present, args.rm_first_bin)
     trend = parse_trend_data(args.trend_data, args.trend_index, args.rm_first_bin)
     if len(trend) != n_bins:
         raise SystemExit("the trend table must hold one row per unit bin from the first birth time plus one (%d rows); it has %d"
                          % (n_bins + 1 + (1 if args.rm_first_bin else 0), len(trend) + 1 + (1 if args.rm_first_bin else 0)))
-    n_max = max(len(p[0]) for p in parsed)
-    ts = np.full((n_tab, n_max), np.nan); te = np.full((n_tab, n_max), np.nan)      # NaN rows carry no event and no time at risk
-    for i, p in enumerate(parsed):
-        ts[i, :len(p[0])], te[i, :len(p[1])] = p[0], p[1]
     dev = device if device is not None else E.Device(local_rank if world > 1 else args.device)
     t0 = time.time()
     stats = dev.bin_stats(ts, te, first_bin=first_bin, n_bins=n_bins, death_jitter=args.death_jitter)
@@ -302,25 +170,8 @@ def run(args, device=None):
         w.writerow(header(n_bins))
         paths.append(path); files.append(fh); writers.append(w)
 
-    s_freq = max(1, args.s)
-    max_rec = max(1, (256 << 20) // (n_local * chains.rec_doubles * 8))            # at most ~256 MB of records per launch
-    per_launch = max(s_freq, min(max_rec * s_freq, 4_000_000) // s_freq * s_freq)
-    done = 0
-    t_run = time.time()
-    while done < args.n:
-        n_it = min(per_launch, args.n - done)
-        recs = chains.run(n_it, s_freq)
-        done += n_it
-        for r in range(recs.shape[0]):
-            for k in range(n_local):
-                writers[k].writerow(record_row(recs[r, k], n_bins))
-            if not args.quiet:
-                print(int(recs[r, 0, 0]), recs[r, 0, 1], recs[r, 0, 5:11])       # :187
-        for fh in files:
-            fh.flush()
-    t_run = time.time() - t_run
-    for fh in files:
-        fh.close()
+    t_run = L.sample_and_write(chains, args.n, args.s, files, writers, lambda rec: record_row(rec, n_bins),
+                               lambda rec: print(int(rec[0]), rec[1], rec[5:11]), args.quiet)       # :187
     if not args.quiet:
         acc = chains.state()[:, 10].sum() / max(1, n_local * args.n)
         print("literate_b200: %d TrendRate chains x %d iterations in %.3f s (%.3g it/s, acceptance %.3f); binning %.4f s"

@@ -9,7 +9,7 @@ import pytest
 
 from oracle import ddrate_oracle as D
 from literate_b200 import ddrate as DD
-from literate_b200 import trend as TR
+from literate_b200 import library as L
 from test_oracle_ddrate_golden import DG, _flag, _jobs, setup_job
 
 
@@ -56,8 +56,8 @@ def test_rows_from_records_are_byte_identical_to_the_reference_log(tag, tmp_path
 def test_window_and_flags(tmp_path):
     job = _jobs()[0]
     data, S, gbins = setup_job(job, tmp_path)
-    ts, te, present, origin = TR.parse_ts_te(data)
-    first, nb = TR.bin_window(origin, present, 0)
+    ts, te, present, origin = L.parse_ts_te(data)
+    first, nb = L.bin_window(origin, present, 0)
     assert (first, nb) == (S.origin, S.n) and present == S.present
     a = DD.build_parser().parse_args(["-d", "x.tsv"])
     assert (a.m_birth, a.m_death, a.n, a.s, a.seed, a.genre_times, a.chains) == (2, 2, 10000000, 1000, -1, "", 1)

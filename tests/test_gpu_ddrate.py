@@ -13,7 +13,7 @@ import pytest
 
 from oracle import ddrate_oracle as D
 from literate_b200 import ddrate as DD
-from literate_b200 import trend as TR
+from literate_b200 import library as L
 from test_oracle_ddrate_golden import DG, _jobs, stage
 
 pytestmark = pytest.mark.gpu
@@ -27,10 +27,10 @@ def _job(tag):
 def _setup(device, tmp_path, tag="ex_g_mddn", mb=3, md=2, n_chains=8, seed=1, rm=0):
     job = _job(tag)
     data, genre = stage(job, tmp_path)
-    ts, te, present, origin = TR.parse_ts_te(data)
-    first, nb = TR.bin_window(origin, present, rm)
+    ts, te, present, origin = L.parse_ts_te(data)
+    first, nb = L.bin_window(origin, present, rm)
     st = device.bin_stats(ts, te, first_bin=first, n_bins=nb)
-    gts, gte, _, _ = TR.parse_ts_te(genre)
+    gts, gte, _, _ = L.parse_ts_te(genre)
     bins = D.create_bins(origin, present, ts, te, rm)
     assert np.array_equal(st.sp[0], bins.n_spec) and np.array_equal(st.ex[0], bins.n_exti) and np.array_equal(st.br[0], bins.dt)
     S = D.Setup(bins, mb, md, gts, gte)
@@ -119,7 +119,7 @@ def test_bin_counts_from_one_to_two_hundred(device, nb, mb, md):
 
 @pytest.mark.parametrize("nb,mb,md", [(65, 3, 2), (100, 2, 1), (129, 1, 2), (200, 3, 2), (200, 0, 0), (300, 3, 1)])
 def test_wide_build_gives_the_chains_of_the_one_warp_build(device, nb, mb, md, monkeypatch):
-    """More than 64 bins and few chains: 2 or 4 warps share a chain's bins (k7_dd_wide_kernel), exchange the per-bin terms and add
+    """More than 64 bins and few chains: 2 or 4 warps share a chain's bins (k7_dd_kernel<2> and <4>), exchange the per-bin terms and add
     them in the one-warp kernel's order -- records and final states identical, bit for bit, over split launches."""
     rng = np.random.default_rng(77 + nb + mb)
     t = np.arange(nb)
@@ -307,9 +307,9 @@ def test_replicates_and_directory_of_imputations(device, tmp_path):
     paths = DD.run(DD.build_parser().parse_args(["-d", d, "-m_birth", "3", "-g", genre, "-n", "1001", "-s", "500", "-seed", "3", "-chains", "4",
                                                  "-quiet", "1"]), device=device)
     assert [os.path.basename(p) for p in paths] == ["imp_%d_%d_GLDDN_MDDN.log" % (k % 2, 3 + k // 2) for k in range(4)]
-    gts, gte, _, _ = TR.parse_ts_te(genre)
+    gts, gte, _, _ = L.parse_ts_te(genre)
     for k, p in enumerate(paths):
-        ts, te, present, origin = TR.parse_ts_te(os.path.join(d, "imp_%d.tsv" % (k % 2)))
+        ts, te, present, origin = L.parse_ts_te(os.path.join(d, "imp_%d.tsv" % (k % 2)))
         S = D.Setup(D.create_bins(origin, present, ts, te), 3, 2, gts, gte)
         got = np.loadtxt(p, skiprows=1)
         assert got.shape[0] == 3

@@ -12,6 +12,7 @@ import numpy as np
 import pytest
 
 from oracle import trendrate_oracle as T
+from literate_b200 import library as L
 from literate_b200 import trend as TR
 from test_oracle_trend_golden import TG, _jobs, stage
 
@@ -27,8 +28,8 @@ def _setup(device, tmp_path, tag="ex_ramp", n_chains=8, seed=1, const_birth=Fals
     job = _job(tag)
     data, trend_path = stage(job, tmp_path)
     idx = int(job["args"][job["args"].index("-trend_index") + 1])
-    ts, te, present, origin = TR.parse_ts_te(data, death_jitter=jitter)
-    first, nb = TR.bin_window(origin, present, rm)
+    ts, te, present, origin = L.parse_ts_te(data, death_jitter=jitter)
+    first, nb = L.bin_window(origin, present, rm)
     st = device.bin_stats(ts, te, first_bin=first, n_bins=nb, death_jitter=jitter)
     trend = TR.parse_trend_data(trend_path, idx, rm)
     ots, ote, opresent, oorigin = T.parse_ts_te(data, death_jitter=jitter)

@@ -8,6 +8,7 @@ import numpy as np
 import pytest
 
 from oracle import trendrate_oracle as T
+from literate_b200 import library as L
 from literate_b200 import trend as TR
 from test_oracle_trend_golden import TG, _flag, _jobs, setup_job, stage
 
@@ -17,11 +18,11 @@ def test_parsing_and_window_equal_the_oracle(job, tmp_path):
     a = job["args"]
     data, trend_path = stage(job, tmp_path)
     rm, jit = _flag(a, "-rm_first_bin", 0.0), _flag(a, "-death_jitter", 0.5)
-    ts, te, present, origin = TR.parse_ts_te(data, death_jitter=jit)
+    ts, te, present, origin = L.parse_ts_te(data, death_jitter=jit)
     ots, ote, opresent, oorigin = T.parse_ts_te(data, death_jitter=jit)
     assert np.array_equal(ts, ots) and np.array_equal(te, ote) and (present, origin) == (opresent, oorigin)
     bins = T.create_bins(oorigin, opresent, ots, ote, rm)
-    first, nb = TR.bin_window(origin, present, rm)
+    first, nb = L.bin_window(origin, present, rm)
     assert nb == bins.n_bins and first == bins.origin
     idx = _flag(a, "-trend_index", 0, int)
     assert np.array_equal(TR.parse_trend_data(trend_path, idx, rm), T.normalise_trend(T.read_trend_column(trend_path, idx), rm))
@@ -58,4 +59,4 @@ def test_flags_follow_the_reference_parser():
     assert a.const_B is True and a.no_death is True and a.const_D is False      # argparse type=bool: any non-empty string
     assert (a.n, a.s, a.p, a.seed, a.death_jitter, a.trend_index, a.chains) == (10000000, 1000, 1000, -1, .5, 0, 1)
     with pytest.raises(SystemExit):
-        TR.bin_window(1994.25, 2017.5)
+        L.bin_window(1994.25, 2017.5)
