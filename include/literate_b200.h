@@ -344,7 +344,8 @@ int lr_trend_destroy(lr_trend_t t);
 /* One sample record = lr_trend_record_doubles(n_bins) = LR_TREND_REC_HEAD + 2 n_bins doubles (the row of :191):
  *   [0] iteration  [1] likelihood  [2] likelihood_birth  [3] likelihood_death  [4] prior
  *   [5..10] l_min, m_min, alpha, beta, delta, gamma  [11..13] adequacy (coeff, r2, gelman_r2)
- *   [14] proposals accepted so far  [15] reserved  [16 .. 16+n_bins) birth rates  [16+n_bins .. 16+2 n_bins) death rates */
+ *   [14] proposals accepted so far  [15] inverse temperature beta of the chain (1 unless tempered, lr_trend_set_beta_host)
+ *   [16 .. 16+n_bins) birth rates  [16+n_bins .. 16+2 n_bins) death rates */
 #define LR_TREND_REC_HEAD 16
 int64_t lr_trend_record_doubles(int32_t n_bins);
 /* A record is written after every iteration `it` with it % sample_every == 0 (:184: the sample follows the accept step, so
@@ -363,6 +364,20 @@ int lr_trend_eval_host(lr_trend_t t, int32_t n, const int32_t* rep, const double
  * prior, iterations done, proposals accepted, replicate */
 #define LR_TREND_STATE_DOUBLES 12
 int lr_trend_state_host(lr_trend_t t, double* h_state);
+/* Tempered ladders, as lr_chains_set_beta_host .. lr_chains_swap_step (new; the reference has no tempering).  A chain at
+ * beta = 1 is the reference's chain; a heated chain raises the likelihood (not the prior) to the power beta < 1.  Swap rounds
+ * exchange temperatures between neighbours of a ladder of `ladder` consecutive GLOBAL chain ids by the rule of
+ * lr_chains_swap_apply; the exchanged likelihood is the stored one of the current state.
+ *   set_beta_host: beta[n_chains] (HOST), each in [0, 1]; chains start at 1.
+ *   swap_info / swap_apply: as lr_chains_swap_info / lr_chains_swap_apply, async on `stream`.
+ *   swap_step: one round on the handle's stream for a shard that holds whole ladders, each on a single replicate.
+ *   temper_host: current beta[n_chains] and swaps proposed / accepted [n_chains][2] (HOST; either may be NULL). */
+int lr_trend_set_beta_host(lr_trend_t t, const double* h_beta);
+int lr_trend_swap_info(lr_trend_t t, double* d_info, void* stream);
+int lr_trend_swap_apply(lr_trend_t t, const double* d_info_all, int64_t n_all, int64_t first, int32_t ladder, uint64_t round,
+                        void* stream);
+int lr_trend_swap_step(lr_trend_t t, int32_t ladder, uint64_t round);
+int lr_trend_temper_host(lr_trend_t t, double* h_beta, int64_t* h_swaps);
 
 /* ---------------------------------------------------------------- DDRate (SURVEY 8 f-4): diversity-dependent rates on the same statistics
  *
@@ -389,7 +404,7 @@ int lr_dd_destroy(lr_dd_t t);
  *   [0] iteration  [1] likelihood (sum of the three terms; the genre term is the constant 1 unless m_birth = 3, :84)
  *   [2] likelihood_birth  [3] likelihood_death  [4] prior  [5..15] the 11 parameters as the chain holds them (x0 relative to
  *   origin, L without div_0: the log row adds them, :278-279)  [16] genre term  [17..19] adequacy  [20] proposals accepted
- *   [21..23] reserved  then birth rates, death rates, niche, niche fraction, n_bins each */
+ *   [21] inverse temperature beta of the chain (1 unless tempered, lr_dd_set_beta_host)  [22..23] reserved  then birth rates, death rates, niche, niche fraction, n_bins each */
 #define LR_DD_REC_HEAD 24
 int64_t lr_dd_record_doubles(int32_t n_bins);
 int64_t lr_dd_records_per_run(lr_dd_t t, int64_t n_iter, int64_t sample_every);
@@ -407,6 +422,12 @@ int lr_dd_eval_host(lr_dd_t t, int32_t n, const int32_t* rep, const double* para
  * the four cached genre statistics, replicate, 2 reserved */
 #define LR_DD_STATE_DOUBLES 24
 int lr_dd_state_host(lr_dd_t t, double* h_state);
+/* Tempered ladders: as the lr_trend_* calls of the same names; the tempered likelihood includes the genre term. */
+int lr_dd_set_beta_host(lr_dd_t t, const double* h_beta);
+int lr_dd_swap_info(lr_dd_t t, double* d_info, void* stream);
+int lr_dd_swap_apply(lr_dd_t t, const double* d_info_all, int64_t n_all, int64_t first, int32_t ladder, uint64_t round, void* stream);
+int lr_dd_swap_step(lr_dd_t t, int32_t ladder, uint64_t round);
+int lr_dd_temper_host(lr_dd_t t, double* h_beta, int64_t* h_swaps);
 
 #ifdef __cplusplus
 }

@@ -34,8 +34,10 @@ EXPORTS = [
     "lr_chains_swap_info", "lr_chains_swap_apply", "lr_chains_swap_step", "lr_summarize_records", "lr_marginal_rates",
     "lr_trend_create", "lr_trend_create_host", "lr_trend_destroy", "lr_trend_record_doubles", "lr_trend_records_per_run",
     "lr_trend_run", "lr_trend_run_host", "lr_trend_eval_host", "lr_trend_state_host",
+    "lr_trend_set_beta_host", "lr_trend_swap_info", "lr_trend_swap_apply", "lr_trend_swap_step", "lr_trend_temper_host",
     "lr_dd_create", "lr_dd_create_host", "lr_dd_destroy", "lr_dd_record_doubles", "lr_dd_records_per_run",
     "lr_dd_run", "lr_dd_run_host", "lr_dd_eval_host", "lr_dd_state_host",
+    "lr_dd_set_beta_host", "lr_dd_swap_info", "lr_dd_swap_apply", "lr_dd_swap_step", "lr_dd_temper_host",
 ]
 
 
@@ -137,6 +139,12 @@ def load(build_if_missing=False):
     sig("lr_dd_run_host", C.c_int, vp, i64, i64, vp)
     sig("lr_dd_eval_host", C.c_int, vp, i32, *([vp] * 12))
     sig("lr_dd_state_host", C.c_int, vp, vp)
+    for p in ("trend", "dd"):
+        sig("lr_%s_set_beta_host" % p, C.c_int, vp, vp)
+        sig("lr_%s_swap_info" % p, C.c_int, vp, vp, vp)
+        sig("lr_%s_swap_apply" % p, C.c_int, vp, vp, i64, i64, i32, u64, vp)
+        sig("lr_%s_swap_step" % p, C.c_int, vp, i32, u64)
+        sig("lr_%s_temper_host" % p, C.c_int, vp, vp, vp)
     if lib.lr_abi_version() != LR_ABI_VERSION:
         raise NativeError("libliterate_b200.so ABI version mismatch; rebuild with `python -m literate_b200.build --force`")
     _lib = lib

@@ -1103,58 +1103,19 @@ __global__ void k3_swap_info_kernel(const ChainState* st, int n_chains, double* 
     if (lane == 0) { info[2 * chain] = d.C + L.lik + M.lik; info[2 * chain + 1] = S->beta; }
 }
 
-// One swap round.  Chains are grouped into ladders of `ladder` consecutive GLOBAL chain ids; within a ladder the
-// members are ordered by temperature and neighbours (2p + parity, 2p + 1 + parity) exchange their TEMPERATURES with
-// probability min(1, exp((beta_i - beta_j)(lik_j - lik_i))).  Every rank holding a member of a ladder recomputes the
-// whole ladder's decisions from the gathered (lik, beta) table and a Philox draw keyed by (seed, ladder, round, pair),
-// so the outcome is identical everywhere and no state crosses the interconnect.
+// One swap round (lr_swap_round): beta and the swap counters of K3's chain state
 __global__ void k3_swap_apply_kernel(ChainState* st, int n_local, const double* __restrict__ info_all, long long table_first,
                                      long long n_all, long long first, int ladder, unsigned long long round, uint32_t k0, uint32_t k1) {
     const int lane = threadIdx.x & 31;
     const int local = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) >> 5);
     if (local >= n_local) return;
-    const long long g = first + local;
-    const long long lad = g / ladder;
-    const int me = (int)(g - lad * ladder);
-    const long long m = lad * ladder + lane;
-    const bool on = lane < ladder && m >= table_first && m < table_first + n_all;     // table row of global chain m: m - table_first
-    const double lik = on ? info_all[2 * (m - table_first)] : 0.0;
-    const double beta = on ? info_all[2 * (m - table_first) + 1] : -1.0;
-    // rank by temperature: 0 = coldest (largest beta); ties broken by position
-    int rank = 0;
-    for (int k = 0; k < ladder; ++k) {
-        const double bk = __shfl_sync(0xffffffffu, beta, k);
-        if (bk > beta || (bk == beta && k < lane)) rank++;
-    }
-    const int parity = (int)(round & 1ull);
-    const int q = rank - parity;
-    int partner_rank = -1;
-    if (on && q >= 0) {
-        partner_rank = (q ^ 1) + parity;
-        if (partner_rank >= ladder) partner_rank = -1;
-    }
-    int partner = -1;
-    for (int k = 0; k < ladder; ++k) {
-        const int rk = __shfl_sync(0xffffffffu, rank, k);
-        const bool onk = __shfl_sync(0xffffffffu, (int)on, k) != 0;
-        if (onk && rk == partner_rank) partner = k;
-    }
-    const double lik_p = __shfl_sync(0xffffffffu, lik, partner < 0 ? 0 : partner);
-    const double beta_p = __shfl_sync(0xffffffffu, beta, partner < 0 ? 0 : partner);
-    bool accept = false;
-    if (partner >= 0) {
-        const int pair = (rank < partner_rank ? rank : partner_rank);
-        const Philox4 r = philox4x32_10((uint32_t)round, (uint32_t)(round >> 32), (uint32_t)pair | (0x5157u << 16), (uint32_t)lad, k0, k1 ^ 0x7e3a9u);
-        const double u = u01(r.x, r.y);
-        accept = log(u) <= (beta - beta_p) * (lik_p - lik);
-    }
-    if (lane == me) {
+    lr_swap_round(info_all, table_first, n_all, first + local, ladder, round, k0, k1, lane, [&](bool paired, bool accept, double beta_p) {
         ChainState* S = st + local;
-        if (partner >= 0) {
+        if (paired) {
             S->counters[8] += 1;
             if (accept) { S->counters[9] += 1; S->beta = beta_p; }
         }
-    }
+    });
 }
 
 int upload_lnfact() {
@@ -1668,21 +1629,12 @@ extern "C" int lr_chains_swap_info(lr_chains_t c, double* d_info, void* stream) 
 
 static int swap_apply(lr_chains_t c, const double* d_info_all, int64_t table_first, int64_t n_all, int64_t first, int32_t ladder,
                       uint64_t round, void* stream, const char* who) {
-    LR_REQUIRE(c && d_info_all, "%s: null pointer", who);
-    LR_REQUIRE(ladder >= 2 && ladder <= 32, "%s: ladder size must be 2..32", who);
-    LR_REQUIRE(first >= table_first && first + c->n_chains <= table_first + n_all,
-               "%s: this shard [first, first + n_chains) lies outside the gathered table", who);
-    lr_handle_t h = c->h;
-    LR_CUDA(cudaSetDevice(h->device));
-    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-    { int rc0 = lr_order(h, &c->last, st); if (rc0 != LR_OK) return rc0; }
-    int threads;
-    const int blocks = lr_chain_grid(c->n_chains, threads);
-    k3_swap_apply_kernel<<<blocks, threads, 0, st>>>(c->st, c->n_chains, d_info_all, table_first, n_all, first, ladder, round,
-                                                     (uint32_t)c->seed, (uint32_t)(c->seed >> 32));
-    LR_CUDA(cudaGetLastError());
-    h->launches += 1;
-    return LR_OK;
+    LR_REQUIRE(c, "%s: null pointer", who);
+    return lr_swap_apply(c->h, &c->last, c->n_chains, d_info_all, table_first, n_all, first, ladder, stream, who,
+                         [&](int blocks, int threads, cudaStream_t st) {
+                             k3_swap_apply_kernel<<<blocks, threads, 0, st>>>(c->st, c->n_chains, d_info_all, table_first, n_all, first,
+                                                                              ladder, round, (uint32_t)c->seed, (uint32_t)(c->seed >> 32));
+                         });
 }
 
 extern "C" int lr_chains_swap_apply(lr_chains_t c, const double* d_info_all, int64_t n_all, int64_t first, int32_t ladder,
@@ -1692,14 +1644,11 @@ extern "C" int lr_chains_swap_apply(lr_chains_t c, const double* d_info_all, int
 
 extern "C" int lr_chains_swap_step(lr_chains_t c, int32_t ladder, uint64_t round) {
     LR_REQUIRE(c != nullptr, "lr_chains_swap_step: null chains");
-    LR_REQUIRE(ladder >= 2 && c->chain_id0 % ladder == 0 && c->n_chains % ladder == 0,
-               "lr_chains_swap_step: the shard must hold whole ladders (chain_id0 and n_chains multiples of the ladder size); "
-               "use lr_chains_swap_info + an all-gather + lr_chains_swap_apply for ladders that span devices");
-    lr_handle_t h = c->h;
-    int rc = lr_ws_acquire(h, (size_t)c->n_chains * 16, h->stream);
-    if (rc != LR_OK) return rc;
-    rc = lr_chains_swap_info(c, (double*)h->ws, h->stream);
-    if (rc != LR_OK) return rc;
     // ladders and their Philox keys are numbered by GLOBAL chain id, so the outcome does not depend on the sharding
-    return swap_apply(c, (const double*)h->ws, c->chain_id0, c->n_chains, c->chain_id0, ladder, round, h->stream, "lr_chains_swap_step");
+    return lr_swap_step(c->h, c->chain_id0, c->n_chains, ladder, nullptr, "lr_chains",
+                        [&](double* d_info) { return lr_chains_swap_info(c, d_info, c->h->stream); },
+                        [&](const double* d_info) {
+                            return swap_apply(c, d_info, c->chain_id0, c->n_chains, c->chain_id0, ladder, round, c->h->stream,
+                                              "lr_chains_swap_step");
+                        });
 }

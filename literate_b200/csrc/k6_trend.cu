@@ -34,6 +34,8 @@ struct TrendChain {
     long long accepted;
     unsigned chain;        // global chain id (Philox key)
     int rep;
+    double beta;           // inverse temperature of a tempered ladder (1: the reference's chain)
+    long long swaps[2];    // temperature swaps proposed, accepted
 };
 
 struct lr_trend_s {
@@ -45,6 +47,8 @@ struct lr_trend_s {
     double* cst;                   // device [n_rep][2]: sum x, sum x^2 of the empirical rates (adequacy)
     int n_chains;
     uint64_t seed;
+    int64_t chain_id0;             // global id of chain 0 (ladders are numbered by global id)
+    int* rep_of_chain;             // host [n_chains]: replicate of every chain (swap_step refuses ladders that mix replicates)
     TrendChain* st;                // device [n_chains]
     double f_mult[TR_NPAR], f_norm[TR_NPAR];
 };
@@ -221,15 +225,15 @@ __device__ __forceinline__ void trend_adequacy(const TrendView& v, const double*
 }
 
 // record: [0] it [1] likelihood [2] likelihood_birth [3] likelihood_death [4] prior [5..10] parameters [11..13] adequacy
-//         [14] accepted so far [15] reserved [16 .. 16+nb) birth rates [16+nb .. 16+2nb) death rates
+//         [14] accepted so far [15] beta [16 .. 16+nb) birth rates [16+nb .. 16+2nb) death rates
 __device__ __forceinline__ void trend_record(double* rec, const TrendView& v, const double* p, double mine, double likB, double likD,
-                                             long long it, long long accepted, int lane) {
+                                             long long it, long long accepted, double beta, int lane) {
     double adq[3];
     trend_adequacy(v, p, lane, adq);
     const double prior = warp_sum(trend_prior_term(lane, mine));
     if (lane == 0) {
         rec[0] = (double)it; rec[1] = likB + likD; rec[2] = likB; rec[3] = likD; rec[4] = prior;
-        rec[11] = adq[0]; rec[12] = adq[1]; rec[13] = adq[2]; rec[14] = (double)accepted; rec[15] = 0.0;
+        rec[11] = adq[0]; rec[12] = adq[1]; rec[13] = adq[2]; rec[14] = (double)accepted; rec[15] = beta;
     }
 #pragma unroll
     for (int k = 0; k < TR_NPAR; ++k)
@@ -279,6 +283,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W, W == 1 ? 4 : 2) k6_tren
     pc.d = v.const_d ? 1.0 : exp(p[5] * v.lnT0);
     long long it = S->it, accepted = S->accepted;
     const long long it_end = it + P.n_iter;
+    const double beta = S->beta;                           // read by every warp before warp 0 may rewrite the state
     // this lane's Bernoulli probabilities (lanes >= 6: never on)
     const double fm = lane < TR_NPAR ? P.fd_mult[lane] : 0.0, fn = lane < TR_NPAR ? P.fd_norm[lane] : 0.0;
     long long next_sample = (it + P.sample_every - 1) / P.sample_every * P.sample_every;
@@ -309,7 +314,8 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W, W == 1 ? 4 : 2) k6_tren
         double* tB = terms + (size_t)(it & 1) * 2 * P.nbp;
         double* tD = tB + P.nbp;
         trend_lik<W>(v, q, lane, (touched & 0x15u) != 0, (touched & 0x2au) != 0, (touched & 0x10u) != 0, (touched & 0x20u) != 0, npc, nB, nD, hp, tB, tD);
-        const double x = ((nB + nD) - (likB + likD)) + hp;
+        // tempered: only the likelihood is raised to the power beta (1.0 * d == d: at beta = 1 this is the untempered test)
+        const double x = beta * ((nB + nD) - (likB + likD)) + hp;
         if (it == 0 || mh_accept_gt(x, u_acc)) {                            // trend_rate.py:176
 #pragma unroll
             for (int k = 0; k < TR_NPAR; ++k) p[k] = q[k];
@@ -321,7 +327,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W, W == 1 ? 4 : 2) k6_tren
             if (P.records && (W == 1 || w == 0)) {
                 // W > 1: re-reading the view here keeps its constants out of registers across the loop (142, not 146)
                 const TrendView v0 = W == 1 ? v : trend_view(P.tab, P.cst, S->rep, P.nb, P.nbp, P.const_b, P.const_d, lane);
-                trend_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v0, p, mine, likB, likD, it, accepted, lane);
+                trend_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v0, p, mine, likB, likD, it, accepted, beta, lane);
             }
             ++rec_idx;
             next_sample += P.sample_every;
@@ -355,7 +361,34 @@ __global__ void k6_init_kernel(TrendChain* st, int n_chains, const int* rep_of_c
     if (lane == 0) {
         st[c].likB = likB; st[c].likD = likD; st[c].prior = pr; st[c].it = 0; st[c].accepted = 0;
         st[c].chain = (unsigned)(chain_id0 + c); st[c].rep = rep;
+        st[c].beta = 1.0; st[c].swaps[0] = 0; st[c].swaps[1] = 0;
     }
+}
+
+// ---- tempered ladders (new: the reference has no tempering, SURVEY A-15; the swap rule is lr_swap_round, shared with K3)
+__global__ void k6_set_beta_kernel(TrendChain* st, int n, const double* beta) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) st[i].beta = beta[i];
+}
+
+// (likelihood, beta) of every chain, as stored: the untempered likelihood of the current state
+__global__ void k6_swap_info_kernel(const TrendChain* st, int n, double* __restrict__ info) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) { info[2 * i] = st[i].likB + st[i].likD; info[2 * i + 1] = st[i].beta; }
+}
+
+__global__ void k6_swap_apply_kernel(TrendChain* st, int n_local, const double* __restrict__ info_all, long long table_first,
+                                     long long n_all, long long first, int ladder, unsigned long long round, uint32_t k0, uint32_t k1) {
+    const int lane = threadIdx.x & 31;
+    const int local = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) >> 5);
+    if (local >= n_local) return;
+    lr_swap_round(info_all, table_first, n_all, first + local, ladder, round, k0, k1, lane, [&](bool paired, bool accept, double beta_p) {
+        TrendChain* S = st + local;
+        if (paired) {
+            S->swaps[0] += 1;
+            if (accept) { S->swaps[1] += 1; S->beta = beta_p; }
+        }
+    });
 }
 
 // per-replicate table: statistics as doubles, ln(trend), empirical rates and their sums
@@ -456,7 +489,9 @@ extern "C" int lr_trend_create(lr_handle_t h, int32_t n_rep, int32_t n_bins, con
     memset(t, 0, sizeof(*t));
     t->last.s = st; t->last.valid = 1;
     t->h = h; t->n_rep = n_rep; t->n_bins = n_bins; t->nbp = (n_bins + 3) & ~3;
-    t->const_b = const_birth != 0; t->const_d = const_death != 0; t->n_chains = n_chains; t->seed = seed;
+    t->const_b = const_birth != 0; t->const_d = const_death != 0; t->n_chains = n_chains; t->seed = seed; t->chain_id0 = chain_id0;
+    t->rep_of_chain = new int[n_chains];
+    for (int i = 0; i < n_chains; ++i) t->rep_of_chain[i] = h_rep_of_chain ? h_rep_of_chain[i] : 0;
     move_weights(t->const_b, t->const_d, t->f_mult, t->f_norm);
     const size_t tab_bytes = (size_t)n_rep * TR_ROWS * t->nbp * sizeof(double);
     cudaError_t e = cudaMallocAsync((void**)&t->tab, tab_bytes, st);
@@ -507,6 +542,7 @@ extern "C" int lr_trend_destroy(lr_trend_t t) {
     if (t->tab) cudaFreeAsync(t->tab, t->h->stream);
     if (t->cst) cudaFreeAsync(t->cst, t->h->stream);
     if (t->st) cudaFreeAsync(t->st, t->h->stream);
+    delete[] t->rep_of_chain;
     delete t;
     return LR_OK;
 }
@@ -618,4 +654,48 @@ extern "C" int lr_trend_state_host(lr_trend_t t, double* h_state) {
     }
     delete[] tmp;
     return LR_OK;
+}
+
+extern "C" int lr_trend_set_beta_host(lr_trend_t t, const double* h_beta) {
+    LR_REQUIRE(t && h_beta, "lr_trend_set_beta_host: null pointer");
+    return lr_set_beta(t->h, &t->last, t->n_chains, h_beta, "lr_trend_set_beta_host", [&](const double* d_beta, cudaStream_t st) {
+        k6_set_beta_kernel<<<(t->n_chains + 127) / 128, 128, 0, st>>>(t->st, t->n_chains, d_beta);
+    });
+}
+
+extern "C" int lr_trend_swap_info(lr_trend_t t, double* d_info, void* stream) {
+    LR_REQUIRE(t && d_info, "lr_trend_swap_info: null pointer");
+    return lr_launch_ordered(t->h, &t->last, stream, [&](cudaStream_t st) {
+        k6_swap_info_kernel<<<(t->n_chains + 127) / 128, 128, 0, st>>>(t->st, t->n_chains, d_info);
+    });
+}
+
+static int trend_swap_apply(lr_trend_t t, const double* d_info_all, int64_t table_first, int64_t n_all, int64_t first, int32_t ladder,
+                            uint64_t round, void* stream, const char* who) {
+    LR_REQUIRE(t, "%s: null pointer", who);
+    return lr_swap_apply(t->h, &t->last, t->n_chains, d_info_all, table_first, n_all, first, ladder, stream, who,
+                         [&](int blocks, int threads, cudaStream_t st) {
+                             k6_swap_apply_kernel<<<blocks, threads, 0, st>>>(t->st, t->n_chains, d_info_all, table_first, n_all, first,
+                                                                              ladder, round, (uint32_t)t->seed, (uint32_t)(t->seed >> 32));
+                         });
+}
+
+extern "C" int lr_trend_swap_apply(lr_trend_t t, const double* d_info_all, int64_t n_all, int64_t first, int32_t ladder, uint64_t round,
+                                   void* stream) {
+    return trend_swap_apply(t, d_info_all, 0, n_all, first, ladder, round, stream, "lr_trend_swap_apply");
+}
+
+extern "C" int lr_trend_swap_step(lr_trend_t t, int32_t ladder, uint64_t round) {
+    LR_REQUIRE(t != nullptr, "lr_trend_swap_step: null chains");
+    return lr_swap_step(t->h, t->chain_id0, t->n_chains, ladder, t->rep_of_chain, "lr_trend",
+                        [&](double* d_info) { return lr_trend_swap_info(t, d_info, t->h->stream); },
+                        [&](const double* d_info) {
+                            return trend_swap_apply(t, d_info, t->chain_id0, t->n_chains, t->chain_id0, ladder, round, t->h->stream,
+                                                    "lr_trend_swap_step");
+                        });
+}
+
+extern "C" int lr_trend_temper_host(lr_trend_t t, double* h_beta, int64_t* h_swaps) {
+    LR_REQUIRE(t != nullptr, "lr_trend_temper_host: null chains");
+    return lr_temper_host(t->h, &t->last, t->st, t->n_chains, h_beta, h_swaps, "lr_trend_temper_host");
 }

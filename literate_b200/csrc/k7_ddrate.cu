@@ -46,6 +46,8 @@ struct DDChain {
     long long it, accepted;
     unsigned chain;
     int rep;
+    double beta;           // inverse temperature of a tempered ladder (1: the reference's chain)
+    long long swaps[2];    // temperature swaps proposed, accepted
 };
 
 struct lr_dd_s {
@@ -58,6 +60,8 @@ struct lr_dd_s {
     double* genre;         // device [2][n_genre] (ts, te) or null
     int n_chains;
     uint64_t seed;
+    int64_t chain_id0;     // global id of chain 0 (ladders are numbered by global id)
+    int* rep_of_chain;     // host [n_chains]: replicate of every chain (swap_step refuses ladders that mix replicates)
     DDChain* st;
     double f[DD_NPAR];     // Bernoulli probability of every parameter in the multiplier move (:208-225)
     unsigned depB, depD;   // parameters the birth side / the death side depend on
@@ -357,13 +361,13 @@ __device__ __forceinline__ void dd_series(double* out, const DDView& v, const do
 }
 
 __device__ __forceinline__ void dd_record(double* rec, const DDView& v, const double* p, double mine, double likB, double likD,
-                                          double likG, long long it, long long accepted, int lane) {
+                                          double likG, long long it, long long accepted, double beta, int lane) {
     double adq[3];
     dd_adequacy(v, p, lane, adq);
     const double prior = warp_sum(dd_prior_term(v, lane, mine));
     if (lane == 0) {
         rec[0] = (double)it; rec[1] = likB + likD + likG; rec[2] = likB; rec[3] = likD; rec[4] = prior; rec[16] = likG;
-        rec[17] = adq[0]; rec[18] = adq[1]; rec[19] = adq[2]; rec[20] = (double)accepted; rec[21] = 0.0; rec[22] = 0.0; rec[23] = 0.0;
+        rec[17] = adq[0]; rec[18] = adq[1]; rec[19] = adq[2]; rec[20] = (double)accepted; rec[21] = beta; rec[22] = 0.0; rec[23] = 0.0;
     }
 #pragma unroll
     for (int k = 0; k < DD_NPAR; ++k)
@@ -456,7 +460,10 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W, W == 1 ? 3 : 2) k7_dd_k
             if (touched & ((1u << P_X0) | (1u << P_G1) | (1u << P_G2)))
                 nG = dd_genre_lik(q, ng, (touched & (1u << P_G1)) != 0, (touched & (1u << P_G2)) != 0, nc);
         }
-        const double x = ((nB + nD + nG) - (likB + likD + likG)) + hp;
+        // tempered: only the likelihood (genre term included) is raised to the power beta (1.0 * d == d at beta = 1).  beta is
+        // read from the state here rather than held from before the loop: with the register copy nvcc contracts the rate
+        // bound l_f + l_f l_mul of the one-warp build into an fma, which moves an untempered chain by an ulp
+        const double x = S->beta * ((nB + nD + nG) - (likB + likD + likG)) + hp;
         if (it == 0 || mh_accept_gt(x, u_acc)) {                                                 // :263
 #pragma unroll
             for (int k = 0; k < DD_NPAR; ++k) p[k] = q[k];
@@ -467,7 +474,7 @@ __global__ void __launch_bounds__(W == 1 ? 128 : 32 * W, W == 1 ? 3 : 2) k7_dd_k
         }
         if (it == next_sample) {                                                                 // :274
             if (P.records && (W == 1 || wq == 0))
-                dd_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v, p, mine, likB, likD, likG, it, accepted, lane);
+                dd_record(P.records + ((size_t)rec_idx * P.n_chains + c) * P.rec_doubles, v, p, mine, likB, likD, likG, it, accepted, S->beta, lane);
             ++rec_idx;
             next_sample += P.sample_every;
         }
@@ -516,7 +523,34 @@ __global__ void k7_init_kernel(DDChain* st, int n_chains, const int* rep_of_chai
         st[c].likB = likB; st[c].likD = likD; st[c].likG = likG; st[c].prior = prior;
         st[c].g[0] = g[0]; st[c].g[1] = g[1]; st[c].g[2] = g[2]; st[c].g[3] = g[3];
         st[c].it = 0; st[c].accepted = 0; st[c].chain = (unsigned)(chain_id0 + c); st[c].rep = rep;
+        st[c].beta = 1.0; st[c].swaps[0] = 0; st[c].swaps[1] = 0;
     }
+}
+
+// ---- tempered ladders (new: the reference has no tempering, SURVEY A-15; the swap rule is lr_swap_round, shared with K3)
+__global__ void k7_set_beta_kernel(DDChain* st, int n, const double* beta) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) st[i].beta = beta[i];
+}
+
+// (likelihood, beta) of every chain, as stored: the untempered likelihood of the current state, genre term included
+__global__ void k7_swap_info_kernel(const DDChain* st, int n, double* __restrict__ info) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n) { info[2 * i] = st[i].likB + st[i].likD + st[i].likG; info[2 * i + 1] = st[i].beta; }
+}
+
+__global__ void k7_swap_apply_kernel(DDChain* st, int n_local, const double* __restrict__ info_all, long long table_first,
+                                     long long n_all, long long first, int ladder, unsigned long long round, uint32_t k0, uint32_t k1) {
+    const int lane = threadIdx.x & 31;
+    const int local = (int)((blockIdx.x * (unsigned)blockDim.x + threadIdx.x) >> 5);
+    if (local >= n_local) return;
+    lr_swap_round(info_all, table_first, n_all, first + local, ladder, round, k0, k1, lane, [&](bool paired, bool accept, double beta_p) {
+        DDChain* S = st + local;
+        if (paired) {
+            S->swaps[0] += 1;
+            if (accept) { S->swaps[1] += 1; S->beta = beta_p; }
+        }
+    });
 }
 
 __global__ void k7_build_tables(const long long* __restrict__ sp_all, const long long* __restrict__ ex_all, const double* __restrict__ br_all,
@@ -630,6 +664,9 @@ extern "C" int lr_dd_create(lr_handle_t h, int32_t n_rep, int32_t n_bins, const 
     t->last.s = st; t->last.valid = 1;
     t->h = h; t->n_rep = n_rep; t->n_bins = n_bins; t->nbp = (n_bins + 3) & ~3; t->m_birth = m_birth; t->m_death = m_death;
     t->n_genre = m_birth == 3 ? n_genre : 0; t->origin = origin; t->present = present; t->n_chains = n_chains; t->seed = seed;
+    t->chain_id0 = chain_id0;
+    t->rep_of_chain = new int[n_chains];
+    for (int i = 0; i < n_chains; ++i) t->rep_of_chain[i] = h_rep_of_chain ? h_rep_of_chain[i] : 0;
     dd_model_tables(m_birth, m_death, t->f, t->depB, t->depD);
     int* d_rep = nullptr;
     cudaError_t e = cudaMallocAsync((void**)&t->tab, (size_t)n_rep * DD_ROWS * t->nbp * sizeof(double), st);
@@ -689,6 +726,7 @@ extern "C" int lr_dd_destroy(lr_dd_t t) {
     if (t->cst) cudaFreeAsync(t->cst, t->h->stream);
     if (t->st) cudaFreeAsync(t->st, t->h->stream);
     if (t->genre) cudaFreeAsync(t->genre, t->h->stream);
+    delete[] t->rep_of_chain;
     delete t;
     return LR_OK;
 }
@@ -808,4 +846,48 @@ extern "C" int lr_dd_state_host(lr_dd_t t, double* h_state) {
     }
     delete[] tmp;
     return LR_OK;
+}
+
+extern "C" int lr_dd_set_beta_host(lr_dd_t t, const double* h_beta) {
+    LR_REQUIRE(t && h_beta, "lr_dd_set_beta_host: null pointer");
+    return lr_set_beta(t->h, &t->last, t->n_chains, h_beta, "lr_dd_set_beta_host", [&](const double* d_beta, cudaStream_t st) {
+        k7_set_beta_kernel<<<(t->n_chains + 127) / 128, 128, 0, st>>>(t->st, t->n_chains, d_beta);
+    });
+}
+
+extern "C" int lr_dd_swap_info(lr_dd_t t, double* d_info, void* stream) {
+    LR_REQUIRE(t && d_info, "lr_dd_swap_info: null pointer");
+    return lr_launch_ordered(t->h, &t->last, stream, [&](cudaStream_t st) {
+        k7_swap_info_kernel<<<(t->n_chains + 127) / 128, 128, 0, st>>>(t->st, t->n_chains, d_info);
+    });
+}
+
+static int dd_swap_apply(lr_dd_t t, const double* d_info_all, int64_t table_first, int64_t n_all, int64_t first, int32_t ladder,
+                         uint64_t round, void* stream, const char* who) {
+    LR_REQUIRE(t, "%s: null pointer", who);
+    return lr_swap_apply(t->h, &t->last, t->n_chains, d_info_all, table_first, n_all, first, ladder, stream, who,
+                         [&](int blocks, int threads, cudaStream_t st) {
+                             k7_swap_apply_kernel<<<blocks, threads, 0, st>>>(t->st, t->n_chains, d_info_all, table_first, n_all, first,
+                                                                              ladder, round, (uint32_t)t->seed, (uint32_t)(t->seed >> 32));
+                         });
+}
+
+extern "C" int lr_dd_swap_apply(lr_dd_t t, const double* d_info_all, int64_t n_all, int64_t first, int32_t ladder, uint64_t round,
+                                void* stream) {
+    return dd_swap_apply(t, d_info_all, 0, n_all, first, ladder, round, stream, "lr_dd_swap_apply");
+}
+
+extern "C" int lr_dd_swap_step(lr_dd_t t, int32_t ladder, uint64_t round) {
+    LR_REQUIRE(t != nullptr, "lr_dd_swap_step: null chains");
+    return lr_swap_step(t->h, t->chain_id0, t->n_chains, ladder, t->rep_of_chain, "lr_dd",
+                        [&](double* d_info) { return lr_dd_swap_info(t, d_info, t->h->stream); },
+                        [&](const double* d_info) {
+                            return dd_swap_apply(t, d_info, t->chain_id0, t->n_chains, t->chain_id0, ladder, round, t->h->stream,
+                                                 "lr_dd_swap_step");
+                        });
+}
+
+extern "C" int lr_dd_temper_host(lr_dd_t t, double* h_beta, int64_t* h_swaps) {
+    LR_REQUIRE(t != nullptr, "lr_dd_temper_host: null chains");
+    return lr_temper_host(t->h, &t->last, t->st, t->n_chains, h_beta, h_swaps, "lr_dd_temper_host");
 }

@@ -136,6 +136,91 @@ int lr_run_into_host(lr_handle_t h, const char* fn, int64_t nrec, size_t sample_
     return LR_OK;
 }
 
+// One launch on `stream` (null: the handle's own), ordered after everything submitted to the object so far (lr_order)
+template <class Launch>
+int lr_launch_ordered(lr_handle_t h, lr_last_stream* last, void* stream, Launch launch) {
+    LR_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    { int rc0 = lr_order(h, last, st); if (rc0 != LR_OK) return rc0; }
+    launch(st);
+    LR_CUDA(cudaGetLastError());
+    h->launches += 1;
+    return LR_OK;
+}
+
+// ---- tempered ladders of the chain objects (K3, K6, K7) ------------------------------------------------------------------------
+// The swap_apply entry points: shard [first, first + n_chains) of global chain ids, gathered (lik, beta) table d_info_all[n_all][2]
+// whose row 0 is global chain table_first.  launch(blocks, threads, stream) starts the sampler's apply kernel, one warp per chain.
+template <class Launch>
+int lr_swap_apply(lr_handle_t h, lr_last_stream* last, int n_chains, const double* d_info_all, int64_t table_first, int64_t n_all,
+                  int64_t first, int32_t ladder, void* stream, const char* who, Launch launch) {
+    LR_REQUIRE(d_info_all, "%s: null pointer", who);
+    LR_REQUIRE(ladder >= 2 && ladder <= 32, "%s: ladder size must be 2..32", who);
+    LR_REQUIRE(first >= table_first && first + n_chains <= table_first + n_all,
+               "%s: this shard [first, first + n_chains) lies outside the gathered table", who);
+    int threads;
+    const int blocks = lr_chain_grid(n_chains, threads);
+    return lr_launch_ordered(h, last, stream, [&](cudaStream_t st) { launch(blocks, threads, st); });
+}
+
+// The swap_step entry points (`prefix` lr_chains, lr_trend, lr_dd): one round for ladders that all live on this shard, on the
+// handle's stream.  info(d_info) fills the (lik, beta) table of the shard in the workspace, apply(d_info) applies the round.
+// rep_of_chain (host, may be null): a ladder whose members run on different replicates is refused -- its swaps would mix two
+// posteriors.
+template <class Info, class Apply>
+int lr_swap_step(lr_handle_t h, int64_t chain_id0, int n_chains, int32_t ladder, const int* rep_of_chain, const char* prefix, Info info,
+                 Apply apply) {
+    LR_REQUIRE(ladder >= 2 && chain_id0 % ladder == 0 && n_chains % ladder == 0,
+               "%s_swap_step: the shard must hold whole ladders (chain_id0 and n_chains multiples of the ladder size); "
+               "use %s_swap_info + an all-gather + %s_swap_apply for ladders that span devices", prefix, prefix, prefix);
+    if (rep_of_chain)
+        for (int c = 0; c < n_chains; ++c)
+            LR_REQUIRE(rep_of_chain[c] == rep_of_chain[c - c % ladder],
+                       "%s_swap_step: the ladder of chain %lld runs on replicates %d and %d; swaps would mix two posteriors", prefix,
+                       (long long)(chain_id0 + c), rep_of_chain[c - c % ladder], rep_of_chain[c]);
+    int rc = lr_ws_acquire(h, (size_t)n_chains * 16, h->stream);
+    if (rc != LR_OK) return rc;
+    rc = info((double*)h->ws);
+    if (rc != LR_OK) return rc;
+    return apply((const double*)h->ws);
+}
+
+// lr_trend_set_beta_host / lr_dd_set_beta_host: every beta in [0, 1], staged through the workspace; set(d_beta, stream) launches
+// the sampler's kernel.  Returns when the betas are in place.
+template <class Set>
+int lr_set_beta(lr_handle_t h, lr_last_stream* last, int n_chains, const double* h_beta, const char* who, Set set) {
+    for (int c = 0; c < n_chains; ++c)
+        LR_REQUIRE(h_beta[c] >= 0.0 && h_beta[c] <= 1.0, "%s: beta of chain %d = %g outside [0, 1]", who, c, h_beta[c]);
+    LR_CUDA(cudaSetDevice(h->device));
+    { int rc0 = lr_order(h, last, h->stream); if (rc0 != LR_OK) return rc0; }
+    int rc = lr_ws_acquire(h, (size_t)n_chains * 8, h->stream);
+    if (rc != LR_OK) return rc;
+    LR_CUDA(cudaMemcpyAsync(h->ws, h_beta, (size_t)n_chains * 8, cudaMemcpyHostToDevice, h->stream));
+    set((const double*)h->ws, h->stream);
+    LR_CUDA(cudaGetLastError());
+    h->launches += 1;
+    LR_CUDA(cudaStreamSynchronize(h->stream));
+    return LR_OK;
+}
+
+// lr_trend_temper_host / lr_dd_temper_host: beta [n] and swaps proposed / accepted [n][2] of the chain states d_st (K6 TrendChain,
+// K7 DDChain: fields beta and swaps); either output may be null
+template <class Chain>
+int lr_temper_host(lr_handle_t h, lr_last_stream* last, const Chain* d_st, int n_chains, double* h_beta, int64_t* h_swaps, const char* who) {
+    LR_CUDA(cudaSetDevice(h->device));
+    { int rc0 = lr_order(h, last, h->stream); if (rc0 != LR_OK) return rc0; }
+    LR_CUDA(cudaStreamSynchronize(h->stream));
+    Chain* tmp = new Chain[n_chains];
+    cudaError_t e = cudaMemcpy(tmp, d_st, (size_t)n_chains * sizeof(Chain), cudaMemcpyDeviceToHost);
+    if (e != cudaSuccess) { delete[] tmp; lr_set_error("%s: %s", who, cudaGetErrorString(e)); return LR_ERR_CUDA; }
+    for (int c = 0; c < n_chains; ++c) {
+        if (h_beta) h_beta[c] = tmp[c].beta;
+        if (h_swaps) { h_swaps[2 * c] = tmp[c].swaps[0]; h_swaps[2 * c + 1] = tmp[c].swaps[1]; }
+    }
+    delete[] tmp;
+    return LR_OK;
+}
+
 // The *_create_host entry points of K6 / K7: the per-bin statistics sp, ex, br [cnt] from the host into the workspace, on the
 // handle's stream
 inline int lr_upload_bin_stats(lr_handle_t h, size_t cnt, const int64_t* h_sp, const int64_t* h_ex, const double* h_br, int64_t** d_sp,
@@ -244,4 +329,53 @@ __device__ __forceinline__ bool mh_accept_gt(double x, double u) {
 __device__ __forceinline__ double normal_f32(double u1, uint32_t bits) {
     const float r = sqrtf(-2.0f * __logf((float)u1));
     return (double)(r * cospif(((float)(bits >> 8) + 0.5f) * 1.1920929e-7f));     // angle 2 pi k / 2^24 as cospi(2 k / 2^24)
+}
+
+// ---- the swap rule of the tempered ladders (K3, K6, K7) ----------------------------------------------------------------------
+// One swap round.  Chains are grouped into ladders of `ladder` consecutive GLOBAL chain ids; within a ladder the members are
+// ordered by temperature and neighbours (2p + parity, 2p + 1 + parity) exchange their TEMPERATURES with probability
+// min(1, exp((beta_i - beta_j)(lik_j - lik_i))).  Every rank holding a member of a ladder recomputes the whole ladder's decisions
+// from the gathered (lik, beta) table and a Philox draw keyed by (seed, ladder, round, pair), so the outcome is identical
+// everywhere and no state crosses the interconnect.  Only the likelihood is tempered, so lik is the untempered log-likelihood.
+// Called by one warp for global chain g (table row of global chain m: m - table_first); one lane then calls
+// write(paired, accept, beta_p) for that chain: paired = it has a partner this round, accept = the two exchange, beta_p = the
+// partner's beta.  The sampler's write stores beta and its swap counters.
+template <class Write>
+__device__ __forceinline__ void lr_swap_round(const double* __restrict__ info_all, long long table_first, long long n_all, long long g,
+                                              int ladder, unsigned long long round, uint32_t k0, uint32_t k1, int lane, Write write) {
+    const long long lad = g / ladder;
+    const int me = (int)(g - lad * ladder);
+    const long long m = lad * ladder + lane;
+    const bool on = lane < ladder && m >= table_first && m < table_first + n_all;
+    const double lik = on ? info_all[2 * (m - table_first)] : 0.0;
+    const double beta = on ? info_all[2 * (m - table_first) + 1] : -1.0;
+    // rank by temperature: 0 = coldest (largest beta); ties broken by position
+    int rank = 0;
+    for (int k = 0; k < ladder; ++k) {
+        const double bk = __shfl_sync(0xffffffffu, beta, k);
+        if (bk > beta || (bk == beta && k < lane)) rank++;
+    }
+    const int parity = (int)(round & 1ull);
+    const int q = rank - parity;
+    int partner_rank = -1;
+    if (on && q >= 0) {
+        partner_rank = (q ^ 1) + parity;
+        if (partner_rank >= ladder) partner_rank = -1;
+    }
+    int partner = -1;
+    for (int k = 0; k < ladder; ++k) {
+        const int rk = __shfl_sync(0xffffffffu, rank, k);
+        const bool onk = __shfl_sync(0xffffffffu, (int)on, k) != 0;
+        if (onk && rk == partner_rank) partner = k;
+    }
+    const double lik_p = __shfl_sync(0xffffffffu, lik, partner < 0 ? 0 : partner);
+    const double beta_p = __shfl_sync(0xffffffffu, beta, partner < 0 ? 0 : partner);
+    bool accept = false;
+    if (partner >= 0) {
+        const int pair = (rank < partner_rank ? rank : partner_rank);
+        const Philox4 r = philox4x32_10((uint32_t)round, (uint32_t)(round >> 32), (uint32_t)pair | (0x5157u << 16), (uint32_t)lad, k0, k1 ^ 0x7e3a9u);
+        const double u = u01(r.x, r.y);
+        accept = log(u) <= (beta - beta_p) * (lik_p - lik);
+    }
+    if (lane == me) write(partner >= 0, accept, beta_p);
 }

@@ -9,6 +9,10 @@ As shipped the reference only starts with ``-m_birth 3 -g <genre table>`` (NameE
 and 2 run what its functions define for them.  -m_birth -1 / -m_death -1 (NameError at :192-195) are refused.
 New flags: -chains (chain k is named like a reference run with seed + k), -device, -quiet.  -d may name a directory of tables
 (stochastic imputations of one data set): one replicate each over the common window, chain k on table k % n_tables.
+-temper T > 1 (with -swap_every, -temper_delta, as for literate_b200.forward; the reference has no tempering): every logged
+chain is the cold member (beta = 1, the reference's chain) of a ladder of T Metropolis-coupled chains, all on its table; the
+heated members temper the whole likelihood, genre term included.  Only cold samples reach the logs, whose names, headers and
+rows are those of an untempered run.
 """
 from __future__ import annotations
 
@@ -28,6 +32,7 @@ from .library import bin_window, parse_ts_te
 BANNER = "\n\n             DDRate  (literate_b200: B200-native path)\n"
 PARAMS = ["l_f", "l_mul", "k", "x0", "div_0", "L", "m_mul", "nuB", "nuD", "g_lambda1", "g_lambda2"]
 REC_HEAD, NPAR = N.LR_DD_REC_HEAD, N.LR_DD_NPAR
+REC_BETA = 21                                            # record field of the chain's inverse temperature
 
 
 def build_parser():
@@ -42,7 +47,7 @@ def build_parser():
 
 class DDChains(L.ChainObject):
     """lr_dd_t: the per-bin table, the genre table and a population of independent DDRate chains on one device."""
-    PREFIX, STATE_DOUBLES = "dd", N.LR_DD_STATE_DOUBLES
+    PREFIX, STATE_DOUBLES, REC_BETA = "dd", N.LR_DD_STATE_DOUBLES, REC_BETA
 
     def __init__(self, dev: E.Device, sp, ex, br, origin, present, m_birth=2, m_death=2, gts=None, gte=None, n_chains=1, seed=1,
                  chain_id0=0, rep_of_chain=None):
@@ -161,9 +166,11 @@ def run(args, device=None):
             print("EMPIRICAL DEATH RATES:"); print(ex[0] / br[0])
 
     c0, n_local = P.shard_range(args.chains, world, rank)
-    rep_of_chain = (np.arange(c0, c0 + n_local) % n_tab).astype(np.int32)
-    chains = DDChains(dev, sp, ex, br, origin, present, args.m_birth, args.m_death, gts, gte, n_local, seed, chain_id0=c0,
+    chain_id0, n_dev, rep_of_chain, beta = L.ladders(args, c0, n_local, n_tab)
+    chains = DDChains(dev, sp, ex, br, origin, present, args.m_birth, args.m_death, gts, gte, n_dev, seed, chain_id0=chain_id0,
                       rep_of_chain=rep_of_chain)
+    if beta is not None:
+        chains.set_beta(beta)
     paths, files, writers = [], [], []
     for k in range(c0, c0 + n_local):
         r = k % n_tab
@@ -177,12 +184,16 @@ def run(args, device=None):
         else:
             write_div_log(stem + ".div.log", sp[r], ex[r], br[r], gstats.sp[0], gstats.ex[0], gstats.br[0])
 
-    t_run = L.sample_and_write(chains, args.n, args.s, files, writers, lambda rec: record_row(rec, n_bins, args.m_birth, origin),
-                               lambda rec: print(int(rec[0]), rec[1], rec[5:5 + NPAR]), args.quiet)       # :280
+    t_run, rounds = L.sample_and_write(chains, args.n, args.s, files, writers, lambda rec: record_row(rec, n_bins, args.m_birth, origin),
+                                       lambda rec: print(int(rec[0]), rec[1], rec[5:5 + NPAR]), args.quiet, args.temper,
+                                       args.swap_every)       # :280
     if not args.quiet:
-        acc = chains.state()[:, 16].sum() / max(1, n_local * args.n)
+        acc = chains.state()[:, 16].sum() / max(1, n_dev * args.n)
         print("literate_b200: %d DDRate chains x %d iterations in %.3f s (%.3g it/s, acceptance %.3f); binning %.4f s"
-              % (n_local, args.n, t_run, n_local * args.n / max(t_run, 1e-9), acc, t_bin))
+              % (n_dev, args.n, t_run, n_dev * args.n / max(t_run, 1e-9), acc, t_bin))
+        if args.temper > 1:
+            swaps = chains.temper()[1].sum(0)
+            print("literate_b200: %d swap rounds, %.3f of the proposed temperature swaps accepted" % (rounds, swaps[1] / max(swaps[0], 1)))
     chains.close()
     return paths
 

@@ -447,8 +447,62 @@ COUNTER_NAMES = ["iterations", "accepted", "lik_evals", "rate_updates", "move_sh
                  "swaps_proposed", "swaps_accepted"]
 
 
-class Chains:
+class Tempered:
+    """Tempered ladders of Metropolis-coupled chains (new; the reference has no MC3), for the chain objects of all three
+    samplers: engine.Chains (RJMCMC, PREFIX "chains") and the TrendRate / DDRate objects of library.ChainObject ("trend",
+    "dd").  The methods call the C entry points lr_<PREFIX>_set_beta_host / _swap_step / _swap_info / _swap_apply on the
+    object's handle; a subclass provides dev, n_chains, rec_doubles, _handle() and run(n_iter, sample_every)."""
+    PREFIX = ""
+
+    def _lr(self, name):
+        return getattr(self.dev.lib, "lr_%s_%s" % (self.PREFIX, name))
+
+    def set_beta(self, beta):
+        """Inverse temperature of every chain (a scalar or [n_chains]); a chain at beta = 1 is the reference's chain."""
+        beta = np.ascontiguousarray(np.broadcast_to(np.asarray(beta, np.float64), (self.n_chains,)))
+        N.check(self._lr("set_beta_host")(self._handle(), N.np_ptr(beta)), "lr_%s_set_beta_host" % self.PREFIX)
+
+    def swap_step(self, ladder: int, round_: int):
+        """One swap round for ladders of `ladder` consecutive chains that all live on this device."""
+        N.check(self._lr("swap_step")(self._handle(), int(ladder), C.c_uint64(int(round_))), "lr_%s_swap_step" % self.PREFIX)
+
+    def run_tempered(self, n_iter: int, sample_every: int, ladder: int, swap_every: int, round0: int = 0, swap=None):
+        """n_iter iterations with a swap round every `swap_every` iterations (ladders on this device unless `swap`
+        -- a callable round -> None, e.g. parallel.tempered_swap bound to this shard -- is given).
+        Returns (records of ALL chains [n_samples, n_chains, rec_doubles], number of swap rounds done); cold_records()
+        keeps the records of the chains at beta = 1."""
+        out, done, rnd = [], 0, int(round0)
+        while done < n_iter:
+            n = min(int(swap_every), n_iter - done)
+            r = self.run(n, sample_every)
+            if r is not None and len(r):
+                out.append(r)
+            done += n
+            if done < n_iter or n == swap_every:
+                if swap is None:
+                    self.swap_step(ladder, rnd)
+                else:
+                    swap(rnd)
+                rnd += 1
+        recs = np.concatenate(out) if out else np.empty((0, self.n_chains, self.rec_doubles))
+        return recs, rnd - int(round0)
+
+    def swap_info_device(self, info, stream=None):
+        """(likelihood, beta) of every chain into the float64 CUDA tensor info[n_chains, 2]."""
+        N.check(self._lr("swap_info")(self._handle(), C.c_void_p(info.data_ptr()), _stream_ptr(stream, info.device)),
+                "lr_%s_swap_info" % self.PREFIX)
+        return info
+
+    def swap_apply_device(self, info_all, first: int, ladder: int, round_: int, stream=None):
+        """Apply a swap round given the gathered table info_all[n_all, 2] of the whole ensemble (see parallel.tempered_swap)."""
+        N.check(self._lr("swap_apply")(self._handle(), C.c_void_p(info_all.data_ptr()), int(info_all.shape[0]), int(first), int(ladder),
+                                       C.c_uint64(int(round_)), _stream_ptr(stream, info_all.device)), "lr_%s_swap_apply" % self.PREFIX)
+
+
+class Chains(Tempered):
     """A population of independent RJMCMC chains on one device (runMCMC, LiteRateForward.py:216-373)."""
+    PREFIX = "chains"
+    rec_doubles = LR_REC_DOUBLES
 
     def __init__(self, ds: Dataset, n_chains: int, seed: int, cfg: ChainConfig = None, chain_id0: int = 0, rep_of_chain=None):
         self.ds, self.dev, self.n_chains = ds, ds.dev, int(n_chains)
@@ -464,6 +518,9 @@ class Chains:
         N.check(self.dev.lib.lr_chains_create(self.dev.h, ds.ds, self.n_chains, C.byref(cfg), C.c_uint64(int(seed) & (2**64 - 1)),
                                               int(chain_id0), N.np_ptr(rep), C.byref(c)), "lr_chains_create")
         self.c = c
+
+    def _handle(self):
+        return self.c
 
     def close(self):
         if getattr(self, "c", None):
@@ -523,46 +580,6 @@ class Chains:
         N.check(self.dev.lib.lr_chains_team_stats_host(self.c, N.np_ptr(out)), "lr_chains_team_stats_host")
         return out
 
-    # ---- tempered ensembles (new; the reference has no MC3)
-    def set_beta(self, beta):
-        beta = np.ascontiguousarray(np.broadcast_to(np.asarray(beta, np.float64), (self.n_chains,)))
-        N.check(self.dev.lib.lr_chains_set_beta_host(self.c, N.np_ptr(beta)), "lr_chains_set_beta_host")
-
-    def swap_step(self, ladder: int, round_: int):
-        """One swap round for ladders of `ladder` consecutive chains that all live on this device."""
-        N.check(self.dev.lib.lr_chains_swap_step(self.c, int(ladder), C.c_uint64(int(round_))), "lr_chains_swap_step")
-
-    def run_tempered(self, n_iter: int, sample_every: int, ladder: int, swap_every: int, round0: int = 0, swap=None):
-        """n_iter iterations with a swap round every `swap_every` iterations (ladders on this device unless `swap`
-        -- a callable round -> None, e.g. parallel.tempered_swap bound to this shard -- is given).
-        Returns (records of ALL chains [n_samples, n_chains, 144], number of swap rounds done); filter on
-        records[..., REC_BETA] == 1 for the cold chains (cold_records())."""
-        out, done, rnd = [], 0, int(round0)
-        while done < n_iter:
-            n = min(int(swap_every), n_iter - done)
-            r = self.run(n, sample_every)
-            if r is not None and len(r):
-                out.append(r)
-            done += n
-            if done < n_iter or n == swap_every:
-                if swap is None:
-                    self.swap_step(ladder, rnd)
-                else:
-                    swap(rnd)
-                rnd += 1
-        recs = np.concatenate(out) if out else np.empty((0, self.n_chains, LR_REC_DOUBLES))
-        return recs, rnd - int(round0)
-
-    def swap_info_device(self, info, stream=None):
-        """(likelihood, beta) of every chain into the float64 CUDA tensor info[n_chains, 2]."""
-        N.check(self.dev.lib.lr_chains_swap_info(self.c, C.c_void_p(info.data_ptr()), _stream_ptr(stream, info.device)), "lr_chains_swap_info")
-        return info
-
-    def swap_apply_device(self, info_all, first: int, ladder: int, round_: int, stream=None):
-        """Apply a swap round given the gathered table info_all[n_all, 2] of the whole ensemble (see parallel.tempered_swap)."""
-        N.check(self.dev.lib.lr_chains_swap_apply(self.c, C.c_void_p(info_all.data_ptr()), int(info_all.shape[0]), int(first), int(ladder),
-                                                  C.c_uint64(int(round_)), _stream_ptr(stream, info_all.device)), "lr_chains_swap_apply")
-
 
 def default_config(model_BDI=0, const_rates=0, const_death_rate=0, use_rate_HP=1, Poisson_prior=0.0, update_fraction=0.75,
                    real_move_shift=0, beta=1.0, loop_variant=0) -> ChainConfig:
@@ -571,14 +588,15 @@ def default_config(model_BDI=0, const_rates=0, const_death_rate=0, use_rate_HP=1
                        float(update_fraction), int(real_move_shift), int(loop_variant), float(beta))
 
 
-def cold_records(records, ladder: int):
-    """[n_samples, n_chains, 144] of a tempered run -> [n_samples, n_chains // ladder, 144]: per ladder and sample, the
-    record of the member that held beta = 1 when the sample was written."""
+def cold_records(records, ladder: int, col: int = REC_BETA):
+    """[n_samples, n_chains, w] of a tempered run -> [n_samples, n_chains // ladder, w]: per ladder and sample, the
+    record of the member that held beta = 1 when the sample was written.  `col`: the field of beta in the record layout
+    (REC_BETA of the RJMCMC records, trend.REC_BETA, ddrate.REC_BETA)."""
     ns, nc, w = records.shape
     r = records.reshape(ns, nc // ladder, ladder, w)
-    idx = np.argmax(r[..., REC_BETA], axis=2)
+    idx = np.argmax(r[..., col], axis=2)
     out = np.take_along_axis(r, idx[:, :, None, None], axis=2)[:, :, 0, :]
-    if not np.all(out[..., REC_BETA] == 1.0):
+    if not np.all(out[..., col] == 1.0):
         raise ValueError("a ladder has no chain at beta = 1")
     return out
 

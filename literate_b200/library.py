@@ -1,6 +1,7 @@
 """What the TrendRate and DDRate command lines share, as the reference keeps it in literate_library.py: the table parser
 (parse_ts_te), the unit bins (create_bins), the core flags (core_arguments) and the seed rule (set_seed), plus the host
-plumbing of their chain objects (K6 lr_trend_t, K7 lr_dd_t) and the sampling loop that writes their logs.
+plumbing of their chain objects (K6 lr_trend_t, K7 lr_dd_t), their tempered ladders (-temper) and the sampling loop that
+writes their logs.
 """
 from __future__ import annotations
 
@@ -15,6 +16,7 @@ import numpy as np
 
 from . import _native as N
 from . import engine as E
+from . import parallel as P
 
 
 def parse_ts_te(path, TBP=False, first_year=-1, last_year=-1, death_jitter=0.5):
@@ -69,7 +71,7 @@ def bin_window(origin, present, rm_first_bin=0):
 
 def build_parser(prog, add_own):
     """The flags of literate_library.core_arguments (:290-308), then the script's own (add_own(parser)), then -chains,
-    -device and -quiet."""
+    -device, -quiet and the tempering flags of literate_b200.forward (-temper, -swap_every, -temper_delta)."""
     p = argparse.ArgumentParser(prog=prog)
     p.add_argument('-v', action='version', version='%(prog)s')
     p.add_argument('-d', type=str, help='data file', default="", metavar="")
@@ -88,12 +90,17 @@ def build_parser(prog, add_own):
     p.add_argument('-chains', type=int, help='number of independent chains run concurrently on the GPU', default=1, metavar=1)
     p.add_argument('-device', type=int, help='CUDA device index', default=0, metavar=0)
     p.add_argument('-quiet', type=int, help='1: no per-sample progress on stdout', default=0, metavar=0)
+    p.add_argument('-temper', type=int, help='temperatures per logged chain (1: no tempering, as the reference)', default=1, metavar=1)
+    p.add_argument('-swap_every', type=int, help='iterations between temperature-swap rounds', default=1000, metavar=1000)
+    p.add_argument('-temper_delta', type=float, help='ladder beta_k = 1/(1 + delta k)', default=0.1, metavar=0.1)
     return p
 
 
 def seed_and_chains(args, world):
     """set_seed (literate_library.py:282-288): -seed -1 draws the seed; with several GPUs every rank must be given the same
-    one.  There must be at least one chain per GPU."""
+    one.  There must be at least one chain per GPU, and -temper must be 1..32 (checked before any device is touched)."""
+    if not (1 <= args.temper <= 32):
+        raise SystemExit("-temper must be 1..32")
     if args.seed == -1:
         if world > 1:
             raise SystemExit("give -seed explicitly when running on several GPUs (every rank must use the same one)")
@@ -130,14 +137,15 @@ def read_tables(args, exclude):
     return tables, ts, te, present, origin
 
 
-class ChainObject:
+class ChainObject(E.Tempered):
     """A population of independent chains of one of the sibling samplers on one device: the C entry points
-    lr_<PREFIX>_* of lr_trend_t (K6) and lr_dd_t (K7).  Subclasses create the object and set dev, n_chains, n_bins and t."""
-    PREFIX = ""
+    lr_<PREFIX>_* of lr_trend_t (K6) and lr_dd_t (K7), tempered ladders included (engine.Tempered).  Subclasses create the
+    object and set dev, n_chains, n_bins and t; REC_BETA is the field of beta in their records."""
     STATE_DOUBLES = 0
+    REC_BETA = 0
 
-    def _lr(self, name):
-        return getattr(self.dev.lib, "lr_%s_%s" % (self.PREFIX, name))
+    def _handle(self):
+        return self.t
 
     @staticmethod
     def _inputs(sp, ex, br, rep_of_chain, n_chains):
@@ -191,21 +199,45 @@ class ChainObject:
         N.check(self._lr("state_host")(self.t, N.np_ptr(out)), "lr_%s_state_host" % self.PREFIX)
         return out
 
+    def temper(self):
+        """(beta [n_chains], temperature swaps proposed / accepted int64 [n_chains, 2]) of every chain."""
+        beta = np.empty(self.n_chains, dtype=np.float64)
+        swaps = np.empty((self.n_chains, 2), dtype=np.int64)
+        N.check(self._lr("temper_host")(self.t, N.np_ptr(beta), N.np_ptr(swaps)), "lr_%s_temper_host" % self.PREFIX)
+        return beta, swaps
 
-def sample_and_write(chains, n_iter, s, files, writers, row, progress, quiet):
+
+def ladders(args, c0, n_local, n_tab):
+    """Device chains of this rank's logged chains [c0, c0 + n_local): with -temper T every logged chain k is the ladder of
+    device chains [k T, (k + 1) T), all on table k % n_tab.  Returns (chain_id0, n_chains, rep_of_chain, beta or None)."""
+    T = args.temper
+    rep_of_chain = np.repeat(np.arange(c0, c0 + n_local) % n_tab, T).astype(np.int32)
+    beta = np.tile(P.temperature_ladder(T, args.temper_delta), n_local) if T > 1 else None
+    return c0 * T, n_local * T, rep_of_chain, beta
+
+
+def sample_and_write(chains, n_iter, s, files, writers, row, progress, quiet, ladder=1, swap_every=1000):
     """Runs n_iter iterations of every chain, sampling every s-th, in launches of at most ~256 MB of records and 4M
-    iterations; every sample of chain k becomes the log row row(rec) of writers[k], and unless quiet progress(rec) of chain
-    0 goes to stdout.  Closes the files; returns the wall time of the run."""
-    n_local = chains.n_chains
+    iterations; every sample of logged chain k becomes the log row row(rec) of writers[k], and unless quiet progress(rec) of
+    chain 0 goes to stdout.  ladder > 1: the chains are ladders of `ladder` consecutive chains with a swap round every
+    swap_every iterations (run_tempered, the round counter carried across launches), and only the cold member of each
+    ladder is logged.  Closes the files; returns (wall time of the run, swap rounds done)."""
+    n_dev = chains.n_chains
     s_freq = max(1, s)
-    max_rec = max(1, (256 << 20) // (n_local * chains.rec_doubles * 8))
+    max_rec = max(1, (256 << 20) // (n_dev * chains.rec_doubles * 8))
     per_launch = max(s_freq, min(max_rec * s_freq, 4_000_000) // s_freq * s_freq)
-    done = 0
+    done = rounds = 0
     t_run = time.time()
     while done < n_iter:
         n_it = min(per_launch, n_iter - done)
-        recs = chains.run(n_it, s_freq)
+        if ladder > 1:
+            recs, r = chains.run_tempered(n_it, s_freq, ladder, max(1, swap_every), round0=rounds)
+            rounds += r
+            recs = E.cold_records(recs, ladder, chains.REC_BETA)
+        else:
+            recs = chains.run(n_it, s_freq)
         done += n_it
+        n_local = recs.shape[1]
         for r in range(recs.shape[0]):
             for k in range(n_local):
                 writers[k].writerow(row(recs[r, k]))
@@ -216,4 +248,4 @@ def sample_and_write(chains, n_iter, s, files, writers, row, progress, quiet):
     t_run = time.time() - t_run
     for fh in files:
         fh.close()
-    return t_run
+    return t_run, rounds

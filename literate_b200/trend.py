@@ -6,10 +6,13 @@ name, header and row layout (trend_rate.py:110-118, :191).  The statistics come 
 K6 (`lr_trend_*`); this module parses, launches and writes text.  There is no CPU path.
 
 New flags: -chains (independent chains, one warp each; chain k is named like a reference run with seed + k), -device,
--quiet.  -d may name a directory of tables (stochastic imputations of one data set, as for literate_b200.forward): every
+-quiet, -temper.  -d may name a directory of tables (stochastic imputations of one data set, as for literate_b200.forward): every
 table is a replicate binned in the same K1 launch over the common window, chain k runs on table k % n_tables and writes
 next to that table.  Under torchrun the chains are block-partitioned over the ranks; a chain keeps its name and its Philox
 stream whatever the number of GPUs.
+-temper T > 1 (with -swap_every, -temper_delta, as for literate_b200.forward; new, the reference has no tempering): every
+logged chain is the cold member (beta = 1, the reference's chain) of a ladder of T Metropolis-coupled chains, all on its
+table; only cold samples reach the logs, whose names, headers and rows are those of an untempered run.
 
   python -m literate_b200.trend -d table.tsv -trend_data trend.tsv -trend_index 1 -n 1000000 -s 1000 -seed 1 -chains 256
 """
@@ -32,6 +35,7 @@ BANNER = "\n\n             TrendRate - 20190205  (literate_b200: B200-native pat
 SMALL_NUMBER = 0.000000000000001                         # trend_rate.py:55
 PARAMS = ["l_min", "m_min", "alpha", "beta", "delta", "gamma"]
 REC_HEAD = N.LR_TREND_REC_HEAD
+REC_BETA = 15                                            # record field of the chain's inverse temperature
 
 
 def _flag(v):
@@ -65,7 +69,7 @@ def parse_trend_data(path, index, rm_first_bin=0):
 
 class TrendChains(L.ChainObject):
     """lr_trend_t: the per-bin table and a population of independent TrendRate chains on one device."""
-    PREFIX, STATE_DOUBLES = "trend", N.LR_TREND_STATE_DOUBLES
+    PREFIX, STATE_DOUBLES, REC_BETA = "trend", N.LR_TREND_STATE_DOUBLES, REC_BETA
 
     def __init__(self, dev: E.Device, sp, ex, br, trend, n_chains, seed, const_birth=False, const_death=False, chain_id0=0,
                  rep_of_chain=None):
@@ -160,8 +164,10 @@ def run(args, device=None):
             print("TREND", trend)
 
     c0, n_local = P.shard_range(args.chains, world, rank)
-    rep_of_chain = (np.arange(c0, c0 + n_local) % n_tab).astype(np.int32)
-    chains = TrendChains(dev, sp, ex, br, trend, n_local, seed, const_birth, const_death, chain_id0=c0, rep_of_chain=rep_of_chain)
+    chain_id0, n_dev, rep_of_chain, beta = L.ladders(args, c0, n_local, n_tab)
+    chains = TrendChains(dev, sp, ex, br, trend, n_dev, seed, const_birth, const_death, chain_id0=chain_id0, rep_of_chain=rep_of_chain)
+    if beta is not None:
+        chains.set_beta(beta)
     paths, files, writers = [], [], []
     for k in range(c0, c0 + n_local):
         path = log_name(tables[k % n_tab], seed + k // n_tab, args.trend_index, const_birth, const_death, no_death)
@@ -170,12 +176,15 @@ def run(args, device=None):
         w.writerow(header(n_bins))
         paths.append(path); files.append(fh); writers.append(w)
 
-    t_run = L.sample_and_write(chains, args.n, args.s, files, writers, lambda rec: record_row(rec, n_bins),
-                               lambda rec: print(int(rec[0]), rec[1], rec[5:11]), args.quiet)       # :187
+    t_run, rounds = L.sample_and_write(chains, args.n, args.s, files, writers, lambda rec: record_row(rec, n_bins),
+                                       lambda rec: print(int(rec[0]), rec[1], rec[5:11]), args.quiet, args.temper, args.swap_every)  # :187
     if not args.quiet:
-        acc = chains.state()[:, 10].sum() / max(1, n_local * args.n)
+        acc = chains.state()[:, 10].sum() / max(1, n_dev * args.n)
         print("literate_b200: %d TrendRate chains x %d iterations in %.3f s (%.3g it/s, acceptance %.3f); binning %.4f s"
-              % (n_local, args.n, t_run, n_local * args.n / max(t_run, 1e-9), acc, t_bin))
+              % (n_dev, args.n, t_run, n_dev * args.n / max(t_run, 1e-9), acc, t_bin))
+        if args.temper > 1:
+            swaps = chains.temper()[1].sum(0)
+            print("literate_b200: %d swap rounds, %.3f of the proposed temperature swaps accepted" % (rounds, swaps[1] / max(swaps[0], 1)))
     chains.close()
     return paths
 
