@@ -315,6 +315,24 @@ int lr_imputation_envelope(lr_handle_t h, const int64_t* d_sp, const int64_t* d_
  * torch.sort on the device, a bin range at a time so that the matrix of a large ensemble need not exist as a whole). */
 int lr_marginal_rates(lr_handle_t h, const double* d_records, int64_t n_records, double first_edge, int32_t n_bins,
                       int32_t bin_lo, int32_t bin_cnt, double* d_birth, double* d_death, void* stream);
+/* K8: per-column means and exact HPD intervals of a row-major fp64 matrix d_rows[n_rows][row_stride] on the device -- the sample
+ * records of any sampler (after the burn-in rows) or the matrices of lr_marginal_rates -- without copying it.
+ *   mask_col     < 0: every row counts; otherwise only rows with row[mask_col] == 1.0 (the cold members of tempered ladders:
+ *                the beta field of the records, e.g. 15 for TrendRate, 21 for DDRate)
+ *   column j     value = row[h_col_a[j]], then + row[b] (h_col_sign[j] = 1) or - row[b] (-1) if b = h_col_b[j] >= 0, then
+ *                + h_col_add[j] if that is non-zero: one fp64 operation each, in this order (the log's net rate l_j - m_j, DDRate's
+ *                maxCarryingCap L + div_0 and midpoint_x0 x0 + origin).  HOST arrays [n_cols]; b, sign and add may be NULL (-1, 1, 0).
+ *   level        in (0, 1]
+ * Outputs [n_cols] fp64: d_mean (compensated sums in a fixed order: within a few ulp of the correctly rounded mean, and repeated calls are
+ * bit-identical) and the HPD bounds d_lo, d_hi under
+ * calcHPD (plotRJforward.v3.py:12-28): n_in = rint(level n), widths x[i + n_in - 1] - x[i] over the sorted column, the first
+ * minimum wins; NaN sorts last as in np.sort and a NaN width wins as in np.argmin; +-inf are ordered normally.  The bounds equal
+ * a host sort's bit for bit up to the sign of a zero.  d_n (int64 [1], may be NULL): the number of rows used.  When
+ * rint(level n) < 2 every output column is NaN.  Scratch (at most ~512 MB of tails at a time) comes from the handle's workspace;
+ * rejects bad sizes and column indices; asynchronous on `stream` (the column specs are staged before it returns). */
+int lr_column_hpd(lr_handle_t h, const double* d_rows, int64_t n_rows, int64_t row_stride, int32_t mask_col, int32_t n_cols,
+                  const int32_t* h_col_a, const int32_t* h_col_b, const int32_t* h_col_sign, const double* h_col_add,
+                  double level, double* d_mean, double* d_lo, double* d_hi, int64_t* d_n, void* stream);
 
 /* ---------------------------------------------------------------- TrendRate (SURVEY 8 f-4): fixed-dimension chains on the same statistics
  *

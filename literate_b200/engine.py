@@ -275,6 +275,39 @@ class Device:
                 "lr_marginal_rates")
         return b, d
 
+    def column_hpd_device(self, rows, cols, level=0.95, mask_col=-1, stream=None):
+        """Means and HPD intervals of columns of a device-resident matrix (K8, lr_column_hpd), without copying it.
+
+        rows: float64 CUDA tensor [n_rows, row_stride] whose rows are contiguous (e.g. records reshaped to rows); cols: one spec
+        per output column, an index a or a tuple (a, b, sign[, add]): value = row[a] (+ or -) row[b] (+ add), one fp64 operation
+        each; b = -1 for none.  mask_col >= 0: only rows with row[mask_col] == 1.0 count (the cold members of tempered ladders).
+        Returns (mean, lo, hi, n): float64 CUDA tensors [n_cols] and the number of rows used as an int64 CUDA tensor [1].
+        Raises RuntimeError("not enough data") as summary.hpd_columns does when round(level n) < 2 (with a mask that needs n: the
+        call then waits for the device)."""
+        import torch
+        if not (rows.is_cuda and rows.dtype == torch.float64 and rows.dim() == 2 and rows.stride(1) == 1):
+            raise ValueError("rows must be a float64 CUDA tensor [n_rows, row_stride] with contiguous rows")
+        spec = [(c, -1, 1, 0.0) if np.ndim(c) == 0 else (tuple(c) + (0.0,))[:4] for c in cols]
+        if not spec:
+            raise ValueError("no columns")
+        a = np.ascontiguousarray([s[0] for s in spec], dtype=np.int32)
+        b = np.ascontiguousarray([s[1] for s in spec], dtype=np.int32)
+        sg = np.ascontiguousarray([s[2] for s in spec], dtype=np.int32)
+        add = np.ascontiguousarray([s[3] for s in spec], dtype=np.float64)
+        n_rows = rows.shape[0]
+        stride = rows.stride(0) if n_rows > 1 else rows.shape[1]
+        if mask_col < 0 and int(round(level * n_rows)) < 2:
+            raise RuntimeError("not enough data")
+        out = torch.empty((3, len(spec)), dtype=torch.float64, device=rows.device)
+        n = torch.empty(1, dtype=torch.int64, device=rows.device)
+        N.check(self.lib.lr_column_hpd(self.h, C.c_void_p(rows.data_ptr()), int(n_rows), int(stride), int(mask_col), len(spec),
+                                       N.np_ptr(a), N.np_ptr(b), N.np_ptr(sg), N.np_ptr(add), float(level),
+                                       C.c_void_p(out[0].data_ptr()), C.c_void_p(out[1].data_ptr()), C.c_void_p(out[2].data_ptr()),
+                                       C.c_void_p(n.data_ptr()), _stream_ptr(stream, rows.device)), "lr_column_hpd")
+        if mask_col >= 0 and int(round(level * int(n.item()))) < 2:
+            raise RuntimeError("not enough data")
+        return out[0], out[1], out[2], n
+
     def new_accumulators(self, n_rep, n_bins, device):
         import torch
         return torch.zeros((n_rep, N.LR_ACC_ROWS, int(self.lib.lr_acc_stride(int(n_bins)))), dtype=torch.int64, device=device)
