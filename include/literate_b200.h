@@ -333,6 +333,27 @@ int lr_marginal_rates(lr_handle_t h, const double* d_records, int64_t n_records,
 int lr_column_hpd(lr_handle_t h, const double* d_rows, int64_t n_rows, int64_t row_stride, int32_t mask_col, int32_t n_cols,
                   const int32_t* h_col_a, const int32_t* h_col_b, const int32_t* h_col_sign, const double* h_col_add,
                   double level, double* d_mean, double* d_lo, double* d_hi, int64_t* d_n, void* stream);
+/* K9: split R-hat and "mean" effective sample size (Vehtari et al. 2021, section 3; Stan's and ArviZ's rhat(method="split") and
+ * ess(method="mean")) of every column over the chains of a run, without copying the records.
+ *   rows         row (s, k) at d_rows + (s n_chains ladder + k) row_stride: [sample][chain][record] for the records of K3 / K6 / K7,
+ *                [n_samples n_chains][bins] for the matrices of lr_marginal_rates (ladder 1).  Burn-in: offset the pointer.
+ *   ladder       1..32; T > 1: logical chain c at sample s is the first of the rows (s, cT .. cT + T - 1) with row[beta_col] == 1.0
+ *   columns      the specs of lr_column_hpd (HOST arrays [n_cols]; b, sign, add may be NULL)
+ * Split chains: n = floor(n_samples / 2), split chain 2c = draws [0, n) of chain c, 2c + 1 = draws [n_samples - n, n_samples) (an
+ * odd n_samples drops the middle draw).  A split chain whose draws are all equal has that value as its mean, exactly; the
+ * between-chain variance is exactly 0 when all split-chain means are equal.  Otherwise literate_b200.diagnostics.rhat_ess is the
+ * definition, step for step: W, var+, rho_t, Geyer's initial positive and monotone sequences, tau >= 1/log10(m n).
+ *   d_out        fp64 [5][n_cols]: mean (of the draws used), sd = sqrt(var+), R-hat, ESS, lag (Geyer's max_t, as a double)
+ *   degenerate   a non-finite draw: every output NaN, lag -1; W = 0, var+ = 0 (constant): R-hat NaN, ESS NaN, lag -1;
+ *                W = 0, var+ > 0 (every split chain stuck on its own value): R-hat +inf, ESS NaN, lag -1
+ *   d_status     int64 [1]: (sample, ladder) pairs among the draws used with no member at beta = 1 (0 when ladder = 1)
+ * Sums are compensated and in a fixed order: repeated calls are bit-identical.  The work follows the largest truncation lag
+ * (lag blocks of doubling width, the count of unfinished columns read once per block), so the call returns when the outputs are
+ * written.  Scratch (at most ~256 MB; columns in batches) comes from the handle's workspace.  Rejects bad sizes, fields outside
+ * the row, n_samples < 4 ("not enough data") and more than 2^31 - 1 rows. */
+int lr_chain_diagnostics(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
+                         int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
+                         const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, void* stream);
 
 /* ---------------------------------------------------------------- TrendRate (SURVEY 8 f-4): fixed-dimension chains on the same statistics
  *

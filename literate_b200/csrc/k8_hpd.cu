@@ -61,27 +61,7 @@ __device__ __forceinline__ unsigned long long k8_key(double x) {
 __device__ __forceinline__ double k8_val(unsigned long long k) {
     return __longlong_as_double((long long)((k & K8_SIGN) ? (k ^ K8_SIGN) : ~k));
 }
-// Compensated (Neumaier) sum: the running sum s and the rounding errors c of its additions, so that a mean over millions of rows
-// stays within a few units in the last place of the correctly rounded one (a plain sum in any order drifts by up to n ulp when the
-// rounding errors share a sign, e.g. a column of the values 0.1, 0.2, 0.3).  A sum that became +-inf or NaN stays so and is
-// returned as it is, as a plain sum would.
-struct K8Sum {
-    double s = 0.0, c = 0.0;
-    __device__ __forceinline__ void add(double v) {
-        const double t = __dadd_rn(s, v);
-        c = __dadd_rn(c, fabs(s) >= fabs(v) ? __dadd_rn(__dsub_rn(s, t), v) : __dadd_rn(__dsub_rn(v, t), s));
-        s = t;
-    }
-    __device__ __forceinline__ double value() const { return isfinite(s) ? __dadd_rn(s, c) : s; }
-};
-
-// value of one column in one row: row[a], then +- row[b], then + c -- one fp64 operation each, in this order (what the logs hold)
-__device__ __forceinline__ double k8_value(const double* row, int a, int b, int s, double c) {
-    double v = row[a];
-    if (b >= 0) v = s > 0 ? __dadd_rn(v, row[b]) : __dsub_rn(v, row[b]);
-    if (c != 0.0) v = __dadd_rn(v, c);
-    return v;
-}
+// (k8_value, the value of a column spec in a row, and K8Sum, the compensated sum, live in lr_common.cuh: K9 uses them too)
 
 // pass < 8: histogram of digit `pass` (most significant first) of the keys that share each threshold's prefix so far (pass 0 also
 // writes the partial sums); pass 8: gathers the keys below the lower / above the upper threshold.  grid (slice, group).
@@ -307,12 +287,7 @@ extern "C" int lr_column_hpd(lr_handle_t h, const double* d_rows, int64_t n_rows
     LR_REQUIRE(n_rows >= 0 && n_rows < ((int64_t)1 << 31) && n_cols >= 1 && row_stride >= 1, "lr_column_hpd: bad sizes");
     LR_REQUIRE(mask_col < row_stride, "lr_column_hpd: mask column %d outside the row of %lld doubles", mask_col, (long long)row_stride);
     LR_REQUIRE(level > 0.0 && level <= 1.0, "lr_column_hpd: level must be in (0, 1]");
-    for (int j = 0; j < n_cols; ++j) {
-        const int a = h_col_a[j], b = h_col_b ? h_col_b[j] : -1, s = h_col_sign ? h_col_sign[j] : 1;
-        LR_REQUIRE(a >= 0 && a < row_stride && b >= -1 && b < row_stride && (s == 1 || s == -1),
-                   "lr_column_hpd: column %d = (%d, %d, %d) names a field outside the row of %lld doubles or a sign other than +-1", j, a, b, s,
-                   (long long)row_stride);
-    }
+    { int rc0 = lr_check_col_specs("lr_column_hpd", n_cols, row_stride, h_col_a, h_col_b, h_col_sign); if (rc0 != LR_OK) return rc0; }
     LR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     static bool attr[64] = {};
@@ -331,34 +306,21 @@ extern "C" int lr_column_hpd(lr_handle_t h, const double* d_rows, int64_t n_rows
     const int groups_per_batch = (int)std::max<size_t>(1, std::min<size_t>(std::min(n_groups, 1023), ((size_t)512 << 20) / per_group));
     const int batch_cols = std::min(n_cols, groups_per_batch * K8_G);
     // workspace: column specs, control block, then one batch's buffers
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    const size_t spec_bytes = al((size_t)n_cols * 8) + 3 * al((size_t)n_cols * 4);
+    auto al = lr_align256;
+    const size_t spec_bytes = lr_col_spec_bytes(n_cols);
     const size_t sel_b = al((size_t)batch_cols * 32), hist_b = al((size_t)batch_cols * 2048), part_b = al((size_t)n_slices * batch_cols * 8);
     const size_t cnt_b = al((size_t)batch_cols * 8), where_b = al((size_t)batch_cols * 8), tail_b = al((size_t)2 * batch_cols * m_stride * 8);
     const size_t bytes = spec_bytes + 256 + sel_b + hist_b + part_b + cnt_b + where_b + 2 * tail_b;
     int rc = lr_ws_acquire(h, bytes, st);
     if (rc != LR_OK) return rc;
     char* w = (char*)h->ws;
-    double* cc = (double*)w;
-    int* ca = (int*)(w + al((size_t)n_cols * 8));
-    int* cb = (int*)((char*)ca + al((size_t)n_cols * 4));
-    int* cs = (int*)((char*)cb + al((size_t)n_cols * 4));
-    {
-        // stage the specs in one host block (defaults for the optional arrays) and copy it in one piece
-        char* stage = (char*)calloc(1, spec_bytes);
-        LR_REQUIRE(stage, "lr_column_hpd: out of host memory");
-        double* hc = (double*)stage;
-        int* ha = (int*)(stage + ((char*)ca - w));
-        int* hb = (int*)(stage + ((char*)cb - w));
-        int* hs = (int*)(stage + ((char*)cs - w));
-        for (int j = 0; j < n_cols; ++j) {
-            ha[j] = h_col_a[j]; hb[j] = h_col_b ? h_col_b[j] : -1; hs[j] = h_col_sign ? h_col_sign[j] : 1;
-            hc[j] = h_col_add ? h_col_add[j] : 0.0;
-        }
-        const cudaError_t e = cudaMemcpyAsync(w, stage, spec_bytes, cudaMemcpyHostToDevice, st);      // pageable: staged before return
-        free(stage);
-        LR_CUDA(e);
-    }
+    lr_col_specs spec;
+    rc = lr_stage_col_specs("lr_column_hpd", w, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st, &spec);
+    if (rc != LR_OK) return rc;
+    double* cc = spec.add;
+    int* ca = spec.a;
+    int* cb = spec.b;
+    int* cs = spec.sign;
     K8Args p;
     memset(&p, 0, sizeof(p));
     p.rows = d_rows; p.n_rows = n_rows; p.stride = row_stride; p.mask_col = mask_col;

@@ -237,6 +237,72 @@ inline int lr_upload_bin_stats(lr_handle_t h, size_t cnt, const int64_t* h_sp, c
     return LR_OK;
 }
 
+// ---- column specs of the record consumers (K8 lr_column_hpd, K9 lr_chain_diagnostics) --------------------------------------------
+// Output column j of a row is row[a_j], then + or - row[b_j] (b_j >= 0, sign_j = +-1), then + add_j (if non-zero): one fp64 operation
+// each, in this order -- what the logs hold (the net rate l_j - m_j, DDRate's midpoint_x0 and maxCarryingCap).
+__device__ __forceinline__ double k8_value(const double* row, int a, int b, int s, double c) {
+    double v = row[a];
+    if (b >= 0) v = s > 0 ? __dadd_rn(v, row[b]) : __dsub_rn(v, row[b]);
+    if (c != 0.0) v = __dadd_rn(v, c);
+    return v;
+}
+// Compensated (Neumaier) sum: the running sum s and the rounding errors c of its additions, so that a mean over millions of rows
+// stays within a few units in the last place of the correctly rounded one (a plain sum in any order drifts by up to n ulp when the
+// rounding errors share a sign, e.g. a column of the values 0.1, 0.2, 0.3).  A sum that became +-inf or NaN stays so and is
+// returned as it is, as a plain sum would.
+struct K8Sum {
+    double s = 0.0, c = 0.0;
+    __device__ __forceinline__ void add(double v) {
+        const double t = __dadd_rn(s, v);
+        c = __dadd_rn(c, fabs(s) >= fabs(v) ? __dadd_rn(__dsub_rn(s, t), v) : __dadd_rn(__dsub_rn(v, t), s));
+        s = t;
+    }
+    __device__ __forceinline__ double value() const { return isfinite(s) ? __dadd_rn(s, c) : s; }
+};
+
+inline size_t lr_align256(size_t x) { return (x + 255) & ~(size_t)255; }
+// bytes of the staged specs at the start of the workspace: add [n] fp64, then a, b, sign [n] int32, each 256-byte aligned
+inline size_t lr_col_spec_bytes(int n_cols) { return lr_align256((size_t)n_cols * 8) + 3 * lr_align256((size_t)n_cols * 4); }
+struct lr_col_specs { double* add; int* a; int* b; int* sign; };
+
+// every field inside the row and every sign +-1 (b, sign and add may be NULL: -1, 1, 0)
+inline int lr_check_col_specs(const char* who, int n_cols, int64_t row_stride, const int32_t* h_col_a, const int32_t* h_col_b,
+                              const int32_t* h_col_sign) {
+    for (int j = 0; j < n_cols; ++j) {
+        const int a = h_col_a[j], b = h_col_b ? h_col_b[j] : -1, s = h_col_sign ? h_col_sign[j] : 1;
+        LR_REQUIRE(a >= 0 && a < row_stride && b >= -1 && b < row_stride && (s == 1 || s == -1),
+                   "%s: column %d = (%d, %d, %d) names a field outside the row of %lld doubles or a sign other than +-1", who, j, a, b, s,
+                   (long long)row_stride);
+    }
+    return LR_OK;
+}
+
+// the specs, staged in one host block (defaults for the optional arrays) and copied to `w` (device) in one piece on `st`; the
+// copy is from pageable memory, so it has been staged when this returns
+inline int lr_stage_col_specs(const char* who, void* w, int n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
+                              const int32_t* h_col_sign, const double* h_col_add, cudaStream_t st, lr_col_specs* out) {
+    const size_t bytes = lr_col_spec_bytes(n_cols);
+    char* base = (char*)w;
+    out->add = (double*)base;
+    out->a = (int*)(base + lr_align256((size_t)n_cols * 8));
+    out->b = (int*)((char*)out->a + lr_align256((size_t)n_cols * 4));
+    out->sign = (int*)((char*)out->b + lr_align256((size_t)n_cols * 4));
+    char* stage = (char*)calloc(1, bytes);
+    LR_REQUIRE(stage, "%s: out of host memory", who);
+    double* hc = (double*)stage;
+    int* ha = (int*)(stage + ((char*)out->a - base));
+    int* hb = (int*)(stage + ((char*)out->b - base));
+    int* hs = (int*)(stage + ((char*)out->sign - base));
+    for (int j = 0; j < n_cols; ++j) {
+        ha[j] = h_col_a[j]; hb[j] = h_col_b ? h_col_b[j] : -1; hs[j] = h_col_sign ? h_col_sign[j] : 1;
+        hc[j] = h_col_add ? h_col_add[j] : 0.0;
+    }
+    const cudaError_t e = cudaMemcpyAsync(w, stage, bytes, cudaMemcpyHostToDevice, st);
+    free(stage);
+    LR_CUDA(e);
+    return LR_OK;
+}
+
 // ---- small device helpers --------------------------------------------------------------------
 __device__ __forceinline__ double2 ld_stream_f64x2(const double2* p) {
     double2 v;

@@ -308,6 +308,42 @@ class Device:
             raise RuntimeError("not enough data")
         return out[0], out[1], out[2], n
 
+    def chain_diagnostics_device(self, records, cols, ladder=1, beta_col=-1, stream=None):
+        """Split R-hat and effective sample size of columns over the chains of a run (K9, lr_chain_diagnostics), without copying
+        the records; diagnostics.rhat_ess is the definition.
+
+        records: float64 CUDA tensor [n_samples, n_chains * ladder, w] with contiguous rows (the post-burn-in samples of a run, or
+        a matrix [n_samples, n_chains, bins]); cols: specs as for column_hpd_device.  ladder > 1: chains are ladders of `ladder`
+        consecutive members and the member whose field beta_col holds 1.0 at a sample is the chain's draw.  Returns a dict of
+        float64 CUDA tensors [n_cols]: mean, sd, rhat, ess, lag.  Raises RuntimeError("not enough data") for fewer than 4 samples
+        and ValueError when a ladder has no member at beta = 1 at some sample.  Returns when the outputs are written."""
+        import torch
+        if not (records.is_cuda and records.dtype == torch.float64 and records.dim() == 3 and records.stride(2) == 1
+                and records.stride(0) == records.shape[1] * records.stride(1)):
+            raise ValueError("records must be a float64 CUDA tensor [n_samples, n_chains * ladder, w] with evenly spaced contiguous rows")
+        S, nk, w = records.shape
+        if S < 4:
+            raise RuntimeError("not enough data")
+        if ladder < 1 or nk % ladder:
+            raise ValueError("the chains of records must be whole ladders of %d" % ladder)
+        spec = [(c, -1, 1, 0.0) if np.ndim(c) == 0 else (tuple(c) + (0.0,))[:4] for c in cols]
+        if not spec:
+            raise ValueError("no columns")
+        a = np.ascontiguousarray([s[0] for s in spec], dtype=np.int32)
+        b = np.ascontiguousarray([s[1] for s in spec], dtype=np.int32)
+        sg = np.ascontiguousarray([s[2] for s in spec], dtype=np.int32)
+        add = np.ascontiguousarray([s[3] for s in spec], dtype=np.float64)
+        stride = records.stride(1) if S * nk > 1 else w
+        out = torch.empty((5, len(spec)), dtype=torch.float64, device=records.device)
+        status = torch.zeros(1, dtype=torch.int64, device=records.device)
+        N.check(self.lib.lr_chain_diagnostics(self.h, C.c_void_p(records.data_ptr()), int(S), int(nk // ladder), int(ladder), int(beta_col),
+                                              int(stride), len(spec), N.np_ptr(a), N.np_ptr(b), N.np_ptr(sg), N.np_ptr(add),
+                                              C.c_void_p(out.data_ptr()), C.c_void_p(status.data_ptr()), _stream_ptr(stream, records.device)),
+                "lr_chain_diagnostics")
+        if ladder > 1 and int(status.item()):
+            raise ValueError("a ladder has no chain at beta = 1 (%d samples)" % int(status.item()))
+        return dict(zip(("mean", "sd", "rhat", "ess", "lag"), out))
+
     def new_accumulators(self, n_rep, n_bins, device):
         import torch
         return torch.zeros((n_rep, N.LR_ACC_ROWS, int(self.lib.lr_acc_stride(int(n_bins)))), dtype=torch.int64, device=device)
