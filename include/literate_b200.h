@@ -354,6 +354,27 @@ int lr_column_hpd(lr_handle_t h, const double* d_rows, int64_t n_rows, int64_t r
 int lr_chain_diagnostics(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
                          int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
                          const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, void* stream);
+/* K10: rank-normalised split R-hat and bulk and tail effective sample sizes (Vehtari et al. 2021; ArviZ's rhat(method="rank"),
+ * ess(method="bulk"), ess(method="tail")) of every column over the chains of a run, without copying the records.  Rows, ladder,
+ * columns, d_status and the split of lr_chain_diagnostics; n = floor(n_samples / 2), N = 2 n n_chains split draws per column.
+ * literate_b200.diagnostics.rank_rhat_ess is the definition.
+ * lr_rank_transform writes
+ *   d_z          fp64 [2n][n_chains][4 n_cols]: row i n_chains + c holds split draw i of chain c (i >= n: draw n_samples - 2n + i);
+ *                slot q n_cols + j of column j: q = 0 z = Phi^-1((r - 3/8) / (N + 1/4)) of the draw's average rank r (1-based)
+ *                among the N split draws, q = 1 the same of |x - median|, q = 2 / 3 the indicator x <= q05 / x <= q95 (0.0 / 1.0)
+ *   d_quant      fp64 [3][n_cols]: median of the split draws (np.median), q05 and q95 of all n_samples n_chains draws
+ *                (np.quantile, method "linear"), bit for bit as numpy computes them up to the sign of a zero (NaN if a NaN is among them)
+ * lr_rank_diagnostics writes d_out fp64 [8][n_cols]: median, q05, q95, rhat_bulk, rhat_tail, rhat_rank, ess_bulk, ess_tail; every
+ * output NaN for a column lr_chain_diagnostics finds non-finite, constant or stuck.  Ties get their average rank; -0 ranks as +0.
+ * Scratch comes from the handle's workspace: at most ~1 GiB of K10 buffers (columns in batches, at least one column per batch)
+ * plus lr_chain_diagnostics' own.  Repeated calls are bit-identical.  lr_rank_transform is asynchronous on `stream`;
+ * lr_rank_diagnostics returns when its outputs are written.  Rejects what lr_chain_diagnostics rejects, under its own name. */
+int lr_rank_transform(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
+                      int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b, const int32_t* h_col_sign,
+                      const double* h_col_add, double* d_z, double* d_quant, int64_t* d_status, void* stream);
+int lr_rank_diagnostics(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
+                        int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b, const int32_t* h_col_sign,
+                        const double* h_col_add, double* d_out, int64_t* d_status, void* stream);
 
 /* ---------------------------------------------------------------- TrendRate (SURVEY 8 f-4): fixed-dimension chains on the same statistics
  *

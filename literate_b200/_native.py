@@ -38,7 +38,7 @@ EXPORTS = [
     "lr_dd_create", "lr_dd_create_host", "lr_dd_destroy", "lr_dd_record_doubles", "lr_dd_records_per_run",
     "lr_dd_run", "lr_dd_run_host", "lr_dd_eval_host", "lr_dd_state_host",
     "lr_dd_set_beta_host", "lr_dd_swap_info", "lr_dd_swap_apply", "lr_dd_swap_step", "lr_dd_temper_host",
-    "lr_column_hpd", "lr_chain_diagnostics",
+    "lr_column_hpd", "lr_chain_diagnostics", "lr_rank_transform", "lr_rank_diagnostics",
 ]
 
 
@@ -124,6 +124,8 @@ def load(build_if_missing=False):
     sig("lr_marginal_rates", C.c_int, vp, vp, i64, f64, i32, i32, i32, vp, vp, vp)
     sig("lr_column_hpd", C.c_int, vp, vp, i64, i64, i32, i32, vp, vp, vp, vp, f64, vp, vp, vp, vp, vp)
     sig("lr_chain_diagnostics", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, vp, vp, vp, vp, vp, vp, vp)
+    sig("lr_rank_transform", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, vp, vp, vp, vp, vp, vp, vp, vp)
+    sig("lr_rank_diagnostics", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, vp, vp, vp, vp, vp, vp, vp)
     sig("lr_trend_create", C.c_int, vp, i32, i32, vp, vp, vp, vp, i32, i32, i32, u64, i64, vp, vp, P(vp))
     sig("lr_trend_create_host", C.c_int, vp, i32, i32, vp, vp, vp, vp, i32, i32, i32, u64, i64, vp, P(vp))
     sig("lr_trend_destroy", C.c_int, vp)

@@ -15,7 +15,7 @@ REPO = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 OUT_DIR = os.path.join(PKG, "_lib")
 LIB = os.path.join(OUT_DIR, "libliterate_b200.so")
-SOURCES = ["lr_api.cu", "k1_binstats.cu", "k3_chains.cu", "k4_direct.cu", "k5_summary.cu", "k6_trend.cu", "k7_ddrate.cu", "k8_hpd.cu", "k9_diag.cu"]
+SOURCES = ["lr_api.cu", "k1_binstats.cu", "k3_chains.cu", "k4_direct.cu", "k5_summary.cu", "k6_trend.cu", "k7_ddrate.cu", "k8_hpd.cu", "k9_diag.cu", "k10_rank.cu"]
 HEADERS = ["lr_common.cuh", "chain_device.cuh", "k3_team.cuh", os.path.join(REPO, "include", "literate_b200.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "-Xptxas", "-v"] + os.environ.get("LR_EXTRA_NVCC_FLAGS", "").split()

@@ -27,7 +27,6 @@ constexpr int K8_HB = 257;                  // padded bins per histogram row: ba
 constexpr int K8_PASS_SMEM = 2 * K8_G * K8_HB * 4 + K8_WARPS * K8_G * 8;
 constexpr int K8_SORT_WARPS = 16;
 constexpr int K8_WIN_THREADS = 256;
-constexpr unsigned long long K8_SIGN = 0x8000000000000000ull;
 
 struct K8Ctrl { long long n, n_in, m; int ok; };
 
@@ -52,16 +51,8 @@ struct K8Args {
     double* mean; double* lo; double* hi; long long* n_out;
 };
 
-// order-preserving key: negative values bit-inverted, the sign bit set on the others; every NaN -> the largest key
-__device__ __forceinline__ unsigned long long k8_key(double x) {
-    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
-    if (x != x) return ~0ull;
-    return (b & K8_SIGN) ? ~b : (b | K8_SIGN);
-}
-__device__ __forceinline__ double k8_val(unsigned long long k) {
-    return __longlong_as_double((long long)((k & K8_SIGN) ? (k ^ K8_SIGN) : ~k));
-}
-// (k8_value, the value of a column spec in a row, and K8Sum, the compensated sum, live in lr_common.cuh: K9 uses them too)
+// (k8_key / k8_val, the order-preserving keys, k8_value, the value of a column spec in a row, and K8Sum, the compensated sum,
+// live in lr_common.cuh: K9 and K10 use them too)
 
 // pass < 8: histogram of digit `pass` (most significant first) of the keys that share each threshold's prefix so far (pass 0 also
 // writes the partial sums); pass 8: gathers the keys below the lower / above the upper threshold.  grid (slice, group).

@@ -271,34 +271,32 @@ void k9_launch_lag(const K9Args& p, int groups, long long t0, long long t1, int 
 
 }  // namespace
 
-extern "C" int lr_chain_diagnostics(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
-                                    int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
-                                    const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, void* stream) {
-    LR_REQUIRE(h && d_out && d_status && h_col_a && d_rows, "lr_chain_diagnostics: null pointer");
-    LR_REQUIRE(n_samples >= 4, "lr_chain_diagnostics: not enough data (%lld samples per chain; at least 4)", (long long)n_samples);
-    LR_REQUIRE(n_chains >= 1 && ladder >= 1 && ladder <= 32 && n_cols >= 1 && row_stride >= 1,
-               "lr_chain_diagnostics: bad sizes (n_chains >= 1, ladder 1..32, n_cols >= 1, row_stride >= 1)");
-    LR_REQUIRE(n_samples * n_chains * ladder < ((int64_t)1 << 31), "lr_chain_diagnostics: %lld rows; at most 2^31 - 1",
-               (long long)(n_samples * n_chains * ladder));
-    LR_REQUIRE(ladder == 1 || (beta_col >= 0 && beta_col < row_stride),
-               "lr_chain_diagnostics: beta column %d outside the row of %lld doubles", beta_col, (long long)row_stride);
-    { int rc0 = lr_check_col_specs("lr_chain_diagnostics", n_cols, row_stride, h_col_a, h_col_b, h_col_sign); if (rc0 != LR_OK) return rc0; }
-    LR_CUDA(cudaSetDevice(h->device));
-    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-    const long long n = n_samples / 2, m = 2 * n_chains;
-    // columns per batch: the per split chain moments (20 B) and the partial lag sums of a column within ~256 MB
+// columns per batch: the per split chain moments (20 B) and the partial lag sums of a column within ~256 MB
+static int k9_batch_cols(long long m, int n_cols) {
     const size_t per_col = (size_t)m * 20 + (size_t)K9_PART_LAGS * 8 + sizeof(K9Col) + 4;
-    const int batch_cols = (int)std::max<size_t>(1, std::min<size_t>((size_t)n_cols, ((size_t)256 << 20) / per_col));
+    return (int)std::max<size_t>(1, std::min<size_t>((size_t)n_cols, ((size_t)256 << 20) / per_col));
+}
+
+size_t lr_k9_scratch_bytes(int64_t n_chains, int32_t n_cols) {
+    const long long m = 2 * n_chains;
+    const int batch_cols = k9_batch_cols(m, n_cols);
+    auto al = lr_align256;
+    const size_t sum_b = al((size_t)m * batch_cols * 8), flag_b = al((size_t)m * batch_cols * 4);
+    const size_t part_b = al((size_t)K9_PART_LAGS * batch_cols * 8), col_b = al(sizeof(K9Col) * batch_cols), done_b = al((size_t)batch_cols * 4);
+    return lr_col_spec_bytes(n_cols) + 256 + 2 * sum_b + flag_b + part_b + col_b + done_b;
+}
+
+int lr_k9_run(lr_handle_t h, char* w, const char* who, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder,
+              int32_t beta_col, int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
+              const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, cudaStream_t st) {
+    const long long n = n_samples / 2, m = 2 * n_chains;
+    const int batch_cols = k9_batch_cols(m, n_cols);
     auto al = lr_align256;
     const size_t spec_bytes = lr_col_spec_bytes(n_cols);
     const size_t sum_b = al((size_t)m * batch_cols * 8), flag_b = al((size_t)m * batch_cols * 4);
-    const size_t part_b = al((size_t)K9_PART_LAGS * batch_cols * 8), col_b = al(sizeof(K9Col) * batch_cols), done_b = al((size_t)batch_cols * 4);
-    const size_t bytes = spec_bytes + 256 + 2 * sum_b + flag_b + part_b + col_b + done_b;
-    int rc = lr_ws_acquire(h, bytes, st);
-    if (rc != LR_OK) return rc;
-    char* w = (char*)h->ws;
+    const size_t part_b = al((size_t)K9_PART_LAGS * batch_cols * 8), col_b = al(sizeof(K9Col) * batch_cols);
     lr_col_specs spec;
-    rc = lr_stage_col_specs("lr_chain_diagnostics", w, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st, &spec);
+    int rc = lr_stage_col_specs(who, w, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st, &spec);
     if (rc != LR_OK) return rc;
     K9Args p;
     memset(&p, 0, sizeof(p));
@@ -347,10 +345,30 @@ extern "C" int lr_chain_diagnostics(lr_handle_t h, const double* d_rows, int64_t
             LR_CUDA(cudaMemcpyAsync(&fin, p.finished, sizeof(unsigned), cudaMemcpyDeviceToHost, st));
             LR_CUDA(cudaStreamSynchronize(st));
             if ((int)fin >= p.n_cols) break;
-            LR_REQUIRE(t1 < n, "lr_chain_diagnostics: %d columns unfinished after every lag (internal error)", p.n_cols - (int)fin);
+            LR_REQUIRE(t1 < n, "%s: %d columns unfinished after every lag (internal error)", who, p.n_cols - (int)fin);
             t0 = t1;
             width = std::min(2 * width, K9_MAX_BLOCK);
         }
     }
     return LR_OK;
+}
+
+extern "C" int lr_chain_diagnostics(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
+                                    int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
+                                    const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, void* stream) {
+    LR_REQUIRE(h && d_out && d_status && h_col_a && d_rows, "lr_chain_diagnostics: null pointer");
+    LR_REQUIRE(n_samples >= 4, "lr_chain_diagnostics: not enough data (%lld samples per chain; at least 4)", (long long)n_samples);
+    LR_REQUIRE(n_chains >= 1 && ladder >= 1 && ladder <= 32 && n_cols >= 1 && row_stride >= 1,
+               "lr_chain_diagnostics: bad sizes (n_chains >= 1, ladder 1..32, n_cols >= 1, row_stride >= 1)");
+    LR_REQUIRE(n_samples * n_chains * ladder < ((int64_t)1 << 31), "lr_chain_diagnostics: %lld rows; at most 2^31 - 1",
+               (long long)(n_samples * n_chains * ladder));
+    LR_REQUIRE(ladder == 1 || (beta_col >= 0 && beta_col < row_stride),
+               "lr_chain_diagnostics: beta column %d outside the row of %lld doubles", beta_col, (long long)row_stride);
+    { int rc0 = lr_check_col_specs("lr_chain_diagnostics", n_cols, row_stride, h_col_a, h_col_b, h_col_sign); if (rc0 != LR_OK) return rc0; }
+    LR_CUDA(cudaSetDevice(h->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
+    int rc = lr_ws_acquire(h, lr_k9_scratch_bytes(n_chains, n_cols), st);
+    if (rc != LR_OK) return rc;
+    return lr_k9_run(h, (char*)h->ws, "lr_chain_diagnostics", d_rows, n_samples, n_chains, ladder, beta_col, row_stride, n_cols,
+                     h_col_a, h_col_b, h_col_sign, h_col_add, d_out, d_status, st);
 }

@@ -237,7 +237,7 @@ inline int lr_upload_bin_stats(lr_handle_t h, size_t cnt, const int64_t* h_sp, c
     return LR_OK;
 }
 
-// ---- column specs of the record consumers (K8 lr_column_hpd, K9 lr_chain_diagnostics) --------------------------------------------
+// ---- column specs of the record consumers (K8 lr_column_hpd, K9 lr_chain_diagnostics, K10 lr_rank_*) -----------------------------
 // Output column j of a row is row[a_j], then + or - row[b_j] (b_j >= 0, sign_j = +-1), then + add_j (if non-zero): one fp64 operation
 // each, in this order -- what the logs hold (the net rate l_j - m_j, DDRate's midpoint_x0 and maxCarryingCap).
 __device__ __forceinline__ double k8_value(const double* row, int a, int b, int s, double c) {
@@ -245,6 +245,15 @@ __device__ __forceinline__ double k8_value(const double* row, int a, int b, int 
     if (b >= 0) v = s > 0 ? __dadd_rn(v, row[b]) : __dsub_rn(v, row[b]);
     if (c != 0.0) v = __dadd_rn(v, c);
     return v;
+}
+// order-preserving key of a double: negative values bit-inverted, the sign bit set on the others; every NaN -> the largest key
+__device__ __forceinline__ unsigned long long k8_key(double x) {
+    const unsigned long long b = (unsigned long long)__double_as_longlong(x);
+    if (x != x) return ~0ull;
+    return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
+}
+__device__ __forceinline__ double k8_val(unsigned long long k) {
+    return __longlong_as_double((long long)((k & 0x8000000000000000ull) ? (k ^ 0x8000000000000000ull) : ~k));
 }
 // Compensated (Neumaier) sum: the running sum s and the rounding errors c of its additions, so that a mean over millions of rows
 // stays within a few units in the last place of the correctly rounded one (a plain sum in any order drifts by up to n ulp when the
@@ -302,6 +311,14 @@ inline int lr_stage_col_specs(const char* who, void* w, int n_cols, const int32_
     LR_CUDA(e);
     return LR_OK;
 }
+
+// ---- K9's host driver on a caller's scratch (k9_diag.cu): lr_chain_diagnostics runs it on the workspace, K10 on the part of the
+// workspace behind its own buffers.  lr_k9_scratch_bytes is what lr_k9_run uses from `w` (at most ~256 MB beyond the staged
+// specs); the arguments are those of lr_chain_diagnostics, already checked, `who` names the entry point in errors.
+size_t lr_k9_scratch_bytes(int64_t n_chains, int32_t n_cols);
+int lr_k9_run(lr_handle_t h, char* w, const char* who, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder,
+              int32_t beta_col, int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
+              const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, cudaStream_t st);
 
 // ---- small device helpers --------------------------------------------------------------------
 __device__ __forceinline__ double2 ld_stream_f64x2(const double2* p) {

@@ -7,8 +7,11 @@ in Tracer one log at a time ("ESS >= 200 per parameter"), for thousands of chain
   diagnostic_columns        the (name, record spec) list of a sampler's records, in log column order
   diagnose_records_device   K9 on device-resident records (RJMCMC: plus the per-bin marginal rates of K5's matrices)
   diagnose_logs             K9 on the post-burn-in rows of sample logs, one log per chain
+  rank_rhat_ess             host restatement of the rank-normalised R-hat and bulk and tail ESS (Vehtari et al. 2021, section
+                            4; ArviZ's rhat(method="rank"), ess(method="bulk" / "tail")): the definition K10
+                            (lr_rank_diagnostics) computes; diagnose_records_device and diagnose_logs add it with rank=True
 
-  python -m literate_b200.diagnose <dir> [-burnin .2] [-rhat_max 1.01] [-ess_min 200] [-device 0]
+  python -m literate_b200.diagnose <dir> [-burnin .2] [-rhat_max 1.01] [-ess_min 200] [-device 0] [-rank 0]
 """
 from __future__ import annotations
 
@@ -119,6 +122,99 @@ def rhat_ess_columns(x):
     return {k: np.array([r[k] for r in rows]) for k in ("mean", "sd", "rhat", "ess", "lag", "margin")}
 
 
+def _split(x):
+    x = np.asarray(x, dtype=np.float64)
+    if x.ndim == 1:
+        x = x[None, :]
+    M, Sd = x.shape
+    if Sd < 4:
+        raise RuntimeError("not enough data")
+    n = Sd // 2
+    return x, np.concatenate([x[:, :n], x[:, Sd - n:]], axis=1)
+
+
+def rank_normal(v):
+    """Phi^-1((r - 3/8) / (N + 1/4)) of the average ranks r (1-based, ties averaged) of the N values v, any shape.  The ratio and
+    its complement (N + 5/8 - r) / (N + 1/4) have exact numerators; the smaller one goes to ndtri, so that the most extreme ranks
+    of millions of draws keep full precision (ndtri(1 - eps) cannot)."""
+    from scipy.special import ndtri
+    from scipy.stats import rankdata
+    v = np.asarray(v, dtype=np.float64)
+    r = rankdata(v.ravel(), method="average").reshape(v.shape)
+    N = v.size
+    num, rest, den = r - 0.375, N + 0.625 - r, N + 0.25
+    return np.where(num <= rest, ndtri(num / den), -ndtri(rest / den))
+
+
+def quantile_linear(x, p):
+    """np.quantile(x, p) with numpy's default "linear" method, restated step for step as K10 computes it: h = (N - 1) p,
+    lo = floor(h), g = h - lo; a + (b - a) g when g < 0.5, else b - (b - a)(1 - g); NaN if x holds a NaN."""
+    v = np.sort(np.asarray(x, dtype=np.float64).ravel())
+    if np.isnan(v[-1]):
+        return float("nan")
+    N = v.size
+    h = (N - 1) * p
+    if h >= N - 1:
+        a = b = v[-1]
+        g = h + 1.0
+    else:
+        lo = math.floor(h)
+        a, b, g = v[lo], v[lo + 1], h - lo
+    d = b - a
+    return float(b - d * (1.0 - g)) if g >= 0.5 else float(a + d * g)
+
+
+def rank_rhat_ess(x):
+    """Rank-normalised split R-hat and bulk and tail ESS of one column x [chains M, draws S] -> dict of floats median, q05, q95,
+    rhat_bulk, rhat_tail, rhat_rank, ess_bulk, ess_tail and margin (host only: the smallest margin of the four rhat_ess calls).
+    ArviZ's _rhat_rank, _ess_bulk and _ess_tail in the order they compute:
+
+      1. n = S // 2, N = 2 M n; xs [M, 2n] = draws [0, n) and [S - n, S) of each chain (an odd S drops the middle draw, as
+         rhat_ess does), so that rhat_ess(xs-shaped matrix) splits it into exactly these 2M split chains.  S < 4: RuntimeError.
+      2. rhat_ess(x) non-finite, constant or stuck: every output NaN (+-inf draws included).
+      3. z = Phi^-1((r - 3/8) / (N + 1/4)) of the average ranks r of xs among the N split draws (rank_normal);
+         rhat_bulk, ess_bulk = rhat_ess(z).
+      4. median = np.median(xs) ((a + b) / 2 of the middle two, N is even); f = |xs - median|; rhat_tail = rhat_ess(z of f)
+         (NaN when f is constant, e.g. a 0/1 column split exactly in half).
+      5. rhat_rank = max(rhat_bulk, rhat_tail), a NaN rhat_tail ignored (a stuck z of f gives +inf, which wins).
+      6. q_p = np.quantile(x, p) over all M S draws (middle draws included; quantile_linear) for p = 0.05, 0.95; I_p = (xs <= q_p)
+         as 0.0 / 1.0; ESS_p = rhat_ess(I_p)["ess"], N when I_p is constant (as ArviZ), NaN when it is stuck;
+         ess_tail = min(ESS_0.05, ESS_0.95), NaN if either is.
+    One chain (M = 1) is allowed, as in rhat_ess; ArviZ returns NaN for its rank R-hat instead."""
+    x, xs = _split(x)
+    nan = float("nan")
+    keys = ("median", "q05", "q95", "rhat_bulk", "rhat_tail", "rhat_rank", "ess_bulk", "ess_tail")
+    base = rhat_ess(x)
+    if not math.isfinite(base["rhat"]):
+        out = dict.fromkeys(keys, nan)
+        out["margin"] = math.inf
+        return out
+    N = xs.size
+    bulk = rhat_ess(rank_normal(xs))
+    med = float(np.median(xs))
+    tail = rhat_ess(rank_normal(np.abs(xs - med)))
+    rb, rt = bulk["rhat"], tail["rhat"]
+    margins = [bulk["margin"], tail["margin"]]
+    q, ess = [], []
+    for p in (0.05, 0.95):
+        qp = quantile_linear(x, p)
+        ind = rhat_ess((xs <= qp).astype(np.float64))
+        const = math.isnan(ind["rhat"])
+        ess.append(float(N) if const else ind["ess"])
+        margins.append(ind["margin"])
+        q.append(qp)
+    return {"median": med, "q05": q[0], "q95": q[1], "rhat_bulk": rb, "rhat_tail": rt,
+            "rhat_rank": rb if math.isnan(rt) else max(rb, rt), "ess_bulk": bulk["ess"],
+            "ess_tail": nan if math.isnan(ess[0]) or math.isnan(ess[1]) else min(ess), "margin": min(margins)}
+
+
+def rank_rhat_ess_columns(x):
+    """rank_rhat_ess of every column of x [draws, chains, columns] -> dict of arrays."""
+    x = np.asarray(x, dtype=np.float64)
+    rows = [rank_rhat_ess(x[:, :, j].T) for j in range(x.shape[2])]
+    return {k: np.array([r[k] for r in rows]) for k in rows[0]}
+
+
 def flag(rhat, ess, lag, mean, rhat_max=1.01, ess_min=200.0):
     """ok | rhat | ess | rhat+ess | const | stuck | nonfinite of one column's diagnostics (lag is -1 for these three, but also for
     a regular column of fewer than 10 draws per chain, where Geyer's sequence stops at once)."""
@@ -186,6 +282,15 @@ class Diagnostics:
     lag: np.ndarray               # int, -1 for degenerate columns
     n_chains: int
     n_draws: int                  # per chain, after the burn-in
+    # rank-normalised diagnostics (rank_rhat_ess; None unless asked for)
+    median: np.ndarray = None
+    q05: np.ndarray = None
+    q95: np.ndarray = None
+    rhat_bulk: np.ndarray = None
+    rhat_tail: np.ndarray = None
+    rhat_rank: np.ndarray = None
+    ess_bulk: np.ndarray = None
+    ess_tail: np.ndarray = None
 
     @property
     def mcse(self):
@@ -194,6 +299,27 @@ class Diagnostics:
 
     def flags(self, rhat_max=1.01, ess_min=200.0):
         return [flag(r, e, l, m, rhat_max, ess_min) for r, e, l, m in zip(self.rhat, self.ess, self.lag, self.mean)]
+
+    def rank_flags(self, rhat_max=1.01, ess_min=200.0):
+        """The flags of the rank diagnostics, in the vocabulary of FLAGS: const, stuck and nonfinite as flags() gives them; else
+        rhat when rhat_rank > rhat_max, ess when min(ess_bulk, ess_tail) < ess_min or ess_tail is NaN."""
+        out = []
+        for fl, rr, eb, et in zip(self.flags(rhat_max, ess_min), self.rhat_rank, self.ess_bulk, self.ess_tail):
+            if fl in ("const", "stuck", "nonfinite"):
+                out.append(fl)
+                continue
+            bad = [tag for tag, b in (("rhat", rr > rhat_max), ("ess", math.isnan(et) or min(eb, et) < ess_min)) if b]
+            out.append("+".join(bad) if bad else "ok")
+        return out
+
+    def write_rank_tsv(self, path, rhat_max=1.01, ess_min=200.0):
+        """column median q05 q95 rhat_rank rhat_bulk rhat_tail ess_bulk ess_tail flag: one row per column, values as repr."""
+        with open(path, "w") as fh:
+            fh.write("column\tmedian\tq05\tq95\trhat_rank\trhat_bulk\trhat_tail\tess_bulk\tess_tail\tflag\n")
+            cols = (self.median, self.q05, self.q95, self.rhat_rank, self.rhat_bulk, self.rhat_tail, self.ess_bulk, self.ess_tail)
+            for i, fl in enumerate(self.rank_flags(rhat_max, ess_min)):
+                fh.write("\t".join([self.names[i]] + [repr(float(v[i])) for v in cols] + [fl]) + "\n")
+        return path
 
     def write_tsv(self, path, rhat_max=1.01, ess_min=200.0):
         """column mean sd rhat ess mcse lag flag: one row per column, values as repr (nan, inf)."""
@@ -205,9 +331,13 @@ class Diagnostics:
         return path
 
 
-def _pack(kind, names, parts, n_chains, n_draws):
+def _pack(kind, names, parts, n_chains, n_draws, rank_parts=None):
     cat = {k: np.concatenate([p[k].cpu().numpy() for p in parts]) for k in ("mean", "sd", "rhat", "ess", "lag")}
-    return Diagnostics(kind, list(names), cat["mean"], cat["sd"], cat["rhat"], cat["ess"], cat["lag"].astype(np.int64), n_chains, n_draws)
+    d = Diagnostics(kind, list(names), cat["mean"], cat["sd"], cat["rhat"], cat["ess"], cat["lag"].astype(np.int64), n_chains, n_draws)
+    if rank_parts is not None:
+        for k in E.RANK_FIELDS:
+            setattr(d, k, np.concatenate([p[k].cpu().numpy() for p in rank_parts]))
+    return d
 
 
 # ------------------------------------------------------------------------------------------ device records
@@ -224,13 +354,14 @@ def cold_records_device(records, ladder, col):
     return torch.gather(r, 2, idx[:, :, None, None].expand(Sn, nc // ladder, 1, w))[:, :, 0, :]
 
 
-def diagnose_records_device(dev, records, kind, n_bins, burnin=0.2, ladder=1, origin=0.0, bins=True, genre=False):
+def diagnose_records_device(dev, records, kind, n_bins, burnin=0.2, ladder=1, origin=0.0, bins=True, genre=False, rank=False):
     """K9 on a float64 CUDA tensor of records [n_samples, n_chains * ladder, rec_doubles] of K3 ("forward"), K6 ("trendrate") or
     K7 ("dd"): the columns of diagnostic_columns after removing the burn-in of every chain -> Diagnostics.  ladder > 1: tempered
     ladders, diagnosed over their cold members (K6 / K7: K9 picks them; K3: gathered on the device first).  origin: the run's
     origin (DDRate's midpoint_x0; RJMCMC: the first bin edge, the run's start time).  bins (forward): the per-bin birth, death and
     net marginal rates l_j, m_j, net_j of n_bins unit bins from origin, from lr_marginal_rates matrices in chunks of at most 1 GB,
-    as summary.summarize_records_device expands them."""
+    as summary.summarize_records_device expands them.  rank: the rank-normalised diagnostics too (K10 on the same columns, the
+    Diagnostics fields median .. ess_tail)."""
     b0 = S.burnin_index(records.shape[0], burnin)
     post = records[b0:]
     cols = diagnostic_columns(kind, n_bins, origin, genre)
@@ -239,29 +370,38 @@ def diagnose_records_device(dev, records, kind, n_bins, burnin=0.2, ladder=1, or
     if kind != "forward":
         beta = TR.REC_BETA if kind == "trendrate" else DD.REC_BETA
         out = dev.chain_diagnostics_device(post, specs, ladder, beta if ladder > 1 else -1)
-        return _pack(kind, names, [out], n_chains, post.shape[0])
+        rk = [dev.rank_diagnostics_device(post, specs, ladder, beta if ladder > 1 else -1)] if rank else None
+        return _pack(kind, names, [out], n_chains, post.shape[0], rk)
     if ladder > 1:
         post = cold_records_device(post, ladder, E.REC_BETA)
     post = post.contiguous()
     parts = [dev.chain_diagnostics_device(post, specs)]
+    rparts = [dev.rank_diagnostics_device(post, specs)] if rank else None
     if bins:
         import torch
         Sn, M = post.shape[0], post.shape[1]
         bnames, dnames, nnames = _bin_names(n_bins)
         step = max(1, min(n_bins, int(HPD_BYTES // (8 * max(Sn * M, 1)))))
         per = {"l": [], "m": [], "net": []}
+        rper = {"l": [], "m": [], "net": []}
         for lo in range(0, n_bins, step):
             cnt = min(step, n_bins - lo)
             mb, md = dev.marginal_rates_device(post, origin, n_bins, lo, cnt)
             mat = torch.cat([mb, md], dim=1).reshape(Sn, M, 2 * cnt)
             del mb, md
-            r = dev.chain_diagnostics_device(mat, list(range(2 * cnt)) + [(j, cnt + j, -1) for j in range(cnt)])
+            mspecs = list(range(2 * cnt)) + [(j, cnt + j, -1) for j in range(cnt)]
+            r = dev.chain_diagnostics_device(mat, mspecs)
+            rr = dev.rank_diagnostics_device(mat, mspecs) if rank else None
             for k, sl in (("l", slice(0, cnt)), ("m", slice(cnt, 2 * cnt)), ("net", slice(2 * cnt, 3 * cnt))):
                 per[k].append({f: v[sl] for f, v in r.items()})
+                if rank:
+                    rper[k].append({f: v[sl] for f, v in rr.items()})
             del mat
         parts += per["l"] + per["m"] + per["net"]
+        if rank:
+            rparts += rper["l"] + rper["m"] + rper["net"]
         names += bnames + dnames + nnames
-    return _pack(kind, names, parts, n_chains, post.shape[0])
+    return _pack(kind, names, parts, n_chains, post.shape[0], rparts)
 
 
 # ------------------------------------------------------------------------------------------ logs
@@ -332,15 +472,16 @@ def log_draws(paths, burnin=0.2, bins=True, note=print):
     return kind, blocks[0][0], np.stack([b[1][:k] for b in blocks], axis=1)
 
 
-def diagnose_logs(paths, burnin=0.2, device=None, bins=True, note=print):
+def diagnose_logs(paths, burnin=0.2, device=None, bins=True, note=print, rank=False):
     """K9 on the post-burn-in rows of sample logs of one kind, one log per chain (log_draws) -> Diagnostics.  device: an
-    engine.Device (None: device 0)."""
+    engine.Device (None: device 0).  rank: the rank-normalised diagnostics too (K10)."""
     import torch
     kind, names, x = log_draws(paths, burnin, bins, note)
     dev = device if device is not None else E.Device(0)
     t = torch.from_numpy(np.ascontiguousarray(x)).to(torch.device("cuda", dev.index))
     out = dev.chain_diagnostics_device(t, list(range(x.shape[2])))
-    return _pack(kind, names, [out], x.shape[1], x.shape[0])
+    rk = [dev.rank_diagnostics_device(t, list(range(x.shape[2])))] if rank else None
+    return _pack(kind, names, [out], x.shape[1], x.shape[0], rk)
 
 
 def find_logs(log_dir):

@@ -53,6 +53,7 @@ class BinStats:
         return self.sp.shape[0]
 
 
+RANK_FIELDS = ("median", "q05", "q95", "rhat_bulk", "rhat_tail", "rhat_rank", "ess_bulk", "ess_tail")   # lr_rank_diagnostics
 YEAR_PAD = np.iinfo(np.int32).min      # padding of ragged int32 year tables (both columns): contributes nothing
 
 
@@ -343,6 +344,52 @@ class Device:
         if ladder > 1 and int(status.item()):
             raise ValueError("a ladder has no chain at beta = 1 (%d samples)" % int(status.item()))
         return dict(zip(("mean", "sd", "rhat", "ess", "lag"), out))
+
+    def _rank_call(self, fn, records, cols, ladder, beta_col, outs, stream):
+        import torch
+        if not (records.is_cuda and records.dtype == torch.float64 and records.dim() == 3 and records.stride(2) == 1
+                and records.stride(0) == records.shape[1] * records.stride(1)):
+            raise ValueError("records must be a float64 CUDA tensor [n_samples, n_chains * ladder, w] with evenly spaced contiguous rows")
+        S, nk, w = records.shape
+        if S < 4:
+            raise RuntimeError("not enough data")
+        if ladder < 1 or nk % ladder:
+            raise ValueError("the chains of records must be whole ladders of %d" % ladder)
+        spec = [(c, -1, 1, 0.0) if np.ndim(c) == 0 else (tuple(c) + (0.0,))[:4] for c in cols]
+        if not spec:
+            raise ValueError("no columns")
+        a = np.ascontiguousarray([s[0] for s in spec], dtype=np.int32)
+        b = np.ascontiguousarray([s[1] for s in spec], dtype=np.int32)
+        sg = np.ascontiguousarray([s[2] for s in spec], dtype=np.int32)
+        add = np.ascontiguousarray([s[3] for s in spec], dtype=np.float64)
+        stride = records.stride(1) if S * nk > 1 else w
+        bufs = [torch.empty(sh(S, nk // ladder, len(spec)), dtype=torch.float64, device=records.device) for sh in outs]
+        status = torch.zeros(1, dtype=torch.int64, device=records.device)
+        N.check(getattr(self.lib, fn)(self.h, C.c_void_p(records.data_ptr()), int(S), int(nk // ladder), int(ladder), int(beta_col),
+                                      int(stride), len(spec), N.np_ptr(a), N.np_ptr(b), N.np_ptr(sg), N.np_ptr(add),
+                                      *[C.c_void_p(t.data_ptr()) for t in bufs], C.c_void_p(status.data_ptr()),
+                                      _stream_ptr(stream, records.device)), fn)
+        if ladder > 1 and int(status.item()):
+            raise ValueError("%s: a ladder has no chain at beta = 1 (%d samples)" % (fn, int(status.item())))
+        return bufs
+
+    def rank_transform_device(self, records, cols, ladder=1, beta_col=-1, stream=None):
+        """The rank-normal transform of columns over the chains of a run (K10, lr_rank_transform); records, cols, ladder and
+        beta_col as for chain_diagnostics_device.  Returns (Z, quant): Z float64 [2n, n_chains, 4 n_cols] (n = n_samples // 2;
+        row i, chain c: split draw i of chain c; slots z, z of |x - median|, x <= q05, x <= q95 of column j at j, n_cols + j,
+        2 n_cols + j, 3 n_cols + j) and quant float64 [3, n_cols]: median of the split draws, q05 and q95 of all draws, as numpy
+        computes them.  Raises as chain_diagnostics_device does (errors name lr_rank_transform)."""
+        z, q = self._rank_call("lr_rank_transform", records, cols, ladder, beta_col,
+                               [lambda S, M, k: (2 * (S // 2), M, 4 * k), lambda S, M, k: (3, k)], stream)
+        return z, q
+
+    def rank_diagnostics_device(self, records, cols, ladder=1, beta_col=-1, stream=None):
+        """Rank-normalised split R-hat and bulk and tail ESS of columns over the chains of a run (K10, lr_rank_diagnostics), without
+        copying the records; diagnostics.rank_rhat_ess is the definition.  Arguments as for chain_diagnostics_device.  Returns a
+        dict of float64 CUDA tensors [n_cols]: median, q05, q95, rhat_bulk, rhat_tail, rhat_rank, ess_bulk, ess_tail.  Raises as
+        chain_diagnostics_device does (errors name lr_rank_diagnostics).  Returns when the outputs are written."""
+        (out,) = self._rank_call("lr_rank_diagnostics", records, cols, ladder, beta_col, [lambda S, M, k: (8, k)], stream)
+        return dict(zip(RANK_FIELDS, out))
 
     def new_accumulators(self, n_rep, n_bins, device):
         import torch
