@@ -6,7 +6,7 @@
 // and [S - n, S); N = 2 M n of them per column.  Split position i < 2n of chain c is row i M + c of Z (i >= n: draw S - 2n + i).
 //
 // lr_rank_transform, per batch of columns:
-//   1. gather: every draw of the column (the middle draw of an odd S too) becomes an order-preserving key (k8_key; -0 as +0); the
+//   1. gather: every draw of the column (the middle draw of an odd S too) becomes an order-preserving key (lr_key; -0 as +0); the
 //      split draws go to a segment of N keys in Z-row order, the middle draws to a segment of M keys, and the value of each split
 //      draw to its z slot of Z.  The AND and OR of all keys of a column give the digits every key shares (their sort passes are
 //      skipped: integer columns such as K_l need two or three of eight); flags say whether a split draw is non-finite or NaN.
@@ -39,12 +39,11 @@ constexpr size_t K10_BUDGET = (size_t)1 << 30;   // K10's own scratch per batch 
 constexpr int K10_MAX_BATCH = 8192;
 
 struct K10Args {
-    const double* rows;
-    long long S, n, M, stride;
-    int T, beta_col;
-    const int* ca; const int* cb; const int* cs; const double* cc;     // column specs of this batch
-    int n_cols;                                                       // columns of this batch
-    long long N, Nmid;                                                // split draws, middle draws (M or 0) per column
+    lr_chain_rows src;
+    long long n;                    // split draws per chain and half
+    lr_col_specs cols;              // column specs of this batch
+    int n_cols;                     // columns of this batch
+    long long N, Nmid;              // split draws, middle draws (M or 0) per column
     double* Z; long long zs, zq;    // Z row stride, distance of the slots z, z_f, I_05, I_95; Z points at the batch's first column
     unsigned long long* kx[2];      // [n_cols][N] split keys, ping-pong
     unsigned long long* km[2];      // [n_cols][Nmid] middle keys
@@ -58,7 +57,7 @@ struct K10Args {
     unsigned long long* missing;    // (sample, ladder) pairs without a member at beta = 1
 };
 
-__device__ __forceinline__ unsigned long long k10_key(double v) { return k8_key(v == 0.0 ? 0.0 : v); }
+__device__ __forceinline__ unsigned long long k10_key(double v) { return lr_key(v == 0.0 ? 0.0 : v); }
 
 // the passes a segment needs: bit d set when some keys differ in digit d
 __device__ __forceinline__ unsigned k10_passes(unsigned long long a, unsigned long long o) {
@@ -79,9 +78,9 @@ __global__ void k10_init_kernel(const K10Args p) {
 
 // where row r = (s, chain) goes: its split position i M + chain, or -1 - chain for the middle draw of an odd S
 __device__ __forceinline__ long long k10_pos(const K10Args& p, long long r) {
-    const long long s = r / p.M, ch = r - s * p.M;
-    if (s < p.n) return s * p.M + ch;
-    if (s >= p.S - p.n) return (s - (p.S - 2 * p.n)) * p.M + ch;
+    const long long M = p.src.M, s = r / M, ch = r - s * M;
+    if (s < p.n) return s * M + ch;
+    if (s >= p.src.S - p.n) return (s - (p.src.S - 2 * p.n)) * M + ch;
     return -1 - ch;
 }
 
@@ -92,27 +91,22 @@ __global__ void __launch_bounds__(K10_TW * 32) k10_gather_kernel(const K10Args p
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int col = blockIdx.y * K10_G + lane;
     const bool has = col < p.n_cols;
-    int a = 0, b = -1, s = 1;
-    double c = 0.0;
-    if (has) { a = p.ca[col]; b = p.cb[col]; s = p.cs[col]; c = p.cc[col]; }
-    const long long R = p.S * p.M;
+    lr_col_spec spec;
+    if (has) spec = p.cols.load(col);
+    const long long R = p.src.S * p.src.M;
     unsigned long long kand = ~0ull, kor = 0ull, miss = 0;
     int fl = 0;
     for (long long r0 = ((long long)blockIdx.x * K10_TW + warp) * 32; r0 < R; r0 += (long long)gridDim.x * K10_TW * 32) {
         for (int j = 0; j < 32; ++j) {
             const long long r = r0 + j;
             if (r >= R) break;                                       // warp-uniform
-            const long long sm = r / p.M, ch = r - sm * p.M;
-            const double* row = p.rows + (sm * p.M * p.T + ch * p.T) * p.stride;
-            if (p.T > 1) {
-                const bool cold = lane < p.T && row[(long long)lane * p.stride + p.beta_col] == 1.0;
-                const unsigned bal = __ballot_sync(0xffffffffu, cold);
-                miss += bal == 0;
-                row += (long long)(bal ? __ffs(bal) - 1 : 0) * p.stride;
-            }
+            const long long sm = r / p.src.M;
+            bool m = false;
+            const double* row = lr_chain_row(p.src, sm, r - sm * p.src.M, lane, &m);
+            miss += m;
             unsigned long long k = 0;
             if (has) {
-                const double v = k8_value(row, a, b, s, c);
+                const double v = spec.value(row);
                 k = k10_key(v);
                 kand &= k; kor |= k;
                 const long long pos = k10_pos(p, r);
@@ -272,13 +266,13 @@ __device__ double k10_quantile(const unsigned long long* a, long long na, const 
     const double hv = __dmul_rn((double)(n - 1), p);
     double lo_v, hi_v, g;
     if (hv >= (double)(n - 1)) {                                     // numpy: both neighbours the last, gamma = h + 1
-        lo_v = hi_v = k8_val(k10_kth(a, na, b, nb, n - 1));
+        lo_v = hi_v = lr_val(k10_kth(a, na, b, nb, n - 1));
         g = __dadd_rn(hv, 1.0);
     } else {
         const double fl = floor(hv);
         const long long lo = (long long)fl;
-        lo_v = k8_val(k10_kth(a, na, b, nb, lo));
-        hi_v = k8_val(k10_kth(a, na, b, nb, lo + 1));
+        lo_v = lr_val(k10_kth(a, na, b, nb, lo));
+        hi_v = lr_val(k10_kth(a, na, b, nb, lo + 1));
         g = __dsub_rn(hv, fl);
     }
     const double diff = __dsub_rn(hi_v, lo_v);
@@ -294,7 +288,7 @@ __global__ void k10_quant_kernel(const K10Args p) {
     const unsigned long long* a = p.kx[k10_src(passes, 8)] + (size_t)c * p.N;
     const unsigned long long* b = p.km[k10_src(passes, 8)] + (size_t)c * p.Nmid;
     const int fl = p.flag[c];
-    const double med = (fl & 2) ? CUDART_NAN : __dadd_rn(k8_val(a[p.N / 2 - 1]), k8_val(a[p.N / 2])) / 2.0;
+    const double med = (fl & 2) ? CUDART_NAN : __dadd_rn(lr_val(a[p.N / 2 - 1]), lr_val(a[p.N / 2])) / 2.0;
     const double q05 = (fl & 4) ? CUDART_NAN : k10_quantile(a, p.N, b, p.Nmid, 0.05);
     const double q95 = (fl & 4) ? CUDART_NAN : k10_quantile(a, p.N, b, p.Nmid, 0.95);
     p.quant[c] = med; p.quant[p.qn + c] = q05; p.quant[2 * p.qn + c] = q95;
@@ -412,29 +406,34 @@ K10Plan k10_plan(long long S, long long M, bool with_z) {
     return pl;
 }
 
-// the bytes of one batch's buffers, laid out from `q` when it is not null
-size_t k10_layout(K10Args* p, K10Sort* sx, K10Sort* sm, K10Sort* sf, const K10Plan& pl, int bc, char* q) {
-    auto al = lr_align256;
-    const size_t key_b = al((size_t)bc * pl.N * 8), mid_b = al((size_t)bc * std::max<long long>(pl.Nmid, 1) * 8);
-    const size_t hist_b = al((size_t)bc * 256 * std::max(pl.tiles, 1) * 4), col_b = al((size_t)bc * 8);
-    const size_t bytes = 4 * key_b + 2 * mid_b + hist_b + 5 * col_b;
-    if (!q) return bytes;
-    p->kx[0] = (unsigned long long*)q; q += key_b;
-    p->kx[1] = (unsigned long long*)q; q += key_b;
-    p->kf[0] = (unsigned long long*)q; q += key_b;
-    p->kf[1] = (unsigned long long*)q; q += key_b;
-    p->km[0] = (unsigned long long*)q; q += mid_b;
-    p->km[1] = (unsigned long long*)q; q += mid_b;
-    unsigned* ghist = (unsigned*)q; q += hist_b;
-    p->band = (unsigned long long*)q; q += col_b;
-    p->bor = (unsigned long long*)q; q += col_b;
-    p->fand = (unsigned long long*)q; q += col_b;
-    p->f_or = (unsigned long long*)q; q += col_b;
-    p->flag = (int*)q;
+// lr_rank_diagnostics' buffers besides the transform's: K9's status, Z of a batch, K9's outputs on it, and K9's scratch
+struct K10Diag { int64_t* status; double* Z; double* r9; char* k9; };
+
+// The workspace of one call: the staged specs; with dg (lr_rank_diagnostics) K9's status, Z of a batch and K9's outputs on it;
+// the sort buffers of a batch of bc columns; with dg K9's scratch last.  Placed from `base` (null: only measured) for p's chains;
+// returns its bytes.
+size_t k10_layout(char* base, K10Args* p, K10Sort* sx, K10Sort* sm, K10Sort* sf, lr_col_specs* spec, K10Diag* dg, const K10Plan& pl,
+                  int n_cols, int bc) {
+    lr_carve w{base};
+    *spec = lr_col_specs::carve(w, n_cols);
+    if (dg) {
+        dg->status = w.take<int64_t>(1);
+        dg->Z = w.take<double>((size_t)pl.N * 4 * bc);
+        dg->r9 = w.take<double>((size_t)5 * 4 * bc);
+    }
+    const size_t keys = (size_t)bc * pl.N, mids = (size_t)bc * std::max<long long>(pl.Nmid, 1);
+    p->kx[0] = w.take<unsigned long long>(keys); p->kx[1] = w.take<unsigned long long>(keys);
+    p->kf[0] = w.take<unsigned long long>(keys); p->kf[1] = w.take<unsigned long long>(keys);
+    p->km[0] = w.take<unsigned long long>(mids); p->km[1] = w.take<unsigned long long>(mids);
+    unsigned* ghist = w.take<unsigned>((size_t)bc * 256 * std::max(pl.tiles, 1));
+    p->band = w.take<unsigned long long>(bc); p->bor = w.take<unsigned long long>(bc);
+    p->fand = w.take<unsigned long long>(bc); p->f_or = w.take<unsigned long long>(bc);
+    p->flag = w.take<int>(bc);
     *sx = {p->kx[0], p->kx[1], pl.N, pl.tiles, p->band, p->bor, ghist};
     *sm = {p->km[0], p->km[1], pl.Nmid, pl.mid_tiles, p->band, p->bor, ghist};
     *sf = {p->kf[0], p->kf[1], pl.N, pl.tiles, p->fand, p->f_or, ghist};
-    return bytes;
+    if (dg) dg->k9 = w.take<char>(lr_k9_scratch_bytes(p->src.M, 4 * bc));
+    return w.used;
 }
 
 // steps 1-5 on the batch of p (its specs, Z and quant set)
@@ -443,7 +442,7 @@ int k10_transform_batch(lr_handle_t h, K10Args& p, K10Sort& sx, K10Sort& sm, K10
     const int cb = 128, cg = (p.n_cols + cb - 1) / cb;
     const long long want = std::max<long long>(1, 8LL * h->sm_count / groups);
     k10_init_kernel<<<cg, cb, 0, st>>>(p);
-    const long long rtiles = (p.S * p.M + K10_TW * 32 - 1) / (K10_TW * 32);
+    const long long rtiles = (p.src.S * p.src.M + K10_TW * 32 - 1) / (K10_TW * 32);
     k10_gather_kernel<<<dim3((unsigned)std::min<long long>(rtiles, want), groups), K10_TW * 32, 0, st>>>(p);
     LR_CUDA(cudaGetLastError());
     int rc = k10_sort(h, sx, p.n_cols, st);
@@ -462,24 +461,11 @@ int k10_transform_batch(lr_handle_t h, K10Args& p, K10Sort& sx, K10Sort& sm, K10
     return LR_OK;
 }
 
-int k10_check(const char* who, lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
-              int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b, const int32_t* h_col_sign) {
-    LR_REQUIRE(h && h_col_a && d_rows, "%s: null pointer", who);
-    LR_REQUIRE(n_samples >= 4, "%s: not enough data (%lld samples per chain; at least 4)", who, (long long)n_samples);
-    LR_REQUIRE(n_chains >= 1 && ladder >= 1 && ladder <= 32 && n_cols >= 1 && row_stride >= 1,
-               "%s: bad sizes (n_chains >= 1, ladder 1..32, n_cols >= 1, row_stride >= 1)", who);
-    LR_REQUIRE(n_samples * n_chains * ladder < ((int64_t)1 << 31), "%s: %lld rows; at most 2^31 - 1", who,
-               (long long)(n_samples * n_chains * ladder));
-    LR_REQUIRE(ladder == 1 || (beta_col >= 0 && beta_col < row_stride), "%s: beta column %d outside the row of %lld doubles", who,
-               beta_col, (long long)row_stride);
-    return lr_check_col_specs(who, n_cols, row_stride, h_col_a, h_col_b, h_col_sign);
-}
-
 void k10_args(K10Args* p, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col, int64_t row_stride,
               const K10Plan& pl) {
     memset(p, 0, sizeof(*p));
-    p->rows = d_rows; p->S = n_samples; p->n = pl.n; p->M = n_chains; p->stride = row_stride; p->T = ladder; p->beta_col = beta_col;
-    p->N = pl.N; p->Nmid = pl.Nmid;
+    p->src = {d_rows, n_samples, n_chains, row_stride, ladder, beta_col};
+    p->n = pl.n; p->N = pl.N; p->Nmid = pl.Nmid;
 }
 
 }  // namespace
@@ -489,9 +475,9 @@ extern "C" int lr_rank_transform(lr_handle_t h, const double* d_rows, int64_t n_
                                  const int32_t* h_col_sign, const double* h_col_add, double* d_z, double* d_quant, int64_t* d_status,
                                  void* stream) {
     const char* who = "lr_rank_transform";
-    int rc = k10_check(who, h, d_rows, n_samples, n_chains, ladder, beta_col, row_stride, n_cols, h_col_a, h_col_b, h_col_sign);
+    int rc = lr_check_chain_rows(who, h, d_z && d_quant && d_status, d_rows, n_samples, n_chains, ladder, beta_col, row_stride, n_cols,
+                                 h_col_a, h_col_b, h_col_sign);
     if (rc != LR_OK) return rc;
-    LR_REQUIRE(d_z && d_quant && d_status, "%s: null pointer", who);
     LR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     const K10Plan pl = k10_plan(n_samples, n_chains, false);
@@ -499,20 +485,17 @@ extern "C" int lr_rank_transform(lr_handle_t h, const double* d_rows, int64_t n_
     K10Args p;
     k10_args(&p, d_rows, n_samples, n_chains, ladder, beta_col, row_stride, pl);
     K10Sort sx, sm, sf;
-    const size_t spec_bytes = lr_col_spec_bytes(n_cols);
-    const size_t bytes = spec_bytes + k10_layout(&p, &sx, &sm, &sf, pl, bc, nullptr);
-    rc = lr_ws_acquire(h, bytes, st);
-    if (rc != LR_OK) return rc;
-    char* w = (char*)h->ws;
     lr_col_specs spec;
-    rc = lr_stage_col_specs(who, w, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st, &spec);
+    rc = lr_ws_acquire(h, k10_layout(nullptr, &p, &sx, &sm, &sf, &spec, nullptr, pl, n_cols, bc), st);
     if (rc != LR_OK) return rc;
-    k10_layout(&p, &sx, &sm, &sf, pl, bc, w + spec_bytes);
+    k10_layout((char*)h->ws, &p, &sx, &sm, &sf, &spec, nullptr, pl, n_cols, bc);
+    rc = lr_stage_col_specs(who, spec, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st);
+    if (rc != LR_OK) return rc;
     LR_CUDA(cudaMemsetAsync(d_status, 0, sizeof(int64_t), st));
     p.zs = 4LL * n_cols; p.zq = n_cols; p.qn = n_cols;
     for (int c0 = 0; c0 < n_cols; c0 += bc) {
         p.n_cols = std::min(bc, n_cols - c0);
-        p.ca = spec.a + c0; p.cb = spec.b + c0; p.cs = spec.sign + c0; p.cc = spec.add + c0;
+        p.cols = spec.from(c0);
         p.Z = d_z + c0; p.quant = d_quant + c0;
         p.missing = c0 == 0 ? (unsigned long long*)d_status : nullptr;
         rc = k10_transform_batch(h, p, sx, sm, sf, st);
@@ -525,9 +508,9 @@ extern "C" int lr_rank_diagnostics(lr_handle_t h, const double* d_rows, int64_t 
                                    int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
                                    const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, void* stream) {
     const char* who = "lr_rank_diagnostics";
-    int rc = k10_check(who, h, d_rows, n_samples, n_chains, ladder, beta_col, row_stride, n_cols, h_col_a, h_col_b, h_col_sign);
+    int rc = lr_check_chain_rows(who, h, d_out && d_status, d_rows, n_samples, n_chains, ladder, beta_col, row_stride, n_cols, h_col_a,
+                                 h_col_b, h_col_sign);
     if (rc != LR_OK) return rc;
-    LR_REQUIRE(d_out && d_status, "%s: null pointer", who);
     LR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
     const K10Plan pl = k10_plan(n_samples, n_chains, true);
@@ -535,39 +518,28 @@ extern "C" int lr_rank_diagnostics(lr_handle_t h, const double* d_rows, int64_t 
     K10Args p;
     k10_args(&p, d_rows, n_samples, n_chains, ladder, beta_col, row_stride, pl);
     K10Sort sx, sm, sf;
-    // workspace: K10's specs and control block, Z of a batch, K9's outputs on it, the sort buffers, then K9's own scratch
-    auto al = lr_align256;
-    const size_t spec_bytes = lr_col_spec_bytes(n_cols);
-    const size_t z_b = al((size_t)pl.N * 4 * bc * 8), r9_b = al((size_t)5 * 4 * bc * 8);
-    const size_t k10_b = spec_bytes + 256 + z_b + r9_b + k10_layout(&p, &sx, &sm, &sf, pl, bc, nullptr);
-    const size_t bytes = k10_b + lr_k9_scratch_bytes(n_chains, 4 * bc);
-    rc = lr_ws_acquire(h, bytes, st);
-    if (rc != LR_OK) return rc;
-    char* w = (char*)h->ws;
+    K10Diag dg;
     lr_col_specs spec;
-    rc = lr_stage_col_specs(who, w, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st, &spec);
+    rc = lr_ws_acquire(h, k10_layout(nullptr, &p, &sx, &sm, &sf, &spec, &dg, pl, n_cols, bc), st);
     if (rc != LR_OK) return rc;
-    char* q = w + spec_bytes;
-    int64_t* k9_status = (int64_t*)q; q += 256;
-    double* Z = (double*)q; q += z_b;
-    double* r9 = (double*)q; q += r9_b;
-    k10_layout(&p, &sx, &sm, &sf, pl, bc, q);
-    char* k9_w = w + k10_b;
+    k10_layout((char*)h->ws, &p, &sx, &sm, &sf, &spec, &dg, pl, n_cols, bc);
+    rc = lr_stage_col_specs(who, spec, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st);
+    if (rc != LR_OK) return rc;
     std::vector<int32_t> zcols(4 * (size_t)bc);
     for (int j = 0; j < 4 * bc; ++j) zcols[j] = j;
     LR_CUDA(cudaMemsetAsync(d_status, 0, sizeof(int64_t), st));
     for (int c0 = 0; c0 < n_cols; c0 += bc) {
         p.n_cols = std::min(bc, n_cols - c0);
-        p.ca = spec.a + c0; p.cb = spec.b + c0; p.cs = spec.sign + c0; p.cc = spec.add + c0;
-        p.Z = Z; p.zs = 4LL * p.n_cols; p.zq = p.n_cols;
+        p.cols = spec.from(c0);
+        p.Z = dg.Z; p.zs = 4LL * p.n_cols; p.zq = p.n_cols;
         p.quant = d_out + c0; p.qn = n_cols;
         p.missing = c0 == 0 ? (unsigned long long*)d_status : nullptr;
         rc = k10_transform_batch(h, p, sx, sm, sf, st);
         if (rc != LR_OK) return rc;
-        rc = lr_k9_run(h, k9_w, who, Z, 2 * pl.n, n_chains, 1, -1, 4LL * p.n_cols, 4 * p.n_cols, zcols.data(), nullptr, nullptr, nullptr,
-                       r9, k9_status, st);
+        rc = lr_k9_run(h, dg.k9, who, dg.Z, 2 * pl.n, n_chains, 1, -1, 4LL * p.n_cols, 4 * p.n_cols, zcols.data(), nullptr, nullptr,
+                       nullptr, dg.r9, dg.status, st);
         if (rc != LR_OK) return rc;
-        k10_finish_kernel<<<(p.n_cols + 127) / 128, 128, 0, st>>>(p, r9, d_out + c0, n_cols);
+        k10_finish_kernel<<<(p.n_cols + 127) / 128, 128, 0, st>>>(p, dg.r9, d_out + c0, n_cols);
         LR_CUDA(cudaGetLastError());
         h->launches += 1;
     }

@@ -34,8 +34,8 @@ struct K8Args {
     const double* rows;
     long long n_rows, stride;
     int mask_col;
-    const int* ca; const int* cb; const int* cs; const double* cc;    // column specs of this batch
-    int n_cols;                                                        // columns of this batch
+    lr_col_specs cols;              // column specs of this batch
+    int n_cols;                     // columns of this batch
     long long rows_per_slice;
     int n_slices;
     double level;
@@ -51,9 +51,6 @@ struct K8Args {
     double* mean; double* lo; double* hi; long long* n_out;
 };
 
-// (k8_key / k8_val, the order-preserving keys, k8_value, the value of a column spec in a row, and K8Sum, the compensated sum,
-// live in lr_common.cuh: K9 and K10 use them too)
-
 // pass < 8: histogram of digit `pass` (most significant first) of the keys that share each threshold's prefix so far (pass 0 also
 // writes the partial sums); pass 8: gathers the keys below the lower / above the upper threshold.  grid (slice, group).
 __global__ void __launch_bounds__(K8_WARPS * 32) k8_pass_kernel(const K8Args p, int pass) {
@@ -66,19 +63,18 @@ __global__ void __launch_bounds__(K8_WARPS * 32) k8_pass_kernel(const K8Args p, 
     const bool has = col < p.n_cols;
     if (pass < 8)
         for (int i = threadIdx.x; i < 2 * K8_G * K8_HB; i += blockDim.x) hist[i] = 0;
-    int a = 0, b = -1, s = 1;
-    double c = 0.0;
+    lr_col_spec spec;
     unsigned long long pre0 = 0, pre1 = 0, mhi = 0;
     const int shift = pass < 8 ? 56 - 8 * pass : 0;
     if (has) {
-        a = p.ca[col]; b = p.cb[col]; s = p.cs[col]; c = p.cc[col];
+        spec = p.cols.load(col);
         if (pass > 0) { pre0 = p.sel[4 * col]; pre1 = p.sel[4 * col + 1]; }
     }
     if (pass > 0 && pass < 8) mhi = ~0ull << (shift + 8);
     __syncthreads();
     const long long r0 = (long long)blockIdx.x * p.rows_per_slice;
     const long long r1 = min(p.n_rows, r0 + p.rows_per_slice);
-    K8Sum sum;
+    lr_sum sum;
     if (has) {
         unsigned* h0 = hist + lane * K8_HB;
         unsigned* h1 = hist + (K8_G + lane) * K8_HB;
@@ -86,8 +82,8 @@ __global__ void __launch_bounds__(K8_WARPS * 32) k8_pass_kernel(const K8Args p, 
         for (long long r = r0 + warp; r < r1; r += K8_WARPS) {
             const double* row = p.rows + r * p.stride;
             if (p.mask_col >= 0 && row[p.mask_col] != 1.0) continue;
-            const double v = k8_value(row, a, b, s, c);
-            const unsigned long long k = k8_key(v);
+            const double v = spec.value(row);
+            const unsigned long long k = lr_key(v);
             if (pass < 8) {
                 if (pass == 0) sum.add(v);
                 const unsigned d = (unsigned)(k >> shift) & 255u;
@@ -103,7 +99,7 @@ __global__ void __launch_bounds__(K8_WARPS * 32) k8_pass_kernel(const K8Args p, 
     if (pass == 0) red[warp * K8_G + lane] = sum.value();
     __syncthreads();
     if (pass == 0 && warp == 0 && has) {                 // fixed order: rows of a warp in order, then the warps in order
-        K8Sum t;
+        lr_sum t;
         for (int w = 0; w < K8_WARPS; ++w) t.add(red[w * K8_G + lane]);
         p.part[(size_t)blockIdx.x * p.n_cols + col] = t.value();
     }
@@ -250,7 +246,7 @@ __global__ void __launch_bounds__(K8_WIN_THREADS) k8_window_kernel(const K8Args 
     double bw = CUDART_INF;
     long long bi = LLONG_MAX;
     for (long long i = tid; i < c.m; i += K8_WIN_THREADS) {
-        const double w = __dsub_rn(k8_val(U[i]), k8_val(L[i]));
+        const double w = __dsub_rn(lr_val(U[i]), lr_val(L[i]));
         if (k8_better(w, i, bw, bi)) { bw = w; bi = i; }
     }
     sw[tid] = bw; si[tid] = bi;
@@ -261,12 +257,28 @@ __global__ void __launch_bounds__(K8_WIN_THREADS) k8_window_kernel(const K8Args 
     }
     if (tid == 0) {
         const long long i = si[0];
-        p.lo[col] = k8_val(L[i]);
-        p.hi[col] = k8_val(U[i]);
-        K8Sum t;
+        p.lo[col] = lr_val(L[i]);
+        p.hi[col] = lr_val(U[i]);
+        lr_sum t;
         for (int q = 0; q < p.n_slices; ++q) t.add(p.part[(size_t)q * p.n_cols + col]);
         p.mean[col] = t.value() / (double)c.n;
     }
+}
+
+// the workspace of lr_column_hpd: the staged specs, the control block, then one batch's buffers, placed from `base` (null: only
+// measured) for p.n_slices and p.m_stride; returns its bytes
+size_t k8_layout(char* base, K8Args& p, lr_col_specs& spec, int n_cols, int batch_cols) {
+    lr_carve w{base};
+    spec = lr_col_specs::carve(w, n_cols);
+    p.ctrl = w.take<K8Ctrl>(1);
+    p.sel = w.take<unsigned long long>((size_t)batch_cols * 4);
+    p.ghist = w.take<unsigned>((size_t)batch_cols * 2 * 256);
+    p.part = w.take<double>((size_t)p.n_slices * batch_cols);
+    p.cnt = w.take<unsigned>((size_t)batch_cols * 2);
+    p.where = w.take<int>((size_t)batch_cols * 2);
+    p.tail0 = w.take<unsigned long long>((size_t)2 * batch_cols * p.m_stride);
+    p.tail1 = w.take<unsigned long long>((size_t)2 * batch_cols * p.m_stride);
+    return w.used;
 }
 
 }  // namespace
@@ -296,39 +308,20 @@ extern "C" int lr_column_hpd(lr_handle_t h, const double* d_rows, int64_t n_rows
     const size_t per_group = (size_t)K8_G * (4 * (size_t)m_stride * 8 + 32 + 2048 + 16 + (size_t)n_slices * 8);
     const int groups_per_batch = (int)std::max<size_t>(1, std::min<size_t>(std::min(n_groups, 1023), ((size_t)512 << 20) / per_group));
     const int batch_cols = std::min(n_cols, groups_per_batch * K8_G);
-    // workspace: column specs, control block, then one batch's buffers
-    auto al = lr_align256;
-    const size_t spec_bytes = lr_col_spec_bytes(n_cols);
-    const size_t sel_b = al((size_t)batch_cols * 32), hist_b = al((size_t)batch_cols * 2048), part_b = al((size_t)n_slices * batch_cols * 8);
-    const size_t cnt_b = al((size_t)batch_cols * 8), where_b = al((size_t)batch_cols * 8), tail_b = al((size_t)2 * batch_cols * m_stride * 8);
-    const size_t bytes = spec_bytes + 256 + sel_b + hist_b + part_b + cnt_b + where_b + 2 * tail_b;
-    int rc = lr_ws_acquire(h, bytes, st);
-    if (rc != LR_OK) return rc;
-    char* w = (char*)h->ws;
-    lr_col_specs spec;
-    rc = lr_stage_col_specs("lr_column_hpd", w, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st, &spec);
-    if (rc != LR_OK) return rc;
-    double* cc = spec.add;
-    int* ca = spec.a;
-    int* cb = spec.b;
-    int* cs = spec.sign;
     K8Args p;
     memset(&p, 0, sizeof(p));
     p.rows = d_rows; p.n_rows = n_rows; p.stride = row_stride; p.mask_col = mask_col;
     p.rows_per_slice = rows_per_slice; p.n_slices = n_slices; p.level = level; p.m_stride = m_stride;
-    char* q = w + spec_bytes;
-    p.ctrl = (K8Ctrl*)q; q += 256;
-    p.sel = (unsigned long long*)q; q += sel_b;
-    p.ghist = (unsigned*)q; q += hist_b;
-    p.part = (double*)q; q += part_b;
-    p.cnt = (unsigned*)q; q += cnt_b;
-    p.where = (int*)q; q += where_b;
-    p.tail0 = (unsigned long long*)q; q += tail_b;
-    p.tail1 = (unsigned long long*)q;
-    LR_CUDA(cudaMemsetAsync(p.ghist, 0, hist_b, st));
+    lr_col_specs spec;
+    int rc = lr_ws_acquire(h, k8_layout(nullptr, p, spec, n_cols, batch_cols), st);
+    if (rc != LR_OK) return rc;
+    k8_layout((char*)h->ws, p, spec, n_cols, batch_cols);
+    rc = lr_stage_col_specs("lr_column_hpd", spec, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st);
+    if (rc != LR_OK) return rc;
+    LR_CUDA(cudaMemsetAsync(p.ghist, 0, (size_t)batch_cols * 2 * 256 * 4, st));
     for (int c0 = 0; c0 < n_cols; c0 += batch_cols) {
         p.n_cols = std::min(batch_cols, n_cols - c0);
-        p.ca = ca + c0; p.cb = cb + c0; p.cs = cs + c0; p.cc = cc + c0;
+        p.cols = spec.from(c0);
         p.mean = d_mean + c0; p.lo = d_lo + c0; p.hi = d_hi + c0;
         p.n_out = c0 == 0 ? (long long*)d_n : nullptr;
         const dim3 grid(n_slices, (p.n_cols + K8_G - 1) / K8_G);

@@ -1,10 +1,8 @@
 // K9: split R-hat and effective sample size ("mean" ESS; Vehtari et al. 2021, section 3, as Stan and ArviZ compute them) of every
 // column of the sample records of a run, over its chains, on the device -- without copying the records.
 //
-// Rows.  Row (s, k) of d_rows is at d_rows + (s n_chains ladder + k) row_stride: [sample][chain][record] for the records of K3 / K6
-// / K7, or [n_samples n_chains][bins] for the matrices of lr_marginal_rates (ladder 1).  With ladder T > 1, logical chain c at
-// sample s is the first of the rows (s, cT) .. (s, cT + T - 1) whose field beta_col holds 1.0 (the cold member of its ladder).
-// A column is a spec of lr_common.cuh (row[a] +- row[b] + add).
+// Rows are lr_chain_rows of lr_common.cuh: the records of K3 / K6 / K7, or the matrices of lr_marginal_rates (ladder 1), read
+// through the cold member of each ladder.  A column is a spec of lr_common.cuh (row[a] +- row[b] + add).
 //
 // Estimator (literate_b200.diagnostics.rhat_ess is its host restatement, step for step).  n = floor(S / 2); split chain 2c is
 // draws [0, n) of chain c, split chain 2c + 1 draws [S - n, S) (the middle draw of an odd S is dropped); m = 2 M split chains.
@@ -42,7 +40,7 @@ constexpr int K9_MAX_BLOCK = 4096;  // widest lag block
 constexpr int K9_PART_LAGS = 8192;  // slices x block width: the partial sums of one column, at most
 
 struct K9Col {                      // per column of the batch
-    K8Sum acc;                      // sum of the monotone pair sums confirmed so far
+    lr_sum acc;                     // sum of the monotone pair sums confirmed so far
     double mean, W, varp;           // the mean of the draws, within variance, var+ (between-chain variance until block 0)
     double mono, ev, od;            // running minimum of the pair sums, the last pair (even, odd)
     long long t;                    // Geyer's t (odd)
@@ -50,12 +48,11 @@ struct K9Col {                      // per column of the batch
 };
 
 struct K9Args {
-    const double* rows;
-    long long S, n, M, stride;
-    int T, beta_col;
-    const int* ca; const int* cb; const int* cs; const double* cc;     // column specs of this batch
-    int n_cols;                                                       // columns of this batch
-    long long m;                                                      // split chains
+    lr_chain_rows src;
+    long long n;                    // draws per split chain
+    lr_col_specs cols;              // column specs of this batch
+    int n_cols;                     // columns of this batch
+    long long m;                    // split chains
     double* sum;                    // [m][n_cols] sum of each split chain
     double* mean;                   // [m][n_cols] mean of each split chain (exact for a constant one)
     int* flag;                      // [m][n_cols] bit 0: a non-finite draw, bit 1: not constant
@@ -68,16 +65,9 @@ struct K9Args {
     long long n_out;
 };
 
-// row of draw i of split chain j; with ladders the cold member is found by the warp (lanes 0..T-1 test one member each)
+// row of draw i of split chain j (lr_chain_row: a warp-wide call)
 __device__ __forceinline__ const double* k9_row(const K9Args& p, long long j, long long i, int lane, bool* missing) {
-    const long long c = j >> 1;
-    const long long s = (j & 1) ? p.S - p.n + i : i;
-    const double* base = p.rows + (s * p.M * p.T + c * p.T) * p.stride;
-    if (p.T == 1) return base;
-    const bool cold = lane < p.T && base[(long long)lane * p.stride + p.beta_col] == 1.0;
-    const unsigned b = __ballot_sync(0xffffffffu, cold);
-    if (missing) *missing = b == 0;
-    return base + (long long)(b ? __ffs(b) - 1 : 0) * p.stride;
+    return lr_chain_row(p.src, (j & 1) ? p.src.S - p.n + i : i, j >> 1, lane, missing);
 }
 
 // grid (block of K9_WARPS split chains, group): warp w takes split chain blockIdx.x K9_WARPS + w, lane c column c of the group
@@ -87,10 +77,9 @@ __global__ void __launch_bounds__(K9_WARPS * 32) k9_moments_kernel(const K9Args 
     if (j >= p.m) return;
     const int col = blockIdx.y * K9_G + lane;
     const bool has = col < p.n_cols;
-    int a = 0, b = -1, s = 1;
-    double c = 0.0;
-    if (has) { a = p.ca[col]; b = p.cb[col]; s = p.cs[col]; c = p.cc[col]; }
-    K8Sum sum;
+    lr_col_spec spec;
+    if (has) spec = p.cols.load(col);
+    lr_sum sum;
     double lo = CUDART_INF, hi = -CUDART_INF, first = 0.0;
     bool finite = true;
     unsigned long long miss = 0;
@@ -99,7 +88,7 @@ __global__ void __launch_bounds__(K9_WARPS * 32) k9_moments_kernel(const K9Args 
         const double* row = k9_row(p, j, i, lane, &m);
         miss += m;
         if (has) {
-            const double v = k8_value(row, a, b, s, c);
+            const double v = spec.value(row);
             if (i == 0) first = v;
             sum.add(v);
             finite &= isfinite(v);
@@ -129,7 +118,7 @@ __global__ void k9_init_kernel(const K9Args p) {
     if (col >= p.n_cols) return;
     K9Col st;
     memset(&st, 0, sizeof(st));
-    K8Sum tot, mm;
+    lr_sum tot, mm;
     int fl_or = 0, fl_and = 2;
     bool equal = true;
     const double m0 = p.mean[col];
@@ -149,7 +138,7 @@ __global__ void k9_init_kernel(const K9Args p) {
         const double xbar = mm.value() / (double)p.m;
         double between = 0.0;
         if (!equal) {
-            K8Sum d2;
+            lr_sum d2;
             for (long long j = 0; j < p.m; ++j) {
                 const double d = p.mean[(size_t)j * p.n_cols + col] - xbar;
                 d2.add(d * d);
@@ -176,10 +165,9 @@ __global__ void __launch_bounds__(K9_WARPS * 32) k9_lag_kernel(const K9Args p, l
     if (!__syncthreads_or(has && !p.done[col])) return;  // every column of the group finished
     const long long tc0 = t0 + (long long)blockIdx.y * CL;
     const long long j0 = (long long)blockIdx.z * per_slice, j1 = min(p.m, j0 + per_slice);
-    int a = 0, b = -1, s = 1;
-    double c = 0.0;
-    if (has) { a = p.ca[col]; b = p.cb[col]; s = p.cs[col]; c = p.cc[col]; }
-    K8Sum acc[LPT];
+    lr_col_spec spec;
+    if (has) spec = p.cols.load(col);
+    lr_sum acc[LPT];
     for (long long j = j0; j < j1; ++j) {
         const double mu = has ? p.mean[(size_t)j * p.n_cols + col] : 0.0;
         for (long long i0 = 0; i0 < p.n - tc0; i0 += K9_TI) {
@@ -188,7 +176,7 @@ __global__ void __launch_bounds__(K9_WARPS * 32) k9_lag_kernel(const K9Args p, l
                 double v = 0.0;
                 if (i < p.n) {                            // warp-uniform
                     const double* row = k9_row(p, j, i, lane, nullptr);
-                    if (has) v = __dsub_rn(k8_value(row, a, b, s, c), mu);
+                    if (has) v = __dsub_rn(spec.value(row), mu);
                 }
                 if (r < K9_TI) sa[r][lane] = v; else sb[r - K9_TI][lane] = v;
             }
@@ -225,7 +213,7 @@ __global__ void k9_step_kernel(const K9Args p, long long t0, long long t1, int w
     K9Col st = p.col[col];
     const double mn = (double)p.m * (double)p.n;
     auto lagsum = [&](long long t) {
-        K8Sum s;
+        lr_sum s;
         for (int z = 0; z < slices; ++z) s.add(p.part[((size_t)z * width + (size_t)(t - t0)) * p.n_cols + col]);
         return s.value();
     };
@@ -242,7 +230,7 @@ __global__ void k9_step_kernel(const K9Args p, long long t0, long long t1, int w
             return;
         }
         st.t = 1; st.ev = 1.0; st.od = rho(1); st.stored = 1; st.mono = CUDART_INF;
-        st.acc = K8Sum();
+        st.acc = lr_sum();
     }
     for (;;) {
         if (!(st.t < p.n - 3 && st.ev + st.od > 0.0)) {               // Geyer's sequence ends: max_t = t - 2
@@ -277,13 +265,27 @@ static int k9_batch_cols(long long m, int n_cols) {
     return (int)std::max<size_t>(1, std::min<size_t>((size_t)n_cols, ((size_t)256 << 20) / per_col));
 }
 
+// K9's scratch: the staged specs, the finished count, then one batch's buffers, placed from `base` (null: only measured) for p.m
+// split chains; returns its bytes
+static size_t k9_layout(char* base, K9Args& p, lr_col_specs& spec, int n_cols) {
+    const int batch_cols = k9_batch_cols(p.m, n_cols);
+    lr_carve w{base};
+    spec = lr_col_specs::carve(w, n_cols);
+    p.finished = w.take<unsigned>(1);
+    p.sum = w.take<double>((size_t)p.m * batch_cols);
+    p.mean = w.take<double>((size_t)p.m * batch_cols);
+    p.flag = w.take<int>((size_t)p.m * batch_cols);
+    p.part = w.take<double>((size_t)K9_PART_LAGS * batch_cols);
+    p.col = w.take<K9Col>(batch_cols);
+    p.done = w.take<int>(batch_cols);
+    return w.used;
+}
+
 size_t lr_k9_scratch_bytes(int64_t n_chains, int32_t n_cols) {
-    const long long m = 2 * n_chains;
-    const int batch_cols = k9_batch_cols(m, n_cols);
-    auto al = lr_align256;
-    const size_t sum_b = al((size_t)m * batch_cols * 8), flag_b = al((size_t)m * batch_cols * 4);
-    const size_t part_b = al((size_t)K9_PART_LAGS * batch_cols * 8), col_b = al(sizeof(K9Col) * batch_cols), done_b = al((size_t)batch_cols * 4);
-    return lr_col_spec_bytes(n_cols) + 256 + 2 * sum_b + flag_b + part_b + col_b + done_b;
+    K9Args p;
+    lr_col_specs spec;
+    p.m = 2 * n_chains;
+    return k9_layout(nullptr, p, spec, n_cols);
 }
 
 int lr_k9_run(lr_handle_t h, char* w, const char* who, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder,
@@ -291,31 +293,18 @@ int lr_k9_run(lr_handle_t h, char* w, const char* who, const double* d_rows, int
               const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, cudaStream_t st) {
     const long long n = n_samples / 2, m = 2 * n_chains;
     const int batch_cols = k9_batch_cols(m, n_cols);
-    auto al = lr_align256;
-    const size_t spec_bytes = lr_col_spec_bytes(n_cols);
-    const size_t sum_b = al((size_t)m * batch_cols * 8), flag_b = al((size_t)m * batch_cols * 4);
-    const size_t part_b = al((size_t)K9_PART_LAGS * batch_cols * 8), col_b = al(sizeof(K9Col) * batch_cols);
-    lr_col_specs spec;
-    int rc = lr_stage_col_specs(who, w, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st, &spec);
-    if (rc != LR_OK) return rc;
     K9Args p;
     memset(&p, 0, sizeof(p));
-    p.rows = d_rows; p.S = n_samples; p.n = n; p.M = n_chains; p.stride = row_stride; p.T = ladder; p.beta_col = beta_col; p.m = m;
-    p.n_out = n_cols;
-    char* q = w + spec_bytes;
-    p.finished = (unsigned*)q;
-    p.missing = (unsigned long long*)(q + 64);
-    q += 256;
-    p.sum = (double*)q; q += sum_b;
-    p.mean = (double*)q; q += sum_b;
-    p.flag = (int*)q; q += flag_b;
-    p.part = (double*)q; q += part_b;
-    p.col = (K9Col*)q; q += col_b;
-    p.done = (int*)q;
+    p.src = {d_rows, n_samples, n_chains, row_stride, ladder, beta_col};
+    p.n = n; p.m = m; p.n_out = n_cols;
+    lr_col_specs spec;
+    k9_layout(w, p, spec, n_cols);
+    int rc = lr_stage_col_specs(who, spec, n_cols, h_col_a, h_col_b, h_col_sign, h_col_add, st);
+    if (rc != LR_OK) return rc;
     LR_CUDA(cudaMemsetAsync(d_status, 0, sizeof(int64_t), st));
     for (int c0 = 0; c0 < n_cols; c0 += batch_cols) {
         p.n_cols = std::min(batch_cols, n_cols - c0);
-        p.ca = spec.a + c0; p.cb = spec.b + c0; p.cs = spec.sign + c0; p.cc = spec.add + c0;
+        p.cols = spec.from(c0);
         p.out = d_out + c0;
         p.missing = c0 == 0 ? (unsigned long long*)d_status : nullptr;
         const int groups = (p.n_cols + K9_G - 1) / K9_G;
@@ -356,18 +345,12 @@ int lr_k9_run(lr_handle_t h, char* w, const char* who, const double* d_rows, int
 extern "C" int lr_chain_diagnostics(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
                                     int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
                                     const int32_t* h_col_sign, const double* h_col_add, double* d_out, int64_t* d_status, void* stream) {
-    LR_REQUIRE(h && d_out && d_status && h_col_a && d_rows, "lr_chain_diagnostics: null pointer");
-    LR_REQUIRE(n_samples >= 4, "lr_chain_diagnostics: not enough data (%lld samples per chain; at least 4)", (long long)n_samples);
-    LR_REQUIRE(n_chains >= 1 && ladder >= 1 && ladder <= 32 && n_cols >= 1 && row_stride >= 1,
-               "lr_chain_diagnostics: bad sizes (n_chains >= 1, ladder 1..32, n_cols >= 1, row_stride >= 1)");
-    LR_REQUIRE(n_samples * n_chains * ladder < ((int64_t)1 << 31), "lr_chain_diagnostics: %lld rows; at most 2^31 - 1",
-               (long long)(n_samples * n_chains * ladder));
-    LR_REQUIRE(ladder == 1 || (beta_col >= 0 && beta_col < row_stride),
-               "lr_chain_diagnostics: beta column %d outside the row of %lld doubles", beta_col, (long long)row_stride);
-    { int rc0 = lr_check_col_specs("lr_chain_diagnostics", n_cols, row_stride, h_col_a, h_col_b, h_col_sign); if (rc0 != LR_OK) return rc0; }
+    int rc = lr_check_chain_rows("lr_chain_diagnostics", h, d_out && d_status, d_rows, n_samples, n_chains, ladder, beta_col, row_stride,
+                                 n_cols, h_col_a, h_col_b, h_col_sign);
+    if (rc != LR_OK) return rc;
     LR_CUDA(cudaSetDevice(h->device));
     cudaStream_t st = stream ? (cudaStream_t)stream : h->stream;
-    int rc = lr_ws_acquire(h, lr_k9_scratch_bytes(n_chains, n_cols), st);
+    rc = lr_ws_acquire(h, lr_k9_scratch_bytes(n_chains, n_cols), st);
     if (rc != LR_OK) return rc;
     return lr_k9_run(h, (char*)h->ws, "lr_chain_diagnostics", d_rows, n_samples, n_chains, ladder, beta_col, row_stride, n_cols,
                      h_col_a, h_col_b, h_col_sign, h_col_add, d_out, d_status, st);

@@ -237,29 +237,35 @@ inline int lr_upload_bin_stats(lr_handle_t h, size_t cnt, const int64_t* h_sp, c
     return LR_OK;
 }
 
-// ---- column specs of the record consumers (K8 lr_column_hpd, K9 lr_chain_diagnostics, K10 lr_rank_*) -----------------------------
-// Output column j of a row is row[a_j], then + or - row[b_j] (b_j >= 0, sign_j = +-1), then + add_j (if non-zero): one fp64 operation
-// each, in this order -- what the logs hold (the net rate l_j - m_j, DDRate's midpoint_x0 and maxCarryingCap).
-__device__ __forceinline__ double k8_value(const double* row, int a, int b, int s, double c) {
-    double v = row[a];
-    if (b >= 0) v = s > 0 ? __dadd_rn(v, row[b]) : __dsub_rn(v, row[b]);
-    if (c != 0.0) v = __dadd_rn(v, c);
-    return v;
-}
+// ---- workspace layout ----------------------------------------------------------------------------------------------------------
+inline size_t lr_align256(size_t x) { return (x + 255) & ~(size_t)255; }
+// Buffers placed one after the other from `base`, each 256-byte aligned.  A null base only measures: every buffer is null and
+// `used` ends as the bytes the same calls need from a real base, so one layout function both sizes a workspace and places it.
+struct lr_carve {
+    char* base;
+    size_t used = 0;
+    template <class T> T* take(size_t n) {
+        T* p = base ? (T*)(base + used) : nullptr;
+        used += lr_align256(n * sizeof(T));
+        return p;
+    }
+};
+
+// ---- record consumers (K8 lr_column_hpd, K9 lr_chain_diagnostics, K10 lr_rank_*) --------------------------------------------------
 // order-preserving key of a double: negative values bit-inverted, the sign bit set on the others; every NaN -> the largest key
-__device__ __forceinline__ unsigned long long k8_key(double x) {
+__device__ __forceinline__ unsigned long long lr_key(double x) {
     const unsigned long long b = (unsigned long long)__double_as_longlong(x);
     if (x != x) return ~0ull;
     return (b & 0x8000000000000000ull) ? ~b : (b | 0x8000000000000000ull);
 }
-__device__ __forceinline__ double k8_val(unsigned long long k) {
+__device__ __forceinline__ double lr_val(unsigned long long k) {
     return __longlong_as_double((long long)((k & 0x8000000000000000ull) ? (k ^ 0x8000000000000000ull) : ~k));
 }
 // Compensated (Neumaier) sum: the running sum s and the rounding errors c of its additions, so that a mean over millions of rows
 // stays within a few units in the last place of the correctly rounded one (a plain sum in any order drifts by up to n ulp when the
 // rounding errors share a sign, e.g. a column of the values 0.1, 0.2, 0.3).  A sum that became +-inf or NaN stays so and is
 // returned as it is, as a plain sum would.
-struct K8Sum {
+struct lr_sum {
     double s = 0.0, c = 0.0;
     __device__ __forceinline__ void add(double v) {
         const double t = __dadd_rn(s, v);
@@ -269,10 +275,31 @@ struct K8Sum {
     __device__ __forceinline__ double value() const { return isfinite(s) ? __dadd_rn(s, c) : s; }
 };
 
-inline size_t lr_align256(size_t x) { return (x + 255) & ~(size_t)255; }
-// bytes of the staged specs at the start of the workspace: add [n] fp64, then a, b, sign [n] int32, each 256-byte aligned
-inline size_t lr_col_spec_bytes(int n_cols) { return lr_align256((size_t)n_cols * 8) + 3 * lr_align256((size_t)n_cols * 4); }
-struct lr_col_specs { double* add; int* a; int* b; int* sign; };
+// Column specs.  Output column j of a row is row[a_j], then + or - row[b_j] (b_j >= 0, sign_j = +-1), then + add_j (if non-zero):
+// one fp64 operation each, in this order -- what the logs hold (the net rate l_j - m_j, DDRate's midpoint_x0 and maxCarryingCap).
+// (a default spec reads field 0: what a lane without a column of its group holds, whose values it never uses)
+struct lr_col_spec {
+    int a = 0, b = -1, s = 1;
+    double c = 0.0;
+    __device__ __forceinline__ double value(const double* row) const {
+        double v = row[a];
+        if (b >= 0) v = s > 0 ? __dadd_rn(v, row[b]) : __dsub_rn(v, row[b]);
+        if (c != 0.0) v = __dadd_rn(v, c);
+        return v;
+    }
+};
+// the specs staged on the device: add [n] fp64, then a, b, sign [n] int32, one block in the workspace
+struct lr_col_specs {
+    int* a; int* b; int* sign; double* add;
+    static lr_col_specs carve(lr_carve& w, int n_cols) {
+        lr_col_specs s;
+        s.add = w.take<double>(n_cols); s.a = w.take<int>(n_cols); s.b = w.take<int>(n_cols); s.sign = w.take<int>(n_cols);
+        return s;
+    }
+    // the specs of a batch of columns from column c0
+    lr_col_specs from(int c0) const { return {a + c0, b + c0, sign + c0, add + c0}; }
+    __device__ __forceinline__ lr_col_spec load(int col) const { return {a[col], b[col], sign[col], add[col]}; }
+};
 
 // every field inside the row and every sign +-1 (b, sign and add may be NULL: -1, 1, 0)
 inline int lr_check_col_specs(const char* who, int n_cols, int64_t row_stride, const int32_t* h_col_a, const int32_t* h_col_b,
@@ -286,35 +313,66 @@ inline int lr_check_col_specs(const char* who, int n_cols, int64_t row_stride, c
     return LR_OK;
 }
 
-// the specs, staged in one host block (defaults for the optional arrays) and copied to `w` (device) in one piece on `st`; the
-// copy is from pageable memory, so it has been staged when this returns
-inline int lr_stage_col_specs(const char* who, void* w, int n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
-                              const int32_t* h_col_sign, const double* h_col_add, cudaStream_t st, lr_col_specs* out) {
-    const size_t bytes = lr_col_spec_bytes(n_cols);
-    char* base = (char*)w;
-    out->add = (double*)base;
-    out->a = (int*)(base + lr_align256((size_t)n_cols * 8));
-    out->b = (int*)((char*)out->a + lr_align256((size_t)n_cols * 4));
-    out->sign = (int*)((char*)out->b + lr_align256((size_t)n_cols * 4));
+// the specs, staged in one host block (defaults for the optional arrays) and copied to the block `spec` (device, carved by
+// lr_col_specs::carve) in one piece on `st`; the copy is from pageable memory, so it has been staged when this returns
+inline int lr_stage_col_specs(const char* who, const lr_col_specs& spec, int n_cols, const int32_t* h_col_a, const int32_t* h_col_b,
+                              const int32_t* h_col_sign, const double* h_col_add, cudaStream_t st) {
+    char* base = (char*)spec.add;
+    const size_t bytes = (char*)(spec.sign + n_cols) - base;
     char* stage = (char*)calloc(1, bytes);
     LR_REQUIRE(stage, "%s: out of host memory", who);
     double* hc = (double*)stage;
-    int* ha = (int*)(stage + ((char*)out->a - base));
-    int* hb = (int*)(stage + ((char*)out->b - base));
-    int* hs = (int*)(stage + ((char*)out->sign - base));
+    int* ha = (int*)(stage + ((char*)spec.a - base));
+    int* hb = (int*)(stage + ((char*)spec.b - base));
+    int* hs = (int*)(stage + ((char*)spec.sign - base));
     for (int j = 0; j < n_cols; ++j) {
         ha[j] = h_col_a[j]; hb[j] = h_col_b ? h_col_b[j] : -1; hs[j] = h_col_sign ? h_col_sign[j] : 1;
         hc[j] = h_col_add ? h_col_add[j] : 0.0;
     }
-    const cudaError_t e = cudaMemcpyAsync(w, stage, bytes, cudaMemcpyHostToDevice, st);
+    const cudaError_t e = cudaMemcpyAsync(base, stage, bytes, cudaMemcpyHostToDevice, st);
     free(stage);
     LR_CUDA(e);
     return LR_OK;
 }
 
+// Rows of the chains of a run (K9, K10): row (s, k) is at rows + (s M T + k) stride -- [sample][chain][record], or a matrix
+// [S M][bins] (T = 1).  With ladders (T > 1) logical chain c at sample s is the first of the rows (s, cT) .. (s, cT + T - 1) whose
+// field beta_col holds 1.0 (the cold member of its ladder).
+struct lr_chain_rows {
+    const double* rows;
+    long long S, M, stride;
+    int T, beta_col;
+};
+// row of logical chain c at sample s; with ladders the cold member is found by the warp (lanes 0..T-1 test one member each) and
+// *missing (if not null) says whether the ladder has none at this sample
+__device__ __forceinline__ const double* lr_chain_row(const lr_chain_rows& r, long long s, long long c, int lane, bool* missing) {
+    const double* base = r.rows + (s * r.M * r.T + c * r.T) * r.stride;
+    if (r.T == 1) return base;
+    const bool cold = lane < r.T && base[(long long)lane * r.stride + r.beta_col] == 1.0;
+    const unsigned b = __ballot_sync(0xffffffffu, cold);
+    if (missing) *missing = b == 0;
+    return base + (long long)(b ? __ffs(b) - 1 : 0) * r.stride;
+}
+
+// the arguments of the entry points that read chain rows (lr_chain_diagnostics, lr_rank_transform, lr_rank_diagnostics); outs:
+// every output pointer of the entry point is set
+inline int lr_check_chain_rows(const char* who, lr_handle_t h, bool outs, const double* d_rows, int64_t n_samples, int64_t n_chains,
+                               int32_t ladder, int32_t beta_col, int64_t row_stride, int32_t n_cols, const int32_t* h_col_a,
+                               const int32_t* h_col_b, const int32_t* h_col_sign) {
+    LR_REQUIRE(h && outs && h_col_a && d_rows, "%s: null pointer", who);
+    LR_REQUIRE(n_samples >= 4, "%s: not enough data (%lld samples per chain; at least 4)", who, (long long)n_samples);
+    LR_REQUIRE(n_chains >= 1 && ladder >= 1 && ladder <= 32 && n_cols >= 1 && row_stride >= 1,
+               "%s: bad sizes (n_chains >= 1, ladder 1..32, n_cols >= 1, row_stride >= 1)", who);
+    LR_REQUIRE(n_samples * n_chains * ladder < ((int64_t)1 << 31), "%s: %lld rows; at most 2^31 - 1", who,
+               (long long)(n_samples * n_chains * ladder));
+    LR_REQUIRE(ladder == 1 || (beta_col >= 0 && beta_col < row_stride), "%s: beta column %d outside the row of %lld doubles", who,
+               beta_col, (long long)row_stride);
+    return lr_check_col_specs(who, n_cols, row_stride, h_col_a, h_col_b, h_col_sign);
+}
+
 // ---- K9's host driver on a caller's scratch (k9_diag.cu): lr_chain_diagnostics runs it on the workspace, K10 on the part of the
-// workspace behind its own buffers.  lr_k9_scratch_bytes is what lr_k9_run uses from `w` (at most ~256 MB beyond the staged
-// specs); the arguments are those of lr_chain_diagnostics, already checked, `who` names the entry point in errors.
+// workspace behind its own buffers.  lr_k9_scratch_bytes is what lr_k9_run uses from `w` (the staged specs and at most ~256 MB);
+// the arguments are those of lr_chain_diagnostics, already checked, `who` names the entry point in errors.
 size_t lr_k9_scratch_bytes(int64_t n_chains, int32_t n_cols);
 int lr_k9_run(lr_handle_t h, char* w, const char* who, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder,
               int32_t beta_col, int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,

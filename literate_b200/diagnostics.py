@@ -32,7 +32,6 @@ FORWARD_COLS = [("posterior", (E.REC_LIK, E.REC_PRIOR, 1, 0.0)), ("likelihood", 
                 ("lambda_avg", E.REC_LAVG), ("mu_avg", E.REC_MAVG), ("K_l", E.REC_KL), ("K_m", E.REC_KM),
                 ("gamma_rate_hp_BI", E.REC_GL), ("gamma_rate_hp_D", E.REC_GM), ("poisson_rate_hp", E.REC_POI)]
 FLAGS = ("ok", "rhat", "ess", "rhat+ess", "const", "stuck", "nonfinite")
-HPD_BYTES = 1 << 30                   # per K5 matrix chunk, as summary.summarize_records_device
 
 
 # ------------------------------------------------------------------------------------------ the estimator
@@ -381,12 +380,9 @@ def diagnose_records_device(dev, records, kind, n_bins, burnin=0.2, ladder=1, or
         import torch
         Sn, M = post.shape[0], post.shape[1]
         bnames, dnames, nnames = _bin_names(n_bins)
-        step = max(1, min(n_bins, int(HPD_BYTES // (8 * max(Sn * M, 1)))))
         per = {"l": [], "m": [], "net": []}
         rper = {"l": [], "m": [], "net": []}
-        for lo in range(0, n_bins, step):
-            cnt = min(step, n_bins - lo)
-            mb, md = dev.marginal_rates_device(post, origin, n_bins, lo, cnt)
+        for _, cnt, mb, md in S.marginal_chunks(dev, post, origin, n_bins):
             mat = torch.cat([mb, md], dim=1).reshape(Sn, M, 2 * cnt)
             del mb, md
             mspecs = list(range(2 * cnt)) + [(j, cnt + j, -1) for j in range(cnt)]
@@ -436,20 +432,9 @@ def _forward_log(path, burnin, bins):
 
 
 def _sibling_log(path, kind, burnin):
-    head = open(path).readline().rstrip("\r\n").split("\t")
-    tbl = np.loadtxt(path, delimiter="\t", skiprows=1, ndmin=2)
-    tbl = tbl[S.burnin_index(tbl.shape[0], burnin):]
-    idx = {h: i for i, h in enumerate(head)}
-    n_bins = sum(1 for h in head if h.startswith("l_") and h[2:].isdigit())
-    names = [c[0] for c in diagnostic_columns(kind, n_bins, 0.0, "genre_lik" in idx)]
-    cols = []
-    for nm in names:
-        if nm.startswith("net_"):
-            j = nm[4:]
-            cols.append(tbl[:, idx["l_" + j]] - tbl[:, idx["m_" + j]])
-        else:
-            cols.append(tbl[:, idx[nm]])
-    return names, np.stack(cols, axis=1), None
+    head, n_bins, col = PD.read_log(path, burnin)
+    names = [c[0] for c in diagnostic_columns(kind, n_bins, 0.0, "genre_lik" in head)]
+    return names, np.stack([col(nm) for nm in names], axis=1), None
 
 
 def log_draws(paths, burnin=0.2, bins=True, note=print):

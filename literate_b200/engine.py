@@ -73,6 +73,28 @@ def window(ts, te):
     return first, int(np.max(te)) - first
 
 
+def _col_specs(cols):
+    """The a, b, sign, add arrays (int32, int32, int32, float64) of column specs: an index a or a tuple (a, b, sign[, add])."""
+    spec = [(c, -1, 1, 0.0) if np.ndim(c) == 0 else (tuple(c) + (0.0,))[:4] for c in cols]
+    if not spec:
+        raise ValueError("no columns")
+    return [np.ascontiguousarray([s[i] for s in spec], dtype=t) for i, t in enumerate((np.int32, np.int32, np.int32, np.float64))]
+
+
+def _chain_records(records, ladder):
+    """(S, n_chains, row stride) of records [n_samples, n_chains * ladder, w] as K9 and K10 read them."""
+    import torch
+    if not (records.is_cuda and records.dtype == torch.float64 and records.dim() == 3 and records.stride(2) == 1
+            and records.stride(0) == records.shape[1] * records.stride(1)):
+        raise ValueError("records must be a float64 CUDA tensor [n_samples, n_chains * ladder, w] with evenly spaced contiguous rows")
+    S, nk, w = records.shape
+    if S < 4:
+        raise RuntimeError("not enough data")
+    if ladder < 1 or nk % ladder:
+        raise ValueError("the chains of records must be whole ladders of %d" % ladder)
+    return S, nk // ladder, records.stride(1) if S * nk > 1 else w
+
+
 class Device:
     """One lr_handle_t: a B200 and its streams/workspace."""
 
@@ -288,21 +310,15 @@ class Device:
         import torch
         if not (rows.is_cuda and rows.dtype == torch.float64 and rows.dim() == 2 and rows.stride(1) == 1):
             raise ValueError("rows must be a float64 CUDA tensor [n_rows, row_stride] with contiguous rows")
-        spec = [(c, -1, 1, 0.0) if np.ndim(c) == 0 else (tuple(c) + (0.0,))[:4] for c in cols]
-        if not spec:
-            raise ValueError("no columns")
-        a = np.ascontiguousarray([s[0] for s in spec], dtype=np.int32)
-        b = np.ascontiguousarray([s[1] for s in spec], dtype=np.int32)
-        sg = np.ascontiguousarray([s[2] for s in spec], dtype=np.int32)
-        add = np.ascontiguousarray([s[3] for s in spec], dtype=np.float64)
+        specs = _col_specs(cols)
         n_rows = rows.shape[0]
         stride = rows.stride(0) if n_rows > 1 else rows.shape[1]
         if mask_col < 0 and int(round(level * n_rows)) < 2:
             raise RuntimeError("not enough data")
-        out = torch.empty((3, len(spec)), dtype=torch.float64, device=rows.device)
+        out = torch.empty((3, len(specs[0])), dtype=torch.float64, device=rows.device)
         n = torch.empty(1, dtype=torch.int64, device=rows.device)
-        N.check(self.lib.lr_column_hpd(self.h, C.c_void_p(rows.data_ptr()), int(n_rows), int(stride), int(mask_col), len(spec),
-                                       N.np_ptr(a), N.np_ptr(b), N.np_ptr(sg), N.np_ptr(add), float(level),
+        N.check(self.lib.lr_column_hpd(self.h, C.c_void_p(rows.data_ptr()), int(n_rows), int(stride), int(mask_col), len(specs[0]),
+                                       *[N.np_ptr(x) for x in specs], float(level),
                                        C.c_void_p(out[0].data_ptr()), C.c_void_p(out[1].data_ptr()), C.c_void_p(out[2].data_ptr()),
                                        C.c_void_p(n.data_ptr()), _stream_ptr(stream, rows.device)), "lr_column_hpd")
         if mask_col >= 0 and int(round(level * int(n.item()))) < 2:
@@ -318,57 +334,20 @@ class Device:
         consecutive members and the member whose field beta_col holds 1.0 at a sample is the chain's draw.  Returns a dict of
         float64 CUDA tensors [n_cols]: mean, sd, rhat, ess, lag.  Raises RuntimeError("not enough data") for fewer than 4 samples
         and ValueError when a ladder has no member at beta = 1 at some sample.  Returns when the outputs are written."""
-        import torch
-        if not (records.is_cuda and records.dtype == torch.float64 and records.dim() == 3 and records.stride(2) == 1
-                and records.stride(0) == records.shape[1] * records.stride(1)):
-            raise ValueError("records must be a float64 CUDA tensor [n_samples, n_chains * ladder, w] with evenly spaced contiguous rows")
-        S, nk, w = records.shape
-        if S < 4:
-            raise RuntimeError("not enough data")
-        if ladder < 1 or nk % ladder:
-            raise ValueError("the chains of records must be whole ladders of %d" % ladder)
-        spec = [(c, -1, 1, 0.0) if np.ndim(c) == 0 else (tuple(c) + (0.0,))[:4] for c in cols]
-        if not spec:
-            raise ValueError("no columns")
-        a = np.ascontiguousarray([s[0] for s in spec], dtype=np.int32)
-        b = np.ascontiguousarray([s[1] for s in spec], dtype=np.int32)
-        sg = np.ascontiguousarray([s[2] for s in spec], dtype=np.int32)
-        add = np.ascontiguousarray([s[3] for s in spec], dtype=np.float64)
-        stride = records.stride(1) if S * nk > 1 else w
-        out = torch.empty((5, len(spec)), dtype=torch.float64, device=records.device)
-        status = torch.zeros(1, dtype=torch.int64, device=records.device)
-        N.check(self.lib.lr_chain_diagnostics(self.h, C.c_void_p(records.data_ptr()), int(S), int(nk // ladder), int(ladder), int(beta_col),
-                                              int(stride), len(spec), N.np_ptr(a), N.np_ptr(b), N.np_ptr(sg), N.np_ptr(add),
-                                              C.c_void_p(out.data_ptr()), C.c_void_p(status.data_ptr()), _stream_ptr(stream, records.device)),
-                "lr_chain_diagnostics")
-        if ladder > 1 and int(status.item()):
-            raise ValueError("a ladder has no chain at beta = 1 (%d samples)" % int(status.item()))
+        (out,) = self._chain_call("lr_chain_diagnostics", records, cols, ladder, beta_col, [lambda S, M, k: (5, k)], stream)
         return dict(zip(("mean", "sd", "rhat", "ess", "lag"), out))
 
-    def _rank_call(self, fn, records, cols, ladder, beta_col, outs, stream):
+    def _chain_call(self, fn, records, cols, ladder, beta_col, outs, stream):
+        """One call of an entry point that reads the chains of records (K9, K10) into new float64 buffers of the shapes
+        outs(S, n_chains, n_cols); raises when a ladder has no member at beta = 1."""
         import torch
-        if not (records.is_cuda and records.dtype == torch.float64 and records.dim() == 3 and records.stride(2) == 1
-                and records.stride(0) == records.shape[1] * records.stride(1)):
-            raise ValueError("records must be a float64 CUDA tensor [n_samples, n_chains * ladder, w] with evenly spaced contiguous rows")
-        S, nk, w = records.shape
-        if S < 4:
-            raise RuntimeError("not enough data")
-        if ladder < 1 or nk % ladder:
-            raise ValueError("the chains of records must be whole ladders of %d" % ladder)
-        spec = [(c, -1, 1, 0.0) if np.ndim(c) == 0 else (tuple(c) + (0.0,))[:4] for c in cols]
-        if not spec:
-            raise ValueError("no columns")
-        a = np.ascontiguousarray([s[0] for s in spec], dtype=np.int32)
-        b = np.ascontiguousarray([s[1] for s in spec], dtype=np.int32)
-        sg = np.ascontiguousarray([s[2] for s in spec], dtype=np.int32)
-        add = np.ascontiguousarray([s[3] for s in spec], dtype=np.float64)
-        stride = records.stride(1) if S * nk > 1 else w
-        bufs = [torch.empty(sh(S, nk // ladder, len(spec)), dtype=torch.float64, device=records.device) for sh in outs]
+        S, M, stride = _chain_records(records, ladder)
+        specs = _col_specs(cols)
+        bufs = [torch.empty(sh(S, M, len(specs[0])), dtype=torch.float64, device=records.device) for sh in outs]
         status = torch.zeros(1, dtype=torch.int64, device=records.device)
-        N.check(getattr(self.lib, fn)(self.h, C.c_void_p(records.data_ptr()), int(S), int(nk // ladder), int(ladder), int(beta_col),
-                                      int(stride), len(spec), N.np_ptr(a), N.np_ptr(b), N.np_ptr(sg), N.np_ptr(add),
-                                      *[C.c_void_p(t.data_ptr()) for t in bufs], C.c_void_p(status.data_ptr()),
-                                      _stream_ptr(stream, records.device)), fn)
+        N.check(getattr(self.lib, fn)(self.h, C.c_void_p(records.data_ptr()), int(S), int(M), int(ladder), int(beta_col), int(stride),
+                                      len(specs[0]), *[N.np_ptr(x) for x in specs], *[C.c_void_p(t.data_ptr()) for t in bufs],
+                                      C.c_void_p(status.data_ptr()), _stream_ptr(stream, records.device)), fn)
         if ladder > 1 and int(status.item()):
             raise ValueError("%s: a ladder has no chain at beta = 1 (%d samples)" % (fn, int(status.item())))
         return bufs
@@ -379,8 +358,8 @@ class Device:
         row i, chain c: split draw i of chain c; slots z, z of |x - median|, x <= q05, x <= q95 of column j at j, n_cols + j,
         2 n_cols + j, 3 n_cols + j) and quant float64 [3, n_cols]: median of the split draws, q05 and q95 of all draws, as numpy
         computes them.  Raises as chain_diagnostics_device does (errors name lr_rank_transform)."""
-        z, q = self._rank_call("lr_rank_transform", records, cols, ladder, beta_col,
-                               [lambda S, M, k: (2 * (S // 2), M, 4 * k), lambda S, M, k: (3, k)], stream)
+        z, q = self._chain_call("lr_rank_transform", records, cols, ladder, beta_col,
+                                [lambda S, M, k: (2 * (S // 2), M, 4 * k), lambda S, M, k: (3, k)], stream)
         return z, q
 
     def rank_diagnostics_device(self, records, cols, ladder=1, beta_col=-1, stream=None):
@@ -388,7 +367,7 @@ class Device:
         copying the records; diagnostics.rank_rhat_ess is the definition.  Arguments as for chain_diagnostics_device.  Returns a
         dict of float64 CUDA tensors [n_cols]: median, q05, q95, rhat_bulk, rhat_tail, rhat_rank, ess_bulk, ess_tail.  Raises as
         chain_diagnostics_device does (errors name lr_rank_diagnostics).  Returns when the outputs are written."""
-        (out,) = self._rank_call("lr_rank_diagnostics", records, cols, ladder, beta_col, [lambda S, M, k: (8, k)], stream)
+        (out,) = self._chain_call("lr_rank_diagnostics", records, cols, ladder, beta_col, [lambda S, M, k: (8, k)], stream)
         return dict(zip(RANK_FIELDS, out))
 
     def new_accumulators(self, n_rep, n_bins, device):

@@ -148,20 +148,28 @@ def log_stem(path):
     return path[:-len(".trendrate.log")] if path.endswith(".trendrate.log") else path[:-len(".log")]
 
 
-def _log_columns(path, kind, burnin):
-    """The post-burn-in rows of one log as the columns of column_specs (the net rate formed as the kernel does)."""
+def read_log(path, burnin):
+    """The post-burn-in rows of a TrendRate / DDRate sample log -> (header, n_bins, col): col(name) is the column of that header
+    name, or for net_<j> the net rate l_<j> - m_<j> formed as the kernels do."""
     with open(path) as fh:
         head = fh.readline().rstrip("\r\n").split("\t")
     tbl = np.loadtxt(path, delimiter="\t", skiprows=1, ndmin=2)
     tbl = tbl[S.burnin_index(tbl.shape[0], burnin):]
     idx = {h: i for i, h in enumerate(head)}
-    n_bins = sum(1 for h in head if re.fullmatch(r"l_\d+", h))
-    col = lambda tag, j: tbl[:, idx["%s_%d" % (tag, j)]]
-    cols = [col("l", j) for j in range(n_bins)] + [col("m", j) for j in range(n_bins)] + [col("l", j) - col("m", j) for j in range(n_bins)]
-    if kind == "dd":
-        cols += [col(t, j) for t in ("niche", "nicheFrac") for j in range(n_bins)]
-    cols += [tbl[:, idx[p]] for p in param_names(kind)]
-    return np.stack(cols, axis=1), n_bins
+
+    def col(name):
+        if name.startswith("net_"):
+            return tbl[:, idx["l_" + name[4:]]] - tbl[:, idx["m_" + name[4:]]]
+        return tbl[:, idx[name]]
+    return head, sum(1 for h in head if re.fullmatch(r"l_\d+", h)), col
+
+
+def _log_columns(path, kind, burnin):
+    """The post-burn-in rows of one log as the columns of column_specs."""
+    _, n_bins, col = read_log(path, burnin)
+    tags = ("l", "m", "net") + (("niche", "nicheFrac") if kind == "dd" else ())
+    names = ["%s_%d" % (t, j) for t in tags for j in range(n_bins)] + param_names(kind)
+    return np.stack([col(nm) for nm in names], axis=1), n_bins
 
 
 def summarize_logs(paths, burnin=0.2, origin=None, name=None):

@@ -181,6 +181,17 @@ def hpd_device(x, level=0.95):
     return s.gather(0, i)[0], s.gather(0, i + (n_in - 1))[0]
 
 
+def marginal_chunks(dev, records, first_edge, n_bins, budget=1 << 30):
+    """K5's per-sample marginal rates of device-resident records [..., 144] (lr_marginal_rates), a range of bins at a time so
+    that each matrix takes at most `budget` bytes (one bin at least): yields (lo, cnt, birth, death), birth and death float64
+    CUDA tensors [n_records, cnt] for the bins [lo, lo + cnt).  A caller that deletes a chunk before taking the next holds one."""
+    n = records.numel() // E.LR_REC_DOUBLES
+    step = max(1, min(n_bins, int(budget // (8 * max(n, 1)))))
+    for lo in range(0, n_bins, step):
+        cnt = min(step, n_bins - lo)
+        yield (lo, cnt) + tuple(dev.marginal_rates_device(records, first_edge, n_bins, lo, cnt))
+
+
 def summarize_records_device(dev, records, start_time, end_time, burnin=0.2, hpd=False, hpd_bytes=1 << 30):
     """Means, shift frequencies and number-of-rates counts of device-resident records (a float64 CUDA tensor
     [n_samples, n_chains, 144]) without bringing them to the host (K5, lr_summarize_records).  With ``hpd`` the 95 % HPD
@@ -198,10 +209,8 @@ def summarize_records_device(dev, records, start_time, end_time, burnin=0.2, hpd
     out["net_mean"] = out["birth"]["mean"] - out["death"]["mean"]
     if hpd:
         import torch
-        step = max(1, min(nb, int(hpd_bytes // (8 * max(n, 1)))))
         parts = {"birth": [], "death": [], "net": []}
-        for lo in range(0, nb, step):
-            mb, md = dev.marginal_rates_device(post, start_time, nb, lo, min(step, nb - lo))
+        for _, _, mb, md in marginal_chunks(dev, post, start_time, nb, hpd_bytes):
             for name, m in (("birth", mb), ("death", md), ("net", mb - md)):
                 parts[name].append(torch.stack(hpd_device(m)))
             del mb, md
