@@ -22,6 +22,7 @@ struct ChainState {
     long long solo_until;               // the team build leaves the chain to the continuation pass while it < solo_until
     unsigned win_iters, win_commits;    // the team build's current observation window (state changes per iteration)
     long long solo_span;                // how long the next hand-over lasts (doubles while the teams keep stopping)
+    long long run_begin;                // first iteration of the current launch (time-sliced teams when the chains' counters differ)
     int K_l, K_m, rep, poi_is_init;
     unsigned chain_id, consistent;
     double priorA, poiA, gL, gM, poi, beta;
@@ -41,6 +42,10 @@ struct lr_chains_s {
     ChainState* st;       // device [n_chains]
     lr_last_stream last;  // stream that touched the chains last (lr_order)
     long long it_host;    // iteration counter of every chain as the host knows it (-1: chains differ, set through set_state)
+    bool fresh;           // not run or set since lr_chains_create: every chain is inside its initial hand-over span
+    int* place;           // device [2 * sm_count]: placement of the time-sliced teams (allocated by the first sliced launch)
+    cudaStream_t side;    // the second stream of the time-sliced teams and its two events (created with `place`)
+    cudaEvent_t fork, join;
 };
 
 namespace {
@@ -1385,14 +1390,19 @@ extern "C" int lr_chains_create(lr_handle_t h, lr_dataset_t ds, int32_t n_chains
     lr_chains_t c = new lr_chains_s();
     c->last.s = h->stream; c->last.valid = 1;
     c->h = h; c->ds = ds; c->n_chains = n_chains; c->cfg = *cfg; c->seed = seed; c->chain_id0 = chain_id0; c->st = nullptr; c->it_host = 0;
+    c->fresh = true; c->place = nullptr; c->side = nullptr; c->fork = nullptr; c->join = nullptr;
     if (c->cfg.beta == 0.0) c->cfg.beta = 1.0;
     cudaError_t e = cudaMallocAsync((void**)&c->st, (size_t)n_chains * sizeof(ChainState), h->stream);
     if (e != cudaSuccess) { lr_set_error("lr_chains_create: cudaMallocAsync: %s", cudaGetErrorString(e)); delete c; return LR_ERR_NOMEM; }
+    // No synchronisation at the end: the handle's stream is ordered behind the dataset and so behind whatever ran before it
+    // (in a sequence of tables: the previous table's chains); waiting for it here would leave the GPU idle while the caller
+    // enqueues the run.  The replicate map therefore gets a block of its own, returned in stream order once the initial
+    // states are written (the shared workspace may be handed to the next entry point before that); the copy from pageable
+    // memory is staged before cudaMemcpyAsync returns, so the caller may free its array at once.
     int* d_rep = nullptr;
     if (h_rep_of_chain) {
-        int rc = lr_ws_acquire(h, (size_t)n_chains * 4, h->stream);
-        if (rc != LR_OK) { cudaFreeAsync(c->st, h->stream); delete c; return rc; }
-        d_rep = (int*)h->ws;
+        e = cudaMallocAsync((void**)&d_rep, (size_t)n_chains * 4, h->stream);
+        if (e != cudaSuccess) { lr_set_error("lr_chains_create: cudaMallocAsync: %s", cudaGetErrorString(e)); cudaFreeAsync(c->st, h->stream); delete c; return LR_ERR_NOMEM; }
         LR_CUDA(cudaMemcpyAsync(d_rep, h_rep_of_chain, (size_t)n_chains * 4, cudaMemcpyHostToDevice, h->stream));
     }
     int threads;
@@ -1401,7 +1411,7 @@ extern "C" int lr_chains_create(lr_handle_t h, lr_dataset_t ds, int32_t n_chains
                                                       ds->start_time, cfg->poisson_prior, c->cfg.beta);
     LR_CUDA(cudaGetLastError());
     h->launches += 1;
-    LR_CUDA(cudaStreamSynchronize(h->stream));
+    if (d_rep) LR_CUDA(cudaFreeAsync(d_rep, h->stream));
     *out = c;
     return LR_OK;
 }
@@ -1411,6 +1421,10 @@ extern "C" int lr_chains_destroy(lr_chains_t c) {
     cudaSetDevice(c->h->device);
     lr_order(c->h, &c->last, c->h->stream);
     cudaFreeAsync(c->st, c->h->stream);
+    if (c->place) {
+        cudaFreeAsync(c->place, c->h->stream);
+        cudaEventDestroy(c->fork); cudaEventDestroy(c->join); cudaStreamDestroy(c->side);    // released once their work is done
+    }
     delete c;
     return LR_OK;
 }
@@ -1493,28 +1507,69 @@ extern "C" int lr_chains_run(lr_chains_t c, int64_t n_iter, int64_t sample_every
             cudaFuncSetAttribute(k3_team_kernel<10>, cudaFuncAttributePreferredSharedMemoryCarveout, 30);
             cudaFuncSetAttribute(k3_team_kernel<12>, cudaFuncAttributePreferredSharedMemoryCarveout, 30);
             cudaFuncSetAttribute(k3_team_kernel<4>, cudaFuncAttributePreferredSharedMemoryCarveout, 30);
+            cudaFuncSetAttribute(k3_team_slot_kernel<16>, cudaFuncAttributePreferredSharedMemoryCarveout, 30);
+            cudaFuncSetAttribute(k3_team_slot_kernel<8>, cudaFuncAttributePreferredSharedMemoryCarveout, 30);
             carve_set = true;
         }
-        auto launch_team = [&]() {
+        // Between one and two chains per SM (the automatic width 8) with at least one SM in eight left to a single chain:
+        // time-sliced teams in one CTA of 16 warps per SM, see k3_team_slot_kernel.  LR_TEAM_SLICE_US sets the slice length in
+        // microseconds (0: one CTA per chain, as for the other widths).  Each slice costs a placement kernel, the drain of the
+        // slowest team and the teams' restart: about 2 % of the teams' time at 2 ms slices, which the lone SMs have to pay for
+        // (B200, bench statistics: 256 chains +6 %, 296 chains -2 %, where every SM holds two).  The number of slices is
+        // planned from the run's work at TEAM_SLICE_PLAN_RATE; a slice with nothing to do returns at once, and the last slice
+        // has no time limit.
+        const char* e_slice = getenv("LR_TEAM_SLICE_US");
+        const long long slice_us = e_slice ? atoll(e_slice) : 2000;
+        const bool sliced = !env_w && c->n_chains > sm && c->n_chains <= 2 * sm - sm / 8 && c->n_chains <= TEAM_PLACE_MAX && slice_us > 0;
+        if (sliced && !c->place) {
+            cudaError_t e = cudaMallocAsync((void**)&c->place, (size_t)2 * sm * sizeof(int), st);
+            if (e != cudaSuccess) { lr_set_error("lr_chains_run: cudaMallocAsync: %s", cudaGetErrorString(e)); return LR_ERR_NOMEM; }
+            LR_CUDA(cudaStreamCreateWithFlags(&c->side, cudaStreamNonBlocking));
+            LR_CUDA(cudaEventCreateWithFlags(&c->fork, cudaEventDisableTiming));
+            LR_CUDA(cudaEventCreateWithFlags(&c->join, cudaEventDisableTiming));
+        }
+        bool first = true;
+        auto launch_team = [&]() -> cudaError_t {
+            if (sliced) {
+                const double work_us = (double)c->n_chains * (double)n_iter / (TEAM_SLICE_PLAN_RATE * sm);
+                const long long n_slices = 1 + (long long)(work_us / (double)slice_us);
+                for (long long k = 0; k < n_slices; ++k) {
+                    const long long budget = k + 1 < n_slices ? slice_us * 1000 : 0;
+                    k3_team_place_kernel<<<1, TEAM_PLACE_MAX, 0, st>>>(P, c->place, sm, first ? 1 : 0);
+                    cudaError_t e = cudaEventRecord(c->fork, st);
+                    if (e == cudaSuccess) e = cudaStreamWaitEvent(c->side, c->fork, 0);
+                    if (e != cudaSuccess) return e;
+                    k3_team_slot_kernel<16><<<sm, 512, 0, st>>>(P, lead, c->place, budget);
+                    k3_team_slot_kernel<8><<<sm, 512, 0, c->side>>>(P, lead, c->place, budget);
+                    e = cudaEventRecord(c->join, c->side);
+                    if (e == cudaSuccess) e = cudaStreamWaitEvent(st, c->join, 0);
+                    if (e != cudaSuccess) return e;
+                    h->launches += 3;
+                    first = false;
+                }
+                return cudaSuccess;
+            }
             if (W >= 16) k3_team_kernel<16><<<c->n_chains, 512, 0, st>>>(P, lead);
             else if (W == 12) k3_team_kernel<12><<<c->n_chains, 384, 0, st>>>(P, lead);
             else if (W == 10) k3_team_kernel<10><<<c->n_chains, 320, 0, st>>>(P, lead);
             else if (W >= 8) k3_team_kernel<8><<<c->n_chains, 256, 0, st>>>(P, lead);
             else k3_team_kernel<4><<<c->n_chains, 128, 0, st>>>(P, lead);
             h->launches += 1;
+            return cudaSuccess;
         };
         // Four passes over the same launch window; every kernel skips the chains that have nothing to do in it.
         //   A  teams; a team whose chain changes state too often stops early and hands the chain over for a while
+        //      (nothing to do for chains fresh from lr_chains_create: they all start inside a hand-over span)
         //   B  latency-optimised build: handed-over chains, up to the end of their hand-over
         //   C  teams again for the chains whose hand-over ended inside the window (burn-in is over: speculation pays now)
         //   D  latency-optimised build: whatever is left
-        launch_team();
+        if (!(c->fresh && P.team_bail)) LR_CUDA(launch_team());
         if (P.team_bail) {
             const int cont = c->n_chains <= 2 * sm ? 1 : 3;
             LR_CUDA(cudaGetLastError());
             P.cont_mode = 1; launch_plain(cont);
             LR_CUDA(cudaGetLastError());
-            P.cont_mode = 0; launch_team();
+            P.cont_mode = 0; LR_CUDA(launch_team());
             LR_CUDA(cudaGetLastError());
             launch_plain(cont);
         }
@@ -1523,6 +1578,7 @@ extern "C" int lr_chains_run(lr_chains_t c, int64_t n_iter, int64_t sample_every
     }
     LR_CUDA(cudaGetLastError());
     if (c->it_host >= 0) c->it_host += n_iter;
+    c->fresh = false;
     return LR_OK;
 }
 
@@ -1581,6 +1637,7 @@ extern "C" int lr_chains_set_state_host(lr_chains_t c, const double* h_records) 
         if ((long long)r[0] != it_all) it_all = -1;
     }
     c->it_host = it_all;
+    c->fresh = false;
     LR_CUDA(cudaSetDevice(h->device));
     { int rc0 = lr_order(h, &c->last, h->stream); if (rc0 == LR_OK) rc0 = lr_order(h, &c->ds->last, h->stream); if (rc0 != LR_OK) return rc0; }
     const size_t bytes = (size_t)c->n_chains * LR_REC_DOUBLES * sizeof(double);

@@ -33,7 +33,10 @@ template <int W>
 struct TeamShared {
     unsigned long long verword;
     unsigned long long prog[W];
-    unsigned n_eff;            // iterations of this launch the team does (lowered when it hands the chain over)
+    unsigned n_eff;            // iterations of this launch the team does (lowered when it hands the chain over or its time slice ends)
+    unsigned stopped;          // n_eff was lowered because the time slice ended (not a hand-over)
+    int chain;                 // time-sliced teams: the chain and the end of the slice (global timer, 0: none), kept here
+    unsigned long long t_stop; // and not in registers, which the loop needs all of
     unsigned win_i, win_c;     // observation window: first offset, state changes since then (only the frontier touches them)
     unsigned cnt[W][8];
     unsigned dbg[W][4];        // commits, evaluations dropped by rollbacks, polls while waiting to be the frontier, polls at the lead limit
@@ -202,21 +205,40 @@ __device__ __forceinline__ int team_rj_eval(const Side& cur, const Side& oth, co
     return TEAM_PEND_NONE;
 }
 
-template <int W>
-__global__ void __launch_bounds__(W * 32, W >= 16 ? 1 : (W >= 8 ? 2 : 4)) k3_team_kernel(const RunParams P, const int lead) {
+// barrier of the W warps of one team: the whole CTA, or named barrier 1 / 2 for the two teams of 8 of a slot CTA
+template <int W, bool SLICED>
+__device__ __forceinline__ void team_sync() {
+    if (SLICED && W == 8) asm volatile("bar.sync %0, 256;" :: "r"(1 + (int)(threadIdx.x >> 8)) : "memory");
+    else __syncthreads();
+}
+__device__ __forceinline__ unsigned long long global_ns() {
+    unsigned long long t;
+    asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t));
+    return t;
+}
+
+// One team of W warps runs `chain` for this launch: the CTA (one chain per CTA), or with SLICED one time slice of the slot
+// kernel below, where a CTA of 16 warps is one team of 16 or two teams of 8 (threads 0-255 and 256-511).  There the chain's
+// first iteration of the run is S->run_begin (set by the placement kernel), and once the global timer passes t_stop (0: no
+// limit) the team stops at an iteration no commit has passed and leaves the rest to the next slice.
+template <int W, bool SLICED>
+__device__ __forceinline__ void team_run(const RunParams& P, const int lead, const int chain_arg, const unsigned long long t_stop) {
     constexpr bool C = true;
-    __shared__ TeamShared<W> T;
-    const int lane = threadIdx.x & 31;
-    const int w = threadIdx.x >> 5;
-    const int chain = (int)blockIdx.x;
-    if (chain >= P.n_chains) return;                                  // whole CTA
-    ChainState* S = P.st + chain;
+    __shared__ TeamShared<W> T_all[SLICED && W == 8 ? 2 : 1];
+    TeamShared<W>& T = T_all[SLICED && W == 8 ? (threadIdx.x >> 8) : 0];
+    const int lane = (int)(threadIdx.x & 31);
+    const int w = (int)(SLICED ? (threadIdx.x >> 5) % W : threadIdx.x >> 5);
+    ChainState* S = P.st + chain_arg;
     const long long it0 = S->it;
-    const long long n_own = (P.it_begin >= 0 ? P.it_begin : it0) + P.n_iter - it0;
-    if (n_own <= 0 || (P.team_bail && it0 < S->solo_until)) return;      // whole CTA: nothing to do / left to the continuation pass
-    if (threadIdx.x == 0) { T.verword = 0ull; T.n_eff = (unsigned)n_own; T.win_i = 0u - S->win_iters; T.win_c = S->win_commits; }
-    if (threadIdx.x < W) T.prog[threadIdx.x] = (unsigned long long)threadIdx.x;
-    __syncthreads();
+    const long long it_begin = P.it_begin >= 0 ? P.it_begin : (SLICED ? S->run_begin : it0);
+    const long long n_own = it_begin + P.n_iter - it0;
+    if (n_own <= 0 || (P.team_bail && it0 < S->solo_until)) return;      // whole team: nothing to do / left to the continuation pass
+    if (w == 0 && lane == 0) {
+        T.verword = 0ull; T.n_eff = (unsigned)n_own; T.stopped = 0u; T.win_i = 0u - S->win_iters; T.win_c = S->win_commits;
+        T.chain = chain_arg; T.t_stop = t_stop;
+    }
+    if (w == 0 && lane < W) T.prog[lane] = (unsigned long long)lane;
+    team_sync<W, SLICED>();
 
     const lr_chain_config& cfg = P.cfg;
     const LoopConsts& K = P.lc;
@@ -231,14 +253,13 @@ __global__ void __launch_bounds__(W * 32, W >= 16 ? 1 : (W >= 8 ? 2 : 4)) k3_tea
     c.hp.gL = S->gL; c.hp.gM = S->gM; c.hp.lgL = log(c.hp.gL); c.hp.lgM = log(c.hp.gM); c.hp.poi = S->poi; c.hp.lpoi = log(c.hp.poi);
     c.priorA = S->priorA; c.poiA = S->poiA; c.beta = S->beta; c.poi_is_init = S->poi_is_init; c.consistent = (int)S->consistent;
     const bool frozen = (d.end_time - d.start_time) <= LR_MIN_DT;
-    __syncthreads();                  // every warp has read the chain's global state before anybody may finish and rewrite it
+    team_sync<W, SLICED>();           // every warp has read the chain's global state before anybody may finish and rewrite it
 
     TeamEvents ev;
     {
         const unsigned long long s_every = (unsigned long long)(P.sample_every > 0 ? P.sample_every : 1);
         ev.s_every = s_every;
         ev.first_sample = P.records != nullptr ? (s_every - (unsigned long long)it0 % s_every) % s_every : ~0ull;
-        const long long it_begin = P.it_begin >= 0 ? P.it_begin : it0;
         ev.rec_done = (unsigned long long)((it0 + (long long)s_every - 1) / (long long)s_every - (it_begin + (long long)s_every - 1) / (long long)s_every);
         ev.first_resync = (LR_RESYNC - (unsigned long long)it0 % LR_RESYNC) % LR_RESYNC;
     }
@@ -291,6 +312,20 @@ __global__ void __launch_bounds__(W * 32, W >= 16 ? 1 : (W >= 8 ? 2 : 4)) k3_tea
             const unsigned nxt = (unsigned)(pw >> 32) == v ? (unsigned)pw : base;
             F_seen = __reduce_min_sync(0xffffffffu, nxt);
             if (i > F_seen + lead_span) { ++n_lead; __nanosleep(100); continue; }
+        }
+        if (SLICED && w == 0 && (i & (16u * W - 1u)) == 15u * W && *(volatile unsigned long long*)&T.t_stop != 0ull &&
+            __shfl_sync(0xffffffffu, global_ns(), 0) >= *(volatile unsigned long long*)&T.t_stop) {
+            // the slice is over (the timer is read every 16th own iteration: a slice does at least 15 W iterations): once every
+            // earlier iteration is published, the team stops BEFORE iteration i, which nobody has committed or observed.  The
+            // state stays as it is; the new version only carries the lowered n_eff to the others, which trim what they
+            // evaluated at or beyond i as after a hand-over.
+            if (!team_wait_frontier<W>(T, v, i, w, lane, n_fwait)) continue;
+            v = (v + 1u) & TEAM_VMASK; base = i; n = i;
+            if (lane == 0) { *(volatile unsigned*)&T.n_eff = i; *(volatile unsigned*)&T.stopped = 1u; }
+            __syncwarp();
+            team_publish_state<W>(T, v, 0u, i, L, M, c, lane);
+            if (lane == 0) st_volatile_shared(&T.prog[w], ((unsigned long long)v << 32) | i);
+            continue;
         }
 
         const long long it = it0 + (long long)i;
@@ -346,6 +381,7 @@ __global__ void __launch_bounds__(W * 32, W >= 16 ? 1 : (W >= 8 ? 2 : 4)) k3_tea
             if (i == ev.next_resync) { resync_log_rates(L, M, lane); changed |= TD_LV | TD_MV; }
             if (i == ev.next_sample) {
                 const unsigned long long k = ev.rec_done + ((unsigned long long)i - ev.first_sample) / ev.s_every;
+                const int chain = SLICED ? *(volatile int*)&T.chain : chain_arg;
                 write_record_ref(P.records + ((size_t)k * P.n_chains + chain) * LR_REC_DOUBLES, it, L, M, c, d, lane, P.with_adequacy != 0);
             }
         }
@@ -381,14 +417,15 @@ __global__ void __launch_bounds__(W * 32, W >= 16 ? 1 : (W >= 8 ? 2 : 4)) k3_tea
     tc_flush(tc);
     if (lane < 8) T.cnt[w][lane] = tc.n[lane];
     if (lane == 0) { T.dbg[w][0] = n_commit; T.dbg[w][1] = n_drop; T.dbg[w][2] = n_fwait; T.dbg[w][3] = n_lead; }
-    __syncthreads();
+    team_sync<W, SLICED>();
     if (w == 0) {
+        ChainState* S = P.st + (SLICED ? *(volatile int*)&T.chain : chain_arg);
         store_sides(S, L, M, lane);
         if (lane == 0) {
             const unsigned n_done = *(volatile unsigned*)&T.n_eff;
             S->it = it0 + (long long)n_done;
             S->team[4] += (long long)n_done;
-            if (n_done < (unsigned)n_own) {
+            if (n_done < (unsigned)n_own && !*(volatile unsigned*)&T.stopped) {
                 S->team[5] += 1;
                 // handed over: for solo_span iterations, twice as long the next time
                 const long long span = S->solo_span < TEAM_SOLO_SPAN_MIN ? TEAM_SOLO_SPAN_MIN : S->solo_span;
@@ -411,5 +448,63 @@ __global__ void __launch_bounds__(W * 32, W >= 16 ? 1 : (W >= 8 ? 2 : 4)) k3_tea
                 S->team[k] += s;
             }
         }
+    }
+}
+
+template <int W>
+__global__ void __launch_bounds__(W * 32, W >= 16 ? 1 : (W >= 8 ? 2 : 4)) k3_team_kernel(const RunParams P, const int lead) {
+    if ((int)blockIdx.x >= P.n_chains) return;                       // whole CTA
+    team_run<W, false>(P, lead, (int)blockIdx.x, 0ull);
+}
+
+// ---- time-sliced teams (between one and two chains per SM).  One CTA per SM of 16 warps hosts either ONE chain as a team
+// of 16 or TWO chains as two teams of 8 (with their own shared state and barrier), as the placement kernel says.  A team of 8
+// that shares its SM runs at about 4 iterations per microsecond, a team of 16 alone at about 6: with one CTA per chain the
+// chains that share an SM set the launch's time while the SMs of the lone chains run out of work.  Slices of a fixed time
+// (measured from the CTA's start) with the chains furthest behind moved to the lone slots in between keep every SM busy to the
+// end; a chain is the same chain however its launch is cut (event iterations sit at absolute iteration numbers).
+#define TEAM_SLICE_PLAN_RATE 6.0     // chain iterations per microsecond and SM the number of slices is planned with (bench statistics:
+                                     // about 8 for two teams of 8, 6 for one of 16; a slower table leaves more to the last slice)
+// The two layouts are two kernels, launched side by side on two streams over all slots; each CTA runs only the slots of its
+// layout and returns at once from the others, so the SMs end up with one CTA each.  (One kernel with both bodies costs the
+// registers of both: spills that made either layout 5 - 8 % slower than the one-chain-per-CTA kernels.)
+template <int W>
+__global__ void __launch_bounds__(512, 1) k3_team_slot_kernel(const RunParams P, const int lead, const int* __restrict__ place, const long long budget_ns) {
+    const int a = place[2 * blockIdx.x], b = place[2 * blockIdx.x + 1];
+    if (a < 0 || (b < 0) != (W == 16)) return;                      // no chain, or the other layout's slot
+    const unsigned long long t_stop = budget_ns > 0 ? global_ns() + (unsigned long long)budget_ns : 0ull;
+    team_run<W, true>(P, lead, W == 16 || threadIdx.x < 256 ? a : b, t_stop);
+}
+
+// Placement of the next slice: slot CTA s runs chain place[2 s] (-1: none), alone if place[2 s + 1] is -1, else beside it.  The
+// chains furthest behind the end of the launch get the lone slots (every chain gets one once at most n_slots are left); chains
+// that are done or inside a hand-over span get none.  first: the first slice of the launch, which records where each chain starts.
+#define TEAM_PLACE_MAX 1024
+__global__ void __launch_bounds__(TEAM_PLACE_MAX) k3_team_place_kernel(const RunParams P, int* __restrict__ place, const int n_slots, const int first) {
+    __shared__ long long left[TEAM_PLACE_MAX];
+    __shared__ int n_active;
+    const int n = P.n_chains;                                        // <= 2 n_slots and <= TEAM_PLACE_MAX (lr_chains_run)
+    if (threadIdx.x == 0) n_active = 0;
+    for (int s = threadIdx.x; s < 2 * n_slots; s += blockDim.x) place[s] = -1;
+    __syncthreads();
+    for (int c = threadIdx.x; c < n; c += blockDim.x) {
+        ChainState* S = P.st + c;
+        const long long it = S->it;
+        if (first) S->run_begin = it;
+        const long long end = (P.it_begin >= 0 ? P.it_begin : S->run_begin) + P.n_iter;
+        const bool active = it < end && !(P.team_bail && it < S->solo_until);
+        left[c] = active ? end - it : -1;
+        if (active) atomicAdd(&n_active, 1);
+    }
+    __syncthreads();
+    const int m = n_active;
+    const int n_lone = m <= n_slots ? m : 2 * n_slots - m;
+    for (int c = threadIdx.x; c < n; c += blockDim.x) {
+        const long long k = left[c];
+        if (k < 0) continue;
+        int r = 0;                                                   // rank: chains with more left go first, ties by index
+        for (int j = 0; j < n; ++j) r += (left[j] > k || (left[j] == k && j < c)) ? 1 : 0;
+        if (r < n_lone) place[2 * r] = c;
+        else { const int q = r - n_lone; place[2 * (n_lone + q / 2) + (q & 1)] = c; }
     }
 }
