@@ -285,11 +285,7 @@ __device__ __forceinline__ Draws make_draws(const Rng& rng, long long it, int la
     rng.draw(it, 0, lane, ua, ub);
     const double r0 = __shfl_sync(0xffffffffu, ua, 31), r1 = __shfl_sync(0xffffffffu, ub, 31);   // np.random.random(2) of :234
     q.u_acc = __shfl_sync(0xffffffffu, ua, 30);
-    // bracket of log(u) for the accept test (error bound: __logf <= 2^-21.4 absolute on [.5,2], 3 ulp elsewhere, plus the
-    // rounding of u to float)
-    const float lf = __logf((float)q.u_acc);
-    const float err = 2e-6f * (1.0f + fabsf(lf));
-    q.thr_hi = (double)(lf + err); q.thr_lo = (double)(lf - err);
+    mh_bracket(q.u_acc, &q.thr_lo, &q.thr_hi);         // bracket of log(u) for the accept test
     q.u_idx = 0.0; q.u_t = 0.0; q.w = 0.0; q.ln_beta = 0.0; q.m = 1.0; q.dlt = 0.0;
     if (r0 < k.d_freq) {
         // update_multiplier_freq (:165-176): each rate w.p. f times exp(2 ln(1.1) (u - .5))
@@ -472,13 +468,8 @@ __device__ __forceinline__ bool propose_move(const Side& cur, Side& nw, const Da
     return true;
 }
 
-// Metropolis-Hastings test `x >= log(u)` (:313).  The double-precision logarithm is only evaluated when the
-// single-precision bracket [thr_lo, thr_hi] of log(u) cannot decide; the decision is the one the exact comparison gives.
-__device__ __forceinline__ bool mh_accept(double x, const Draws& q) {
-    if (x >= q.thr_hi) return true;
-    if (x < q.thr_lo) return false;                // also taken for x = -inf
-    return x >= ool_log(q.u_acc);                  // NaN lands here and is rejected
-}
+// Metropolis-Hastings test `x >= log(u)` (:313) of the iteration's draws (mh_accept_ge, lr_common.cuh)
+__device__ __forceinline__ bool mh_accept(double x, const Draws& q) { return mh_accept_ge(x, q.u_acc, q.thr_lo, q.thr_hi, ool_log); }
 
 // everything of a chain that is not one of the two sides
 struct ChainRegs {

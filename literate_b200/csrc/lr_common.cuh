@@ -455,15 +455,29 @@ __device__ __forceinline__ double exp_small(double x) {
     return p;
 }
 
-// Metropolis-Hastings test `x > log(u)` with the double-precision logarithm evaluated only when a single-precision bracket of
-// log(u) cannot decide (error bound: __logf <= 2^-21.4 absolute on [.5, 2], 3 ulp elsewhere, plus the rounding of u to float);
-// the decision is always the one the exact comparison gives.  NaN and -inf are rejected.
-__device__ __forceinline__ bool mh_accept_gt(double x, double u) {
+// Single-precision bracket [*lo, *hi] of the double log(u) of a uniform u in (0, 1) (error bound: __logf <= 2^-21.4 absolute on
+// [.5, 2], 3 ulp elsewhere, plus the rounding of u to float).  The Metropolis-Hastings tests below evaluate the double-precision
+// logarithm only when x falls inside it; their decision is always the one the exact comparison with log(u) gives.
+__device__ __forceinline__ void mh_bracket(double u, double* lo, double* hi) {
     const float lf = __logf((float)u);
     const float err = 2e-6f * (1.0f + fabsf(lf));
-    if (x > (double)(lf + err)) return true;
-    if (!(x >= (double)(lf - err))) return false;
+    *hi = (double)(lf + err); *lo = (double)(lf - err);
+}
+// `x > log(u)` (K6, K7).  NaN and -inf are rejected.
+__device__ __forceinline__ bool mh_accept_gt(double x, double u) {
+    double lo, hi;
+    mh_bracket(u, &lo, &hi);
+    if (x > hi) return true;
+    if (!(x >= lo)) return false;
     return x > log(u);
+}
+// `x >= log(u)` (K3) from the bracket [lo, hi] of mh_bracket, which K3 computes with its other draws; log_fn(u) is the
+// double-precision logarithm (K3 passes its out-of-line one).  -inf is rejected by the bracket, NaN by the last comparison.
+template <class Log>
+__device__ __forceinline__ bool mh_accept_ge(double x, double u, double lo, double hi, Log log_fn) {
+    if (x >= hi) return true;
+    if (x < lo) return false;
+    return x >= log_fn(u);
 }
 
 // standard normal from two uniforms in single precision (Box-Muller); a proposal step, not a likelihood term: 24 bits suffice
