@@ -162,6 +162,12 @@ int lr_dataset_create_general_host(lr_handle_t h, int32_t n_rep, int32_t n_bins,
                                    const double* h_A_birth, const double* h_B_birth, const double* h_A_death, const double* h_B_death,
                                    const double* h_x_birth, const double* h_x_death, const double* h_C, lr_dataset_t* out);
 int lr_dataset_destroy(lr_dataset_t ds);
+/* The per-bin terms the likelihood of the dataset sums: d_out fp64 [n_rep][4][n_bins] = A_birth, B_birth, A_death, B_death of every
+ * bin (the likelihood is C + sum_j [A_birth_j log lambda_j - B_birth_j lambda_j] + the same for deaths).  For the -model_BDI tables:
+ * model 0 A = sp / ex, B = br, bins with br = 0 masked to 0; model 1 B_birth = 1 on the bins with br > 0; model 2 no mask; model 3
+ * the death side from the extinct-only statistics.  For lr_dataset_create_general_host the A and B given.  These are the values
+ * whose running sums are the prefix tables, stored as computed (not recovered from the tables).  Asynchronous on `stream`. */
+int lr_dataset_bin_terms(lr_dataset_t ds, double* d_out, void* stream);
 
 #define LR_KMAX 30   /* most rates per side a state can hold (slots of one warp minus two control lanes) */
 
@@ -375,6 +381,42 @@ int lr_rank_transform(lr_handle_t h, const double* d_rows, int64_t n_samples, in
 int lr_rank_diagnostics(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
                         int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b, const int32_t* h_col_sign,
                         const double* h_col_add, double* d_out, int64_t* d_status, void* stream);
+/* K11: posterior predictive check of the per-bin births and deaths of a run, without copying the records (new; the reference
+ * has only the adequacy regression).  literate_b200.predictive.predictive_check_host is the definition, step for step.
+ * Model: every likelihood here is C + sum_j [A^b_j log lambda_j - B^b_j lambda_j] + sum_j [A^d_j log mu_j - B^d_j mu_j], so given a
+ * record the count of side s in bin j is Poisson(rate_sj B_sj), with the exposure B held at its observed value (no new lineage
+ * table is simulated).
+ *   rows         the records of K3 / K6 / K7 in the (s, k) layout, ladder and beta_col of lr_chain_diagnostics (cold members of
+ *                tempered ladders).  Burn-in: offset the pointer.  n_samples >= 4.
+ *   layout       0: RJMCMC records (LR_REC_DOUBLES; bin j takes the rate of the segment it falls in under the likelihood's mapping:
+ *                segment k starts at bin floor(t_k) - floor(start_time), clamped to [0, n_bins], slot 0 at bin 0); 1: dense records
+ *                whose birth rates are the fields [rate_col, rate_col + n_bins) and death rates the next n_bins (K6: 16, K7: 24)
+ *   d_terms      fp64 [n_rep][4][n_bins]: A^b, B^b, A^d, B^d (lr_dataset_bin_terms for K3; sp, br, ex, br of the statistics for
+ *                K6 / K7); logical chain c is compared with replicate h_rep_of_chain[c] (HOST [n_chains], NULL: all 0)
+ *   draws        one Poisson count (lr_poisson of lr_common.cuh) per used record, side s (0 birth, 1 death) and bin j with B > 0,
+ *                from Philox-4x32-10 with key (seed low 32 bits, seed high 32 bits) and counter (it low 32 bits, it high 32 bits,
+ *                j | s << 24 | attempt << 25, low 32 bits of chain_id0 + c), it = the record's field 0 as an integer: the result
+ *                depends neither on the burn-in cut nor on how runs were split, nor on whether the records came from logs
+ *   used         a record is used unless its ladder has no member at beta = 1, a rate times B is negative, NaN or above 2^52, its
+ *                iteration field is outside [0, 9.2e18), or (layout 0) K is not 1..32 or its segments are non-finite or out of order
+ * Outputs:
+ *   d_bin_count  int64 [2][4][n_bins]: records used, sum of y_rep, #(y_rep > A), #(y_rep == A), per side and bin (0 where B = 0)
+ *   d_bin_sum    fp64 [2][3][n_bins]: sum of mu = rate B, of mu^2, of A over those records
+ *   d_glob_count int64 [4]: records used, #(D_rep >= D_obs) of the birth side, the death side and the total
+ *   d_glob_sum   fp64 [6]: sums over the used records of D_obs^b, D_rep^b, D_obs^d, D_rep^d, D_obs, D_rep
+ *   d_dev        fp64 [n_samples][n_chains][4] or NULL: D_obs^b, D_rep^b, D_obs^d, D_rep^d of every record (NaN when not used)
+ *   d_status     int64 [3]: records skipped as unusable, exhausted sampler loops (the draw is then 0), (sample, ladder) pairs
+ *                without a member at beta = 1
+ * D(y, mu) = 2 sum_j [y log(y / mu) - (y - mu)] over the bins of a side with B > 0 (0 log 0 = 0), each sum compensated in a fixed
+ * order; D = D^b + D^d.  Counts are exact and every fp64 sum is compensated in a fixed order: repeated calls are bit-identical.
+ * Scratch comes from the handle's workspace (about 48 bytes per record and 112 bytes per side and bin per 1024 records).  Rejects
+ * what lr_chain_diagnostics rejects, n_bins outside 1 .. 16 776 960, rate fields outside the row and replicates outside [0, n_rep).  Asynchronous on
+ * `stream` (h_rep_of_chain is staged before it returns). */
+int lr_predictive_check(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
+                        int64_t row_stride, int32_t layout, int32_t rate_col, double start_time, int32_t n_bins,
+                        const double* d_terms, int32_t n_rep, const int32_t* h_rep_of_chain, int64_t chain_id0, uint64_t seed,
+                        int64_t* d_bin_count, double* d_bin_sum, int64_t* d_glob_count, double* d_glob_sum, double* d_dev,
+                        int64_t* d_status, void* stream);
 
 /* ---------------------------------------------------------------- TrendRate (SURVEY 8 f-4): fixed-dimension chains on the same statistics
  *

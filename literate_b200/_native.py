@@ -39,6 +39,7 @@ EXPORTS = [
     "lr_dd_run", "lr_dd_run_host", "lr_dd_eval_host", "lr_dd_state_host",
     "lr_dd_set_beta_host", "lr_dd_swap_info", "lr_dd_swap_apply", "lr_dd_swap_step", "lr_dd_temper_host",
     "lr_column_hpd", "lr_chain_diagnostics", "lr_rank_transform", "lr_rank_diagnostics",
+    "lr_dataset_bin_terms", "lr_predictive_check",
 ]
 
 
@@ -103,6 +104,7 @@ def load(build_if_missing=False):
     sig("lr_dataset_create_host", C.c_int, vp, i32, i32, i32, f64, f64, vp, vp, vp, vp, vp, P(vp))
     sig("lr_dataset_create_general_host", C.c_int, vp, i32, i32, i32, f64, f64, vp, vp, vp, vp, vp, vp, vp, P(vp))
     sig("lr_dataset_destroy", C.c_int, vp)
+    sig("lr_dataset_bin_terms", C.c_int, vp, vp, vp)
     sig("lr_state_eval_host", C.c_int, vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp)
     sig("lr_proposal_eval_host", C.c_int, vp, i32, *([vp] * 24))
     sig("lr_loglik_direct", C.c_int, vp, vp, vp, i64, i64, i32, vp, vp, i32, vp, vp)
@@ -126,6 +128,8 @@ def load(build_if_missing=False):
     sig("lr_chain_diagnostics", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, vp, vp, vp, vp, vp, vp, vp)
     sig("lr_rank_transform", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, vp, vp, vp, vp, vp, vp, vp, vp)
     sig("lr_rank_diagnostics", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, vp, vp, vp, vp, vp, vp, vp)
+    sig("lr_predictive_check", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, i32, f64, i32, vp, i32, vp, i64, u64,
+        vp, vp, vp, vp, vp, vp, vp)
     sig("lr_trend_create", C.c_int, vp, i32, i32, vp, vp, vp, vp, i32, i32, i32, u64, i64, vp, vp, P(vp))
     sig("lr_trend_create_host", C.c_int, vp, i32, i32, vp, vp, vp, vp, i32, i32, i32, u64, i64, vp, P(vp))
     sig("lr_trend_destroy", C.c_int, vp)

@@ -38,6 +38,7 @@ struct lr_dataset_s {
     int s0f;               // floor(start_time): a shift at time t starts bin floor(t) - s0f (:262, :125-135)
     double* tab;           // device [n_rep][LR_NTAB][n_bins+1]
     double* cst;           // device [n_rep][LR_NCST]
+    double* terms;         // device [n_rep][4][n_bins]: A^b, B^b, A^d, B^d of every bin, the terms the tables sum
     lr_last_stream last;   // stream that built or read the tables last (lr_order)
 };
 

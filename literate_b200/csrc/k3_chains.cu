@@ -56,7 +56,7 @@ namespace {
 __global__ void k2_build_tables(const long long* __restrict__ sp, const long long* __restrict__ ex,
                                 const double* __restrict__ br, const long long* __restrict__ exd,
                                 const double* __restrict__ brd, int nb, int model, double* __restrict__ tab_all,
-                                double* __restrict__ cst_all) {
+                                double* __restrict__ cst_all, double* __restrict__ terms_all) {
     const int rep = blockIdx.x, t = threadIdx.x;
     const long long* U = sp + (size_t)rep * nb;
     const long long* D = ex + (size_t)rep * nb;
@@ -79,6 +79,7 @@ __global__ void k2_build_tables(const long long* __restrict__ sp, const long lon
                 case T_XB: v = (double)U[j] / K[j]; break;
                 case T_XD: v = (double)D[j] / K[j]; break;
             }
+            if (t < 4) terms_all[((size_t)rep * 4 + t) * nb + j] = v;     // the likelihood's per-bin terms (lr_dataset_bin_terms)
             acc += v;
             T[j + 1] = acc;
         }
@@ -107,7 +108,8 @@ __global__ void k2_build_tables(const long long* __restrict__ sp, const long lon
 // running total > 0, B = that mask, C = 0; x_b / x_d are the vectors calculate_r_squared regresses on (:627-628: the counts).
 __global__ void k2_build_tables_general(const double* __restrict__ Ab, const double* __restrict__ Bb, const double* __restrict__ Ad,
                                         const double* __restrict__ Bd, const double* __restrict__ xb, const double* __restrict__ xd,
-                                        const double* __restrict__ C, int nb, double* __restrict__ tab_all, double* __restrict__ cst_all) {
+                                        const double* __restrict__ C, int nb, double* __restrict__ tab_all, double* __restrict__ cst_all,
+                                        double* __restrict__ terms_all) {
     const int rep = blockIdx.x, t = threadIdx.x;
     double* tab = tab_all + (size_t)rep * LR_NTAB * (nb + 1);
     const size_t o = (size_t)rep * nb;
@@ -116,7 +118,10 @@ __global__ void k2_build_tables_general(const double* __restrict__ Ab, const dou
         double acc = 0.0;
         double* T = tab + (size_t)t * (nb + 1);
         T[0] = 0.0;
-        for (int j = 0; j < nb; ++j) { acc += src[o + j]; T[j + 1] = acc; }
+        for (int j = 0; j < nb; ++j) {
+            if (t < 4) terms_all[((size_t)rep * 4 + t) * nb + j] = src[o + j];
+            acc += src[o + j]; T[j + 1] = acc;
+        }
     } else if (t == 32) {
         double sx = 0.0, sxx = 0.0;
         for (int j = 0; j < nb; ++j) { sx += xb[o + j] + xd[o + j]; sxx += xb[o + j] * xb[o + j] + xd[o + j] * xd[o + j]; }
@@ -1151,20 +1156,22 @@ extern "C" int lr_dataset_create(lr_handle_t h, int32_t n_rep, int32_t n_bins, i
     lr_dataset_t ds = new lr_dataset_s();
     ds->h = h; ds->n_rep = n_rep; ds->n_bins = n_bins; ds->model = model_BDI;
     ds->start_time = start_time; ds->end_time = end_time; ds->s0f = (int)floor(start_time);
-    ds->tab = nullptr; ds->cst = nullptr;
+    ds->tab = nullptr; ds->cst = nullptr; ds->terms = nullptr;
     ds->last.s = st; ds->last.valid = 1;
     // stream-ordered allocation: creating/destroying datasets and chains never synchronises the device, so a pipeline can
     // set up batch k+1 while the chains of batch k are still running (cudaFree would wait for them)
     cudaError_t e = cudaMallocAsync((void**)&ds->tab, (size_t)n_rep * LR_NTAB * (n_bins + 1) * sizeof(double), st);
     if (e == cudaSuccess) e = cudaMallocAsync((void**)&ds->cst, (size_t)n_rep * LR_NCST * sizeof(double), st);
+    if (e == cudaSuccess) e = cudaMallocAsync((void**)&ds->terms, (size_t)n_rep * 4 * n_bins * sizeof(double), st);
     if (e != cudaSuccess) {
         lr_set_error("lr_dataset_create: cudaMallocAsync failed: %s", cudaGetErrorString(e));
         if (ds->tab) cudaFreeAsync(ds->tab, st);
+        if (ds->cst) cudaFreeAsync(ds->cst, st);
         delete ds;
         return LR_ERR_NOMEM;
     }
     k2_build_tables<<<n_rep, 64, 0, st>>>((const long long*)d_sp, (const long long*)d_ex, d_br, (const long long*)d_ex_dead,
-                                           d_br_dead, n_bins, model_BDI, ds->tab, ds->cst);
+                                           d_br_dead, n_bins, model_BDI, ds->tab, ds->cst, ds->terms);
     LR_CUDA(cudaGetLastError());
     h->launches += 1;
     *out = ds;
@@ -1221,18 +1228,20 @@ extern "C" int lr_dataset_create_general_host(lr_handle_t h, int32_t n_rep, int3
     lr_dataset_t ds = new lr_dataset_s();
     ds->h = h; ds->n_rep = n_rep; ds->n_bins = n_bins; ds->model = model_tag;
     ds->start_time = start_time; ds->end_time = end_time; ds->s0f = (int)floor(start_time);
-    ds->tab = nullptr; ds->cst = nullptr;
+    ds->tab = nullptr; ds->cst = nullptr; ds->terms = nullptr;
     ds->last.s = h->stream; ds->last.valid = 1;
     cudaError_t e = cudaMallocAsync((void**)&ds->tab, (size_t)n_rep * LR_NTAB * (n_bins + 1) * sizeof(double), h->stream);
     if (e == cudaSuccess) e = cudaMallocAsync((void**)&ds->cst, (size_t)n_rep * LR_NCST * sizeof(double), h->stream);
+    if (e == cudaSuccess) e = cudaMallocAsync((void**)&ds->terms, (size_t)n_rep * 4 * n_bins * sizeof(double), h->stream);
     if (e != cudaSuccess) {
         lr_set_error("lr_dataset_create_general_host: cudaMallocAsync failed: %s", cudaGetErrorString(e));
         if (ds->tab) cudaFreeAsync(ds->tab, h->stream);
+        if (ds->cst) cudaFreeAsync(ds->cst, h->stream);
         delete ds;
         return LR_ERR_NOMEM;
     }
     k2_build_tables_general<<<n_rep, 64, 0, h->stream>>>(w, w + cnt, w + 2 * cnt, w + 3 * cnt, w + 4 * cnt, w + 5 * cnt, h_C ? w + 6 * cnt : nullptr,
-                                                           n_bins, ds->tab, ds->cst);
+                                                           n_bins, ds->tab, ds->cst, ds->terms);
     LR_CUDA(cudaGetLastError());
     h->launches += 1;
     LR_CUDA(cudaStreamSynchronize(h->stream));
@@ -1244,8 +1253,18 @@ extern "C" int lr_dataset_destroy(lr_dataset_t ds) {
     if (!ds) return LR_OK;
     cudaSetDevice(ds->h->device);
     lr_order(ds->h, &ds->last, ds->h->stream);        // readers on caller streams finish before the block returns to the pool
-    cudaFreeAsync(ds->tab, ds->h->stream); cudaFreeAsync(ds->cst, ds->h->stream);
+    cudaFreeAsync(ds->tab, ds->h->stream); cudaFreeAsync(ds->cst, ds->h->stream); cudaFreeAsync(ds->terms, ds->h->stream);
     delete ds;
+    return LR_OK;
+}
+
+extern "C" int lr_dataset_bin_terms(lr_dataset_t ds, double* d_out, void* stream) {
+    LR_REQUIRE(ds && d_out, "lr_dataset_bin_terms: null pointer");
+    LR_CUDA(cudaSetDevice(ds->h->device));
+    cudaStream_t st = stream ? (cudaStream_t)stream : ds->h->stream;
+    int rc = lr_order(ds->h, &ds->last, st);
+    if (rc != LR_OK) return rc;
+    LR_CUDA(cudaMemcpyAsync(d_out, ds->terms, (size_t)ds->n_rep * 4 * ds->n_bins * sizeof(double), cudaMemcpyDeviceToDevice, st));
     return LR_OK;
 }
 

@@ -442,6 +442,58 @@ __device__ __forceinline__ double u01(uint32_t hi, uint32_t lo) {
     return (x - 1.0) + 1.1102230246251565e-16;
 }
 
+// ---- Poisson counts from a Philox stream (K11) -----------------------------------------------------------------------------------
+// lr_poisson(mu) draws one Poisson(mu) count.  The draw takes Philox-4x32-10 blocks at counter (c0, c1, c2 | a << 25, c3) and key
+// (k0, k1) for attempt a = 0, 1, .. (c2 must leave bits 25..31 clear); each block gives the uniforms U1 = u01(x, y), U2 = u01(z, w).
+//   mu == 0          0, no draw
+//   mu < 10          inversion by sequential search (attempt 0, U1): p = exp(-mu), F = p, k = 0; while U1 > F: k += 1, p = p mu / k,
+//                    F = F + p.  More than LR_POIS_SEARCH steps exhaust the search.
+//   10 <= mu         Hormann's PTRS (transformed rejection with squeeze, 1993), the algorithm and constants of numpy's
+//                    random_poisson_ptrs: U = U1 - 1/2, V = U2 of attempt a; LR_POIS_ATTEMPTS attempts at most.
+// Every operation is one IEEE double operation in the order written (no contraction), so a host restatement with the same
+// exp / log / lgamma gives the same count; only those three functions can differ by a few ulp (literate_b200.predictive).
+// Returns -1 for a mu outside [0, LR_POIS_MU_MAX] or NaN (no draw) and 0 with *exhausted incremented when the loop ran out.
+#define LR_POIS_SEARCH 256
+#define LR_POIS_ATTEMPTS 64
+#define LR_POIS_MU_MAX 4503599627370496.0     // 2^52: every candidate count and k log(mu) stays exact in int64 / fp64
+__device__ __forceinline__ long long lr_poisson(double mu, uint32_t c0, uint32_t c1, uint32_t c2, uint32_t c3, uint32_t k0, uint32_t k1,
+                                                unsigned* exhausted) {
+    if (!(mu >= 0.0 && mu <= LR_POIS_MU_MAX)) return -1;
+    if (mu == 0.0) return 0;
+    if (mu < 10.0) {
+        const Philox4 r = philox4x32_10(c0, c1, c2, c3, k0, k1);
+        const double u = u01(r.x, r.y);
+        double p = exp(-mu), F = p;
+        long long k = 0;
+        while (u > F) {
+            if (k == LR_POIS_SEARCH) { ++*exhausted; return 0; }
+            k += 1;
+            p = __ddiv_rn(__dmul_rn(p, mu), (double)k);
+            F = __dadd_rn(F, p);
+        }
+        return k;
+    }
+    const double slam = sqrt(mu), loglam = log(mu);
+    const double b = __dadd_rn(0.931, __dmul_rn(2.53, slam));
+    const double a = __dadd_rn(-0.059, __dmul_rn(0.02483, b));
+    const double invalpha = __dadd_rn(1.1239, __ddiv_rn(1.1328, __dsub_rn(b, 3.4)));
+    const double vr = __dsub_rn(0.9277, __ddiv_rn(3.6224, __dsub_rn(b, 2.0)));
+    const double lia = log(invalpha);
+    for (uint32_t att = 0; att < LR_POIS_ATTEMPTS; ++att) {
+        const Philox4 r = philox4x32_10(c0, c1, c2 | (att << 25), c3, k0, k1);
+        const double U = __dsub_rn(u01(r.x, r.y), 0.5), V = u01(r.z, r.w);
+        const double us = __dsub_rn(0.5, fabs(U));
+        const double kd = floor(__dadd_rn(__dadd_rn(__dmul_rn(__dadd_rn(__ddiv_rn(__dmul_rn(2.0, a), us), b), U), mu), 0.43));
+        if (us >= 0.07 && V <= vr) return (long long)kd;
+        if (kd < 0.0 || (us < 0.013 && V > us)) continue;
+        const double lhs = __dsub_rn(__dadd_rn(log(V), lia), log(__dadd_rn(__ddiv_rn(a, __dmul_rn(us, us)), b)));
+        const double rhs = __dsub_rn(__dadd_rn(-mu, __dmul_rn(kd, loglam)), lgamma(__dadd_rn(kd, 1.0)));
+        if (lhs <= rhs) return (long long)kd;
+    }
+    ++*exhausted;
+    return 0;
+}
+
 // exp(x) for |x| <= 0.1 (the log-multipliers of update_multiplier_proposal_vec: |2 log(1.1) (u - .5)| <= 0.0954): Taylor series to
 // x^11, truncation error < 2e-21, i.e. rounding only.  The coefficients sit in constant memory: as literals every one costs
 // two UMOV before its DFMA (17 extra instructions per call); from the constant bank two arrive per LDCU.128.

@@ -370,6 +370,38 @@ class Device:
         (out,) = self._chain_call("lr_rank_diagnostics", records, cols, ladder, beta_col, [lambda S, M, k: (8, k)], stream)
         return dict(zip(RANK_FIELDS, out))
 
+    def predictive_check_device(self, records, layout, terms, rate_col=0, start_time=0.0, rep_of_chain=None, ladder=1, beta_col=-1,
+                                chain_id0=0, seed=0, per_record=False, stream=None):
+        """Posterior predictive check of the per-bin counts of a run (K11, lr_predictive_check), without copying the records;
+        predictive.predictive_check_host is the definition.  records: float64 CUDA tensor [n_samples, n_chains * ladder, w] with
+        contiguous rows (after the burn-in); layout 0 RJMCMC records, 1 dense per-bin rates from field rate_col (K6: 16, K7: 24);
+        terms [n_rep, 4, n_bins] (A^b, B^b, A^d, B^d; torch or numpy); rep_of_chain [n_chains] (None: 0); ladder / beta_col as for
+        chain_diagnostics_device.  Returns a dict of CUDA tensors: bin_count int64 [2, 4, n_bins], bin_sum float64 [2, 3, n_bins],
+        glob_count int64 [4], glob_sum float64 [6], status int64 [3] and, with per_record, dev float64 [n_samples, n_chains, 4]."""
+        import torch
+        S, M, stride = _chain_records(records, ladder)
+        d = records.device
+        terms = torch.as_tensor(terms, dtype=torch.float64).to(d).contiguous()
+        if terms.dim() == 2:
+            terms = terms[None]
+        if terms.dim() != 3 or terms.shape[1] != 4:
+            raise ValueError("terms must be [n_rep, 4, n_bins]")
+        n_rep, _, nb = terms.shape
+        rep = None if rep_of_chain is None else np.ascontiguousarray(np.broadcast_to(np.asarray(rep_of_chain, np.int32), (M,)))
+        out = {"bin_count": torch.empty((2, 4, nb), dtype=torch.int64, device=d), "bin_sum": torch.empty((2, 3, nb), dtype=torch.float64, device=d),
+               "glob_count": torch.empty(4, dtype=torch.int64, device=d), "glob_sum": torch.empty(6, dtype=torch.float64, device=d),
+               "status": torch.empty(3, dtype=torch.int64, device=d)}
+        if per_record:
+            out["dev"] = torch.empty((S, M, 4), dtype=torch.float64, device=d)
+        ptr = lambda k: C.c_void_p(out[k].data_ptr()) if k in out else None
+        N.check(self.lib.lr_predictive_check(self.h, C.c_void_p(records.data_ptr()), int(S), int(M), int(ladder), int(beta_col), int(stride),
+                                             int(layout), int(rate_col), float(start_time), int(nb), C.c_void_p(terms.data_ptr()), int(n_rep),
+                                             N.np_ptr(rep), int(chain_id0), int(seed) & (2 ** 64 - 1), ptr("bin_count"), ptr("bin_sum"),
+                                             ptr("glob_count"), ptr("glob_sum"), ptr("dev"), ptr("status"), _stream_ptr(stream, d)),
+                "lr_predictive_check")
+        out["terms"] = terms           # keeps the staged terms alive until the stream has used them
+        return out
+
     def new_accumulators(self, n_rep, n_bins, device):
         import torch
         return torch.zeros((n_rep, N.LR_ACC_ROWS, int(self.lib.lr_acc_stride(int(n_bins)))), dtype=torch.int64, device=device)
@@ -468,6 +500,14 @@ class Dataset:
             self.close()
         except Exception:
             pass
+
+    def bin_terms(self, stream=None):
+        """The per-bin terms the likelihood sums (lr_dataset_bin_terms): float64 CUDA tensor [n_rep, 4, n_bins] = A_birth, B_birth,
+        A_death, B_death, the likelihood being C + sum_j [A_b log lambda_j - B_b lambda_j] + sum_j [A_d log mu_j - B_d mu_j]."""
+        import torch
+        out = torch.empty((self.n_rep, 4, self.n_bins), dtype=torch.float64, device=torch.device("cuda", self.dev.index))
+        N.check(self.dev.lib.lr_dataset_bin_terms(self.ds, C.c_void_p(out.data_ptr()), _stream_ptr(stream, out.device)), "lr_dataset_bin_terms")
+        return out
 
     def evaluate(self, states, gamma_rate=None, poi_lambda=None, rep=None):
         """Likelihood / prior / adequacy of explicit states (lr_state_eval_host).
