@@ -417,6 +417,30 @@ int lr_predictive_check(lr_handle_t h, const double* d_rows, int64_t n_samples, 
                         const double* d_terms, int32_t n_rep, const int32_t* h_rep_of_chain, int64_t chain_id0, uint64_t seed,
                         int64_t* d_bin_count, double* d_bin_sum, int64_t* d_glob_count, double* d_glob_sum, double* d_dev,
                         int64_t* d_status, void* stream);
+/* K12: Pareto-smoothed importance-sampling leave-one-out (PSIS-LOO, Vehtari et al.) and WAIC of a run over its per-bin births and
+ * deaths, without copying the records.  literate_b200.loo.loo_host is the definition, step for step.
+ * The observation is the count A of side s in bin j with B > 0 (K11's unit); its pointwise log-likelihood given a record is the
+ * Poisson log pmf  l_sj = A log(r_sj B_sj) - r_sj B_sj - lgamma(A + 1)  (0 for the first term when A = 0): summed over the
+ * columns it is the sampler's likelihood plus a constant of the run.
+ *   rows, layout, rate_col, start_time, n_bins   as for lr_predictive_check (one table: every chain runs on d_terms)
+ *   d_terms      fp64 [4][n_bins]: A^b, B^b, A^d, B^d
+ *   used         a record K11 would use whose every l_sj is finite; the S used records of all chains are pooled
+ * Per column, over the S used draws: r_eff = ESS / S with the "mean" ESS of lr_chain_diagnostics of exp(l - max l) over the
+ * chains (1 when that is NaN: a column with an unused record or constant); PSIS of -l as ArviZ's _psislw / _gpdfit / _gpinv
+ * (tail of M = ceil(min(0.2 S, 3 sqrt(S / r_eff))) draws, T of them above the cutoff, k_hat = +inf and no smoothing for T <= 4);
+ * elpd_loo = logsumexp(l + lw), lppd = logsumexp(l) - log S, p_loo = lppd - elpd_loo, p_waic = var(l, ddof 1),
+ * elpd_waic = lppd - p_waic.
+ * Outputs:
+ *   d_out        fp64 [9][2][n_bins]: A, lppd, elpd_loo, p_loo, elpd_waic, p_waic, k_hat, r_eff, T; NaN where B = 0 (and all
+ *                but A when fewer than 2 records are used)
+ *   d_n          int64 [1]: records used
+ *   d_status     int64 [2]: records skipped as unusable, (sample, ladder) pairs without a member at beta = 1
+ * Every sum is compensated and in a fixed order: repeated calls are bit-identical.  Scratch comes from the handle's workspace: about
+ * 1 GiB of batch buffers (about 25 bytes per record and column, columns in batches) plus lr_chain_diagnostics' own.  Rejects what
+ * lr_chain_diagnostics rejects, a layout other than 0 / 1 and rate fields outside the row.  Returns when the outputs are written. */
+int lr_loo(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
+           int64_t row_stride, int32_t layout, int32_t rate_col, double start_time, int32_t n_bins, const double* d_terms,
+           double* d_out, int64_t* d_n, int64_t* d_status, void* stream);
 
 /* ---------------------------------------------------------------- TrendRate (SURVEY 8 f-4): fixed-dimension chains on the same statistics
  *

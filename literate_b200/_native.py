@@ -39,7 +39,7 @@ EXPORTS = [
     "lr_dd_run", "lr_dd_run_host", "lr_dd_eval_host", "lr_dd_state_host",
     "lr_dd_set_beta_host", "lr_dd_swap_info", "lr_dd_swap_apply", "lr_dd_swap_step", "lr_dd_temper_host",
     "lr_column_hpd", "lr_chain_diagnostics", "lr_rank_transform", "lr_rank_diagnostics",
-    "lr_dataset_bin_terms", "lr_predictive_check",
+    "lr_dataset_bin_terms", "lr_predictive_check", "lr_loo",
 ]
 
 
@@ -130,6 +130,7 @@ def load(build_if_missing=False):
     sig("lr_rank_diagnostics", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, vp, vp, vp, vp, vp, vp, vp)
     sig("lr_predictive_check", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, i32, f64, i32, vp, i32, vp, i64, u64,
         vp, vp, vp, vp, vp, vp, vp)
+    sig("lr_loo", C.c_int, vp, vp, i64, i64, i32, i32, i64, i32, i32, f64, i32, vp, vp, vp, vp, vp)
     sig("lr_trend_create", C.c_int, vp, i32, i32, vp, vp, vp, vp, i32, i32, i32, u64, i64, vp, vp, P(vp))
     sig("lr_trend_create_host", C.c_int, vp, i32, i32, vp, vp, vp, vp, i32, i32, i32, u64, i64, vp, P(vp))
     sig("lr_trend_destroy", C.c_int, vp)

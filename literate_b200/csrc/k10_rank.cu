@@ -59,17 +59,6 @@ struct K10Args {
 
 __device__ __forceinline__ unsigned long long k10_key(double v) { return lr_key(v == 0.0 ? 0.0 : v); }
 
-// the passes a segment needs: bit d set when some keys differ in digit d
-__device__ __forceinline__ unsigned k10_passes(unsigned long long a, unsigned long long o) {
-    const unsigned long long d = a ^ o;
-    unsigned m = 0;
-#pragma unroll
-    for (int q = 0; q < 8; ++q) m |= ((d >> (8 * q)) & 255ull) ? (1u << q) : 0u;
-    return m;
-}
-// the buffer (0 / 1) that holds a segment before pass d, and after the last pass (d = 8)
-__device__ __forceinline__ int k10_src(unsigned passes, int d) { return __popc(passes & ((1u << d) - 1u)) & 1; }
-
 __global__ void k10_init_kernel(const K10Args p) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= p.n_cols) return;
@@ -152,9 +141,9 @@ struct K10Sort {
 __global__ void __launch_bounds__(K10_ST) k10_hist_kernel(const K10Sort q, int d) {
     __shared__ unsigned h[256];
     const int seg = blockIdx.y, tid = threadIdx.x;
-    const unsigned passes = k10_passes(q.band[seg], q.bor[seg]);
+    const unsigned passes = lr_radix_passes(q.band[seg], q.bor[seg]);
     if (!((passes >> d) & 1u)) return;
-    const unsigned long long* in = (k10_src(passes, d) ? q.b1 : q.b0) + (size_t)seg * q.L;
+    const unsigned long long* in = (lr_radix_src(passes, d) ? q.b1 : q.b0) + (size_t)seg * q.L;
     h[tid] = 0;
     __syncthreads();
     const unsigned lt = (1u << (tid & 31)) - 1u;
@@ -174,7 +163,7 @@ __global__ void __launch_bounds__(K10_ST) k10_hist_kernel(const K10Sort q, int d
 __global__ void __launch_bounds__(1024) k10_scan_kernel(const K10Sort q, int d) {
     __shared__ unsigned ws[32];
     const int seg = blockIdx.x, tid = threadIdx.x;
-    const unsigned passes = k10_passes(q.band[seg], q.bor[seg]);
+    const unsigned passes = lr_radix_passes(q.band[seg], q.bor[seg]);
     if (!((passes >> d) & 1u)) return;
     unsigned* g = q.ghist + (size_t)seg * 256 * q.tiles;
     const long long E = 256LL * q.tiles, per = (E + 1023) / 1024;
@@ -205,9 +194,9 @@ __global__ void __launch_bounds__(K10_ST) k10_scatter_kernel(const K10Sort q, in
     __shared__ unsigned cnt[K10_SW][256];
     __shared__ unsigned off[K10_SW][256];
     const int seg = blockIdx.y, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const unsigned passes = k10_passes(q.band[seg], q.bor[seg]);
+    const unsigned passes = lr_radix_passes(q.band[seg], q.bor[seg]);
     if (!((passes >> d) & 1u)) return;
-    const int src = k10_src(passes, d);
+    const int src = lr_radix_src(passes, d);
     const unsigned long long* in = (src ? q.b1 : q.b0) + (size_t)seg * q.L;
     unsigned long long* out = (src ? q.b0 : q.b1) + (size_t)seg * q.L;
     base[tid] = q.ghist[((size_t)seg * 256 + tid) * q.tiles + blockIdx.x];
@@ -284,9 +273,9 @@ __device__ double k10_quantile(const unsigned long long* a, long long na, const 
 __global__ void k10_quant_kernel(const K10Args p) {
     const int c = blockIdx.x * blockDim.x + threadIdx.x;
     if (c >= p.n_cols) return;
-    const unsigned passes = k10_passes(p.band[c], p.bor[c]);
-    const unsigned long long* a = p.kx[k10_src(passes, 8)] + (size_t)c * p.N;
-    const unsigned long long* b = p.km[k10_src(passes, 8)] + (size_t)c * p.Nmid;
+    const unsigned passes = lr_radix_passes(p.band[c], p.bor[c]);
+    const unsigned long long* a = p.kx[lr_radix_src(passes, 8)] + (size_t)c * p.N;
+    const unsigned long long* b = p.km[lr_radix_src(passes, 8)] + (size_t)c * p.Nmid;
     const int fl = p.flag[c];
     const double med = (fl & 2) ? CUDART_NAN : __dadd_rn(lr_val(a[p.N / 2 - 1]), lr_val(a[p.N / 2])) / 2.0;
     const double q05 = (fl & 4) ? CUDART_NAN : k10_quantile(a, p.N, b, p.Nmid, 0.05);
@@ -316,7 +305,7 @@ __global__ void __launch_bounds__(K10_TW * 32) k10_rank_kernel(const K10Args p) 
     const unsigned long long* sorted = nullptr;
     double med = 0.0, q05 = 0.0, q95 = 0.0;
     if (has) {
-        sorted = p.kx[k10_src(k10_passes(p.band[col], p.bor[col]), 8)] + (size_t)col * p.N;
+        sorted = p.kx[lr_radix_src(lr_radix_passes(p.band[col], p.bor[col]), 8)] + (size_t)col * p.N;
         med = p.quant[col]; q05 = p.quant[p.qn + col]; q95 = p.quant[2 * p.qn + col];
     }
     unsigned long long kand = ~0ull, kor = 0ull;
@@ -357,7 +346,7 @@ __global__ void __launch_bounds__(K10_TW * 32) k10_rank_fold_kernel(const K10Arg
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const int col = blockIdx.y * K10_G + lane;
     if (col >= p.n_cols) return;
-    const unsigned long long* sorted = p.kf[k10_src(k10_passes(p.fand[col], p.f_or[col]), 8)] + (size_t)col * p.N;
+    const unsigned long long* sorted = p.kf[lr_radix_src(lr_radix_passes(p.fand[col], p.f_or[col]), 8)] + (size_t)col * p.N;
     for (long long pos = (long long)blockIdx.x * K10_TW + warp; pos < p.N; pos += (long long)gridDim.x * K10_TW) {
         double* zr = p.Z + pos * p.zs + p.zq + col;
         zr[0] = k10_z(sorted, p.N, k10_key(zr[0]));
@@ -469,6 +458,14 @@ void k10_args(K10Args* p, const double* d_rows, int64_t n_samples, int64_t n_cha
 }
 
 }  // namespace
+
+size_t lr_k10_sort_ghist(int64_t L) { return (size_t)256 * std::max<int64_t>(1, (L + K10_TILE - 1) / K10_TILE); }
+
+int lr_k10_sort(lr_handle_t h, unsigned long long* b0, unsigned long long* b1, int64_t L, int segs, const unsigned long long* band,
+                const unsigned long long* bor, unsigned* ghist, cudaStream_t st) {
+    const K10Sort q{b0, b1, L, (int)((L + K10_TILE - 1) / K10_TILE), band, bor, ghist};
+    return k10_sort(h, q, segs, st);
+}
 
 extern "C" int lr_rank_transform(lr_handle_t h, const double* d_rows, int64_t n_samples, int64_t n_chains, int32_t ladder, int32_t beta_col,
                                  int64_t row_stride, int32_t n_cols, const int32_t* h_col_a, const int32_t* h_col_b,

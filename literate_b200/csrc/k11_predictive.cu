@@ -68,36 +68,6 @@ __device__ __forceinline__ double k11_warp_sum(double v) {
     return isfinite(s) ? __dadd_rn(s, c) : s;
 }
 
-// K3 record: stage the first bin of every segment of `side` in sjb[32] (the warp's) and return K (0: the side is unusable --
-// K outside 1..32, a non-finite shift time or segments out of order)
-__device__ __forceinline__ int k11_k3_stage(const K11Args& p, const double* row, int side, int lane, int* sjb) {
-    __syncwarp();                                              // the previous record's searches are done with sjb
-    const double kd = row[side ? 6 : 5];
-    const int K = (kd >= 1.0 && kd <= 32.0 && kd == floor(kd)) ? (int)kd : 0;
-    const double t = row[(side ? 112 : 48) + lane];
-    bool ok = true;
-    int jb = 0;
-    if (lane > 0 && lane < K) {
-        ok = isfinite(t);
-        jb = ok ? (int)fmin(fmax(floor(t) - (double)p.s0f, 0.0), (double)p.nb) : 0;
-    }
-    sjb[lane] = jb;
-    __syncwarp();
-    if (lane > 0 && lane < K && jb < sjb[lane - 1]) ok = false;
-    const bool all = __all_sync(0xffffffffu, ok);
-    __syncwarp();
-    return all ? K : 0;
-}
-// slot of bin j: the last k < K with sjb[k] <= j (sjb[0] = 0)
-__device__ __forceinline__ int k11_k3_slot(const int* sjb, int K, int j) {
-    int lo = 0, hi = K - 1;
-    while (lo < hi) {
-        const int mid = (lo + hi + 1) >> 1;
-        if (sjb[mid] <= j) lo = mid; else hi = mid - 1;
-    }
-    return lo;
-}
-
 // one warp per logical record: which records are used
 __global__ void __launch_bounds__(K11_RB) k11_scan_kernel(const K11Args p) {
     __shared__ int sjb[K11_RB / 32][2][32];
@@ -113,8 +83,8 @@ __global__ void __launch_bounds__(K11_RB) k11_scan_kernel(const K11Args p) {
     } else {
         int K[2] = {0, 0};
         if (p.layout == 0) {
-            K[0] = k11_k3_stage(p, row, 0, lane, sjb[warp][0]);
-            K[1] = k11_k3_stage(p, row, 1, lane, sjb[warp][1]);
+            K[0] = lr_k3_stage(p.s0f, p.nb, row, 0, lane, sjb[warp][0]);
+            K[1] = lr_k3_stage(p.s0f, p.nb, row, 1, lane, sjb[warp][1]);
         }
         bool ok = (p.layout != 0 || (K[0] > 0 && K[1] > 0)) && row[0] >= 0.0 && row[0] < 9.2e18;   // the iteration keys the draws
         if (ok) {
@@ -123,7 +93,7 @@ __global__ void __launch_bounds__(K11_RB) k11_scan_kernel(const K11Args p) {
                 for (int j = lane; j < p.nb; j += 32) {
                     const double B = T[(2 * side + 1) * p.nb + j];
                     if (!(B > 0.0)) continue;
-                    const double rate = p.layout == 0 ? row[(side ? 80 : 16) + k11_k3_slot(sjb[warp][side], K[side], j)]
+                    const double rate = p.layout == 0 ? row[(side ? 80 : 16) + lr_k3_slot(sjb[warp][side], K[side], j)]
                                                       : row[p.rate_col + side * p.nb + j];
                     const double mu = __dmul_rn(rate, B);
                     ok &= mu >= 0.0 && mu <= LR_POIS_MU_MAX;
@@ -158,12 +128,12 @@ __global__ void __launch_bounds__(256) k11_draw_kernel(const K11Args p) {
                 const long long s = r / p.src.M, c = r - s * p.src.M;
                 const double* row = lr_chain_row(p.src, s, c, lane, nullptr);
                 int K = 0;
-                if (p.layout == 0) K = k11_k3_stage(p, row, side, lane, sjb);
+                if (p.layout == 0) K = lr_k3_stage(p.s0f, p.nb, row, side, lane, sjb);
                 const double* T = p.terms + (size_t)p.rep[c] * 4 * p.nb;
                 if (on) {
                     const double A = T[2 * side * p.nb + j], B = T[(2 * side + 1) * p.nb + j];
                     if (B > 0.0) {
-                        const double rate = p.layout == 0 ? row[(side ? 80 : 16) + k11_k3_slot(sjb, K, j)] : row[p.rate_col + side * p.nb + j];
+                        const double rate = p.layout == 0 ? row[(side ? 80 : 16) + lr_k3_slot(sjb, K, j)] : row[p.rate_col + side * p.nb + j];
                         const double mu = __dmul_rn(rate, B);
                         const long long it = (long long)row[0];
                         const unsigned long long g = (unsigned long long)(p.chain_id0 + c);

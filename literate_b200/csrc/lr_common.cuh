@@ -370,6 +370,55 @@ inline int lr_check_chain_rows(const char* who, lr_handle_t h, bool outs, const 
     return lr_check_col_specs(who, n_cols, row_stride, h_col_a, h_col_b, h_col_sign);
 }
 
+// ---- the likelihood's record-to-bin rate mapping of K3 records (K11, K12): segment k of a side starts at bin
+// floor(t_k) - floor(start_time) (s0f), clamped to [0, nb]; bin j takes the last segment starting at or before it.
+// lr_k3_stage stages the first bin of every segment of `side` in sjb[32] (the warp's) and returns K (0: the side is unusable --
+// K outside 1..32, a non-finite shift time or segments out of order); a warp-wide call.
+__device__ __forceinline__ int lr_k3_stage(int s0f, int nb, const double* row, int side, int lane, int* sjb) {
+    __syncwarp();                                              // the previous record's searches are done with sjb
+    const double kd = row[side ? 6 : 5];
+    const int K = (kd >= 1.0 && kd <= 32.0 && kd == floor(kd)) ? (int)kd : 0;
+    const double t = row[(side ? 112 : 48) + lane];
+    bool ok = true;
+    int jb = 0;
+    if (lane > 0 && lane < K) {
+        ok = isfinite(t);
+        jb = ok ? (int)fmin(fmax(floor(t) - (double)s0f, 0.0), (double)nb) : 0;
+    }
+    sjb[lane] = jb;
+    __syncwarp();
+    if (lane > 0 && lane < K && jb < sjb[lane - 1]) ok = false;
+    const bool all = __all_sync(0xffffffffu, ok);
+    __syncwarp();
+    return all ? K : 0;
+}
+// slot of bin j: the last k < K with sjb[k] <= j (sjb[0] = 0)
+__device__ __forceinline__ int lr_k3_slot(const int* sjb, int K, int j) {
+    int lo = 0, hi = K - 1;
+    while (lo < hi) {
+        const int mid = (lo + hi + 1) >> 1;
+        if (sjb[mid] <= j) lo = mid; else hi = mid - 1;
+    }
+    return lo;
+}
+
+// ---- K10's segmented LSD radix sort of 64-bit keys (k10_rank.cu) on a caller's buffers: segment s of length L sits at b0 + s L;
+// its digit d is sorted only when some of its keys differ there (band / bor: the AND and OR of the segment's keys, bit d of
+// lr_radix_passes), so the sorted segment ends in b0 or b1 as lr_radix_src(passes, 8) says.  ghist holds lr_k10_sort_ghist(L)
+// words per segment.  Asynchronous on st.
+__device__ __forceinline__ unsigned lr_radix_passes(unsigned long long a, unsigned long long o) {
+    const unsigned long long d = a ^ o;
+    unsigned m = 0;
+#pragma unroll
+    for (int q = 0; q < 8; ++q) m |= ((d >> (8 * q)) & 255ull) ? (1u << q) : 0u;
+    return m;
+}
+// the buffer (0 / 1) that holds a segment before pass d, and after the last pass (d = 8)
+__device__ __forceinline__ int lr_radix_src(unsigned passes, int d) { return __popc(passes & ((1u << d) - 1u)) & 1; }
+size_t lr_k10_sort_ghist(int64_t L);
+int lr_k10_sort(lr_handle_t h, unsigned long long* b0, unsigned long long* b1, int64_t L, int segs, const unsigned long long* band,
+                const unsigned long long* bor, unsigned* ghist, cudaStream_t st);
+
 // ---- K9's host driver on a caller's scratch (k9_diag.cu): lr_chain_diagnostics runs it on the workspace, K10 on the part of the
 // workspace behind its own buffers.  lr_k9_scratch_bytes is what lr_k9_run uses from `w` (the staged specs and at most ~256 MB);
 // the arguments are those of lr_chain_diagnostics, already checked, `who` names the entry point in errors.

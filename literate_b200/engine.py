@@ -402,6 +402,26 @@ class Device:
         out["terms"] = terms           # keeps the staged terms alive until the stream has used them
         return out
 
+    def loo_device(self, records, layout, terms, rate_col=0, start_time=0.0, ladder=1, beta_col=-1, stream=None):
+        """PSIS-LOO and WAIC of the per-bin counts of a run on one table (K12, lr_loo), without copying the records; loo.loo_host
+        is the definition.  records, layout, rate_col, start_time, ladder and beta_col as for predictive_check_device; terms
+        [4, n_bins] (A^b, B^b, A^d, B^d; torch or numpy).  Returns a dict of CUDA tensors: out float64 [9, 2, n_bins] (A, lppd,
+        elpd_loo, p_loo, elpd_waic, p_waic, k_hat, r_eff, T), n int64 [1] (records used), status int64 [2] (skipped, ladders
+        without a cold member).  Returns when the outputs are written."""
+        import torch
+        S, M, stride = _chain_records(records, ladder)
+        d = records.device
+        terms = torch.as_tensor(terms, dtype=torch.float64).to(d).contiguous()
+        if terms.dim() != 2 or terms.shape[0] != 4:
+            raise ValueError("terms must be [4, n_bins]")
+        nb = terms.shape[1]
+        out = {"out": torch.empty((9, 2, nb), dtype=torch.float64, device=d), "n": torch.empty(1, dtype=torch.int64, device=d),
+               "status": torch.empty(2, dtype=torch.int64, device=d)}
+        N.check(self.lib.lr_loo(self.h, C.c_void_p(records.data_ptr()), int(S), int(M), int(ladder), int(beta_col), int(stride), int(layout),
+                                int(rate_col), float(start_time), int(nb), C.c_void_p(terms.data_ptr()), C.c_void_p(out["out"].data_ptr()),
+                                C.c_void_p(out["n"].data_ptr()), C.c_void_p(out["status"].data_ptr()), _stream_ptr(stream, d)), "lr_loo")
+        return out
+
     def new_accumulators(self, n_rep, n_bins, device):
         import torch
         return torch.zeros((n_rep, N.LR_ACC_ROWS, int(self.lib.lr_acc_stride(int(n_bins)))), dtype=torch.int64, device=device)

@@ -362,14 +362,7 @@ def chain_ids(paths, kind):
     ddrate.py as <table>_<seed + i><model>.log (i counted from the lowest seed among the logs).  K11 keys its draws by the chain
     id, so the logs give the draws of the device records they were written from.  Refuses names outside these patterns and
     logs that are not consecutive chains of one run.  Returns (sorted paths, first chain id)."""
-    keys = []
-    for p in paths:
-        b = os.path.basename(p)
-        m = re.match(r"(.*?)(?:_chain(\d+))?_mcmc\.log$", b) if kind == "forward" else re.match(r"(.*)_(\d+)(_[A-Z]+_M[A-Z]+)\.log$", b)
-        if not m:
-            raise ValueError("%s: not a log name of the sampler (%s)" % (p, "<table><model><out>[_chain<i>]_mcmc.log" if kind == "forward"
-                                                                          else "<table>_<seed><model>.log"))
-        keys.append((m.group(1), int(m.group(2) or 0)) if kind == "forward" else (m.group(1) + m.group(3), int(m.group(2))))
+    keys = [log_key(p, kind) for p in paths]
     stems = sorted({k[0] for k in keys})
     i0 = 0 if kind == "forward" else min(k[1] for k in keys)
     ids = [(i - i0) * len(stems) + stems.index(st) for st, i in keys]
@@ -378,6 +371,17 @@ def chain_ids(paths, kind):
     if ids != list(range(ids[0], ids[0] + len(ids))):
         raise ValueError("the logs are not consecutive chains of one run (chains %s)" % ids)
     return [paths[o] for o in order], ids[0]
+
+
+def log_key(path, kind):
+    """(stem, run index) of a log name: forward.py's <table><model><out>[_chain<i>]_mcmc.log -> (<table><model><out>, i), ddrate.py's
+    <table>_<seed><model>.log -> (<table><model>, seed).  Logs of one run share the stems of its tables."""
+    b = os.path.basename(path)
+    m = re.match(r"(.*?)(?:_chain(\d+))?_mcmc\.log$", b) if kind == "forward" else re.match(r"(.*)_(\d+)(_[A-Z]+_M[A-Z]+)\.log$", b)
+    if not m:
+        raise ValueError("%s: not a log name of the sampler (%s)" % (path, "<table><model><out>[_chain<i>]_mcmc.log" if kind == "forward"
+                                                                         else "<table>_<seed><model>.log"))
+    return (m.group(1), int(m.group(2) or 0)) if kind == "forward" else (m.group(1) + m.group(3), int(m.group(2)))
 
 
 def model_tag(path):
